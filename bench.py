@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's sm_100a path
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                          # the reference's CPU path
+    python bench.py --dump-outputs DIR ...                        # + what the last timed step computed, DIR/*.npy
 
 Workload (BASELINE.json configs[1]; SURVEY.md §8d config 2): ViT-Small (D=384, L=12, h=6,
 M=1536, patch 16), classification, 45 classes, 256x256x3 synthetic RESISC45-shaped images,
@@ -167,7 +168,7 @@ def run_reference(args):
     if rank != 0:
         return
     batch = args.ref_batch
-    steps, warmup = max(1, min(args.steps, 6)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     try:
         ips, ms, threads = cpu_reference_throughput(batch, steps, warmup, args.q_format)
         kind, what = "reference", "unmodified reference package (oracle/_ref) + qtorch shim over oracle/quant_oracle.c"
@@ -411,6 +412,26 @@ def quant_microbench(dev, peaks):
     return quant
 
 
+DUMP_MAX_ELEMENTS = 1 << 18       # per array; with it the ViT-Small gradients come to 47 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (name, tensor) as out_dir/<name>.npy in float32.  An array of more than DUMP_MAX_ELEMENTS values
+    is written as a fixed, seeded sample of its flattened values (sorted positions, the same in every run), so the
+    dumps of two builds can be compared value for value."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays:
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(1234).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))
+            a = a.reshape(-1)[idx]
+        total += a.nbytes
+        assert total <= 64e6, "output dump exceeds 64 MB at %s" % name
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------
 def run_b200(args):
     import torch
@@ -439,8 +460,10 @@ def run_b200(args):
 
     def step(img, y):
         model.zero_grad(set_to_none=True)
-        loss = F.cross_entropy(net(img), y)
+        out = net(img)
+        loss = F.cross_entropy(out, y)
         loss.backward()
+        step.logits = out.detach()        # detached: a live autograd graph breaks the CUDA-graph capture below
         return loss
 
     def barrier():
@@ -564,9 +587,16 @@ def run_b200(args):
         sys.stdout.flush(); sys.stderr.flush()
         os._exit(0)
 
+    if args.dump_outputs:                 # the e2e loop ran the last timed step
+        dump_outputs(args.dump_outputs, [("loss", loss), ("logits", gstep.output if use_graph else step.logits)] +
+                     [("grad." + n, p.grad) for n, p in model.named_parameters() if p.grad is not None])
+
     # ---- roofline of the dominant kernel class
-    with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
-        peaks = json.load(f) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else {}
+    # measured peaks of this GPU, if a measurement left them next to bench.py; the fallbacks are used otherwise
+    peaks = {}
+    if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")):
+        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
+            peaks = json.load(f)
     n_tok = (IMAGE // PATCH) ** 2 + 1
     D, Mm, L = ARCH["dim"], ARCH["mlp_dim"], ARCH["depth"]
     traffic = {}
@@ -604,7 +634,7 @@ def run_b200(args):
                                      ("seg256 (config 4)", "segmentation", args.q_format, args.batch),
                                      ("det800 (config 5)", "detection", args.q_format, 8)):
             try:
-                configs[name] = time_config(name, task, fmt, bsz, dev, max(3, min(args.steps, 10)), peaks)
+                configs[name] = time_config(name, task, fmt, bsz, dev, args.steps, peaks)
             except Exception as e:       # a secondary workload must not cost the headline line
                 configs[name] = {"error": repr(e)[:300]}
                 torch.cuda.empty_cache()
@@ -668,7 +698,11 @@ def main():
     ap.add_argument("--no-quant-bench", action="store_true", help="skip the fake-quant kernel GB/s microbench")
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary workloads (FP16_16, TF32, seg256, det800)")
     ap.add_argument("--no-graph", action="store_true", help="time the eagerly launched step instead of the CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, logits and parameter gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

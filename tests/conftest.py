@@ -3,6 +3,12 @@ import sys
 
 import pytest
 
+# The oracle tests compare CPU fp32 results with stored fixtures to within op-ordering noise, and the fake
+# quantisers turn a last-bit difference into a rounding flip.  The fixtures were computed on MKL's AVX-512 code
+# path; pinning MKL to that branch (conditional numerical reproducibility) makes other x86 hosts compute the same
+# bits.  MKL reads the setting at its first call, so it is set here, before any test runs.
+os.environ.setdefault("MKL_CBWR", "AVX512")
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "myrtle-vision_b200")
 for p in (ROOT, PKG):
