@@ -116,6 +116,15 @@ typedef struct {
     int cluster;                  /* 0 = CTA-pair kernel (tcgen05 cta_group::2, 256 x tile_n cluster tiles; 16-bit operands);
                                    * 1 = single-CTA kernel (always used for tf32); 2 = single-CTA MMAs with the B tile
                                    * TMA-multicast across a CTA pair (kept for comparison) */
+    /* Dropout (see "dropout mask" below); drop_seed == NULL: off.  The output [M, N] is the site tensor (C = N):
+     * value (m, n) is multiplied by keep(seed, site, m*N + n) * drop_scale right after q_out — before the residual
+     * add and q_res; in MV_EPI_GELU both gelu(u) and the stored gelu'(u) are multiplied before they are rounded, so the
+     * MV_EPI_DGELU backward applies the mask without knowing about it.  CTA-pair kernel only (16-bit operands), not
+     * with accumulate or colsum. */
+    const uint64_t* drop_seed;    /* device pointer to the 64-bit seed */
+    uint32_t drop_thr;            /* keep when bits16 >= drop_thr; drop_thr = nearbyint(p * 65536) */
+    float drop_scale;             /* 1 / (1 - p) in fp32 (0 for p == 1) */
+    int drop_site;
 } mv_gemm_args;
 
 int mv_gemm(const mv_gemm_args* args, void* stream);
@@ -157,6 +166,15 @@ int mv_layernorm_q_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const float*
                        float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
                        float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
                        void* stream);
+/* mv_layernorm_q_bwd with a dropout mask (site, see "dropout mask") applied to what feeds the Linear in front of the
+ * residual stream: dx_f16 and the dbias_prev column sums get keep * scale times dx; the fp32 dx (the residual
+ * gradient) stays unmasked unless mask_dx != 0 (then every output is masked: the embedding site).  seed_dev NULL:
+ * exactly mv_layernorm_q_bwd. */
+int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
+                            int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
+                            float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
+                            float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
+                            const uint64_t* seed_dev, int site, uint32_t thr, float scale, int mask_dx, void* stream);
 /* Gradient quantiser (QPyTorch's Quantizer(backward_number=FloatingPoint(exp, man), backward_rounding="nearest"),
  * qtorch/quant/quant_module.py — an option the reference's NumberFormat.quantizer never sets, utils/quantize.py:47-72;
  * named by the north star).  Process-wide; (0, 0) = off, the default.  When on, mv_layernorm_q_bwd rounds the
@@ -181,6 +199,19 @@ int mv_convert_f32(const float* in, void* out, int out_dtype, int64_t n, void* s
  * gradient scale is chosen on the device (no host sync); this applies / removes it in one pass. */
 int mv_scale_f32(const float* in, const float* scale_dev, int invert, float* out_f32, void* out_f16, int64_t n,
                  void* stream);
+/* ---------------------------------------------------------------- dropout mask
+ * nn.Dropout(p) at a site of the encoder (the tensor is token-major [rows = B*N, cols = C]; element i = m*C + c):
+ *   keep(seed, site, i) = bits16(seed, site, i) >= thr,   thr = (uint32) nearbyint(p * 65536)
+ *   bits16 = half-word (i & 7) of Philox4x32-10(key = seed, counter = {i >> 3, site}) — the 16-bit stream of
+ *            mv_float_quantize with offset = site (mv_philox_bits16 dumps it)
+ *   D(y) = y * keep * scale,  scale = 1 / (1 - p) in fp32 (0 for p == 1); the drop probability is thr / 65536.
+ * A pure function of (seed, site, m, c): forward, backward and the oracle see one mask whatever the tiling.
+ * The seed is read from device memory (drawn per training forward from torch's generator), never a host constant.
+ * Sites of encoder block l: 3l + 0 (to_out), 3l + 1 (after GELU), 3l + 2 (fc2); 3 * depth: after the positional add. */
+/* out[rows, cols] = in * keep * scale; in / out MV_F32 or MV_F16 (each with its row pitch), in == out allowed.  An fp16
+ * output saturates and raises the overflow flag (mv_set_overflow_flag) where |value| does not fit. */
+int mv_dropout(const void* in, int in_dtype, int64_t ld_in, void* out, int out_dtype, int64_t ld_out, int rows, int cols,
+               const uint64_t* seed_dev, int site, uint32_t thr, float scale, void* stream);
 /* fp16 / fp32 in[rows, cols] (row pitch ld elements) times `mul` -> fp32 copy out[rows, cols] and / or
  * fp32 transpose out_t[cols, rows] with row pitch ld_t >= rows (either may be NULL).  The 32-bit formats (q_format TF32 / FP32) run
  * their contractions as kind::tf32 on K-major fp32 operands; this prepares dY^T / X^T for wgrad and

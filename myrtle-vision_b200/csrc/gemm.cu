@@ -66,6 +66,7 @@ struct GemmDev {
     int variant;                // CTA-pair kernel: compile-time epilogue variant (0 = generic), see gemm2_host
     float* colsum;              // CTA-pair kernel: fp32 [N] += column sums of the stored values (fused bias gradient)
     int* ovf;                   // overflow sink (mv_set_overflow_flag) or NULL
+    DropDev drop;               // dropout mask of the output (CTA-pair kernel, kDrop instantiations); seed NULL: off
 };
 
 __device__ __forceinline__ float sat16(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
@@ -634,7 +635,9 @@ __device__ __forceinline__ void stage_chunk(const EpiWarp& w, uint32_t taddr, ui
 // Fast path: the chunk lies inside [M, N], every pointer / pitch is vector-aligned (checked on the
 // host, GemmDev::variant) and the epilogue's shape is a compile-time choice, so the unrolled row
 // loop is a few instructions per 4 outputs.  kRes: 0 none, 1 residual[m, n], 2 residual[m % rows_per_img, n].
-template <int kOut, int kEpi, int kRes, int kQO, int kQR, bool kAcc, bool kCS = false>
+// kDrop: dropout after q_out (include/mv_b200.h "dropout mask"; the host guarantees N % 8 == 0, so the four columns of a
+// lane are one half of a Philox block and lanes 2k / 2k+1 share the block: drop_keep4_pair, rows 2j / 2j+1).
+template <int kOut, int kEpi, int kRes, int kQO, int kQR, bool kAcc, bool kCS = false, bool kDrop = false>
 __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, uint32_t taddr, uint32_t release,
                                           int mrow0, int nc0, const uint2* aux_pre = nullptr, const float4* res_pre = nullptr) {
     const int n = nc0 + w.lc;
@@ -657,6 +660,16 @@ __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, ui
     }
     float4 b4 = make_float4(0.f, 0.f, 0.f, 0.f);
     if (!kAcc && p.bias != nullptr) b4 = __ldg(reinterpret_cast<const float4*>(p.bias + n));
+    uint32_t keep = 0;                                 // bit 4 * it + j: row m_first + 4 * it, column n + j is kept
+    if (kDrop) {
+        const uint64_t seed = __ldg(reinterpret_cast<const unsigned long long*>(p.drop.seed));
+        const bool odd = w.lane & 1;
+#pragma unroll
+        for (int it = 0; it < 8; it += 2) {
+            const uint64_t i = uint64_t(m_first + (it + (odd ? 1 : 0)) * 4) * uint64_t(p.N) + uint64_t(n);
+            keep |= drop_keep4_pair(seed, p.drop, i >> 3, odd) << (4 * it);
+        }
+    }
 #ifdef MV_GEMM_TRACE
     if (w.tr != nullptr && w.lane == 0) { w.tr[0] = 20; w.tr[1] = nc0; w.tr[2] = clock64(); }
 #endif
@@ -689,6 +702,13 @@ __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, ui
             float d[4];
             gelu_both2(v[0], v[1], v[0], v[1], d[0], d[1]);
             gelu_both2(v[2], v[3], v[2], v[3], d[2], d[3]);
+            if (kDrop) {
+#pragma unroll
+                for (int j = 0; j < 4; j++) {
+                    const float s = drop_mul(keep, 4 * it + j, p.drop.scale);
+                    v[j] *= s; d[j] *= s;
+                }
+            }
             *reinterpret_cast<uint2*>(p.aux + int64_t(m) * p.ld_aux + n) = pack4_f16_sat(d);
             if (kQR == 1 && kOut == MV_F16 && !kCS) {
                 // fc2's input quantiser: add half an fp16 ulp, convert with RZ (fq_half4_pack) — 1.5 instructions per value
@@ -700,6 +720,10 @@ __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, ui
             const __half2* hh = reinterpret_cast<const __half2*>(&aux2[it]);
             const float2 f0 = __half22float2(hh[0]), f1 = __half22float2(hh[1]);
             v[0] *= f0.x; v[1] *= f0.y; v[2] *= f1.x; v[3] *= f1.y;
+        }
+        if (kDrop && kEpi != MV_EPI_GELU) {
+#pragma unroll
+            for (int j = 0; j < 4; j++) v[j] *= drop_mul(keep, 4 * it + j, p.drop.scale);
         }
         if (kRes != 0) { v[0] += res4[it].x; v[1] += res4[it].y; v[2] += res4[it].z; v[3] += res4[it].w; }
         if (kQR == 1) fq_half4<kOut == MV_F16>(v);
@@ -796,6 +820,8 @@ __device__ __forceinline__ void epi_chunk_acc_t(const GemmDev& p, const EpiWarp&
 }
 
 // Generic path: tails in M / N, unaligned pitches, bf16 / second outputs.  Same arithmetic, rolled loops.
+// kDrop: the dropout mask element by element (any N).
+template <bool kDrop = false>
 __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWarp& w, uint32_t taddr, uint32_t release,
                                                int mrow0, int nc0) {
     stage_chunk(w, taddr, release);
@@ -818,17 +844,27 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
             }
             if (p.bias != nullptr) for (int j = 0; j < 4; j++) if (j < nvalid) v[j] += __ldg(p.bias + n + j);
             if (w.mode_out) for (int j = 0; j < 4; j++) v[j] = fq_apply(v[j], w.mode_out, p.q_out);
+            float dm[4] = {1.f, 1.f, 1.f, 1.f};
+            if (kDrop) {
+                const uint64_t seed = __ldg(reinterpret_cast<const unsigned long long*>(p.drop.seed));
+                for (int j = 0; j < 4; j++)
+                    if (j < nvalid)
+                        dm[j] = philox_half16(seed, uint64_t(m) * uint64_t(p.N) + uint64_t(n + j), uint64_t(uint32_t(p.drop.site))) >= p.drop.thr
+                                    ? p.drop.scale : 0.f;
+            }
             if (p.epilogue == MV_EPI_GELU) {
                 __half* up = p.aux + int64_t(m) * p.ld_aux + n;
                 for (int j = 0; j < 4; j++) {
                     float d;
                     gelu_both(v[j], v[j], d);
+                    if (kDrop) { v[j] *= dm[j]; d *= dm[j]; }
                     if (j < nvalid) up[j] = __float2half_rn(d);
                 }
             } else if (p.epilogue == MV_EPI_DGELU) {
                 const __half* up = p.aux + int64_t(m) * p.ld_aux + n;
                 for (int j = 0; j < 4; j++) if (j < nvalid) v[j] *= __half2float(up[j]);
             }
+            if (kDrop && p.epilogue != MV_EPI_GELU) for (int j = 0; j < 4; j++) v[j] *= dm[j];
             if (p.residual != nullptr) {
                 const int64_t rrow = p.rows_per_img > 0 ? (m % p.rows_per_img) : m;
                 const float* rp = p.residual + rrow * p.ld_res + n;
@@ -847,7 +883,9 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
     __syncwarp();
 }
 
-template <int BN, int EW, int AUX = 0>
+// kDrop: the dropout instantiations (variants 3, 4, 5, 9 and the generic path with the mask).  Separate kernels so that
+// the register allocation of the kernels without dropout — the maximum over every epilogue a kernel contains — stays as it is.
+template <int BN, int EW, int AUX = 0, bool kDrop = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 32 * EW, 1)
 gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
              const __grid_constant__ CUtensorMap tmap_aux, const __grid_constant__ GemmDev p) {
@@ -1020,7 +1058,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                             if (lane == 0) tma_store_wait_read();
                             __syncwarp();
                         }
-                        epi_chunk_generic(p, w, taddr, release, mrow0, nc0);
+                        epi_chunk_generic<kDrop>(p, w, taddr, release, mrow0, nc0);
                     }
                 }
                 GEMM_TRACE(lane == 0 && (warp == 2 || warp == 17), warp == 2 ? 1 : 2, 7, u);    // this warp's chunks done
@@ -1074,12 +1112,39 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                     if (c + kStep < BN / 32) request(u, c + kStep);
                     else if (u + unit_stride < total_units) request(u + unit_stride, cg);
                     if (fast) chunk(taddr, release, mrow0, nc0, aux2, res4);
-                    else epi_chunk_generic(p, w, taddr, release, mrow0, nc0);
+                    else epi_chunk_generic<kDrop>(p, w, taddr, release, mrow0, nc0);
                 }
                 if (++acc == kAccBufs) { acc = 0; acc_phase ^= 1; }
             }
         };
-        if constexpr (AUX == 1) {
+        if constexpr (kDrop && AUX == 2) {
+            if (p.variant == 4)
+                walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2*, const float4* res4) {
+                    epi_chunk<MV_F32, MV_EPI_NONE, 1, 1, 1, false, false, true>(p, w, taddr, release, mrow0, nc0, nullptr, res4);
+                });
+            else
+                walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2*, const float4* res4) {
+                    epi_chunk<MV_F32, MV_EPI_NONE, 1, 0, 0, false, false, true>(p, w, taddr, release, mrow0, nc0, nullptr, res4);
+                });
+        } else if constexpr (kDrop) {
+#define MV_EPI_DROP_CASE(id, ...)                                                                              \
+    case id:                                                                                                   \
+        walk([&](uint32_t taddr, uint32_t release, int mrow0, int nc0) {                                       \
+            epi_chunk<__VA_ARGS__, false, true>(p, w, taddr, release, mrow0, nc0);                             \
+        });                                                                                                    \
+        break;
+            switch (p.variant) {
+                //                   out     epilogue      res qo qr acc
+                MV_EPI_DROP_CASE(3, MV_F32, MV_EPI_NONE, 1, 0, 0, false)
+                MV_EPI_DROP_CASE(4, MV_F32, MV_EPI_NONE, 1, 1, 1, false)
+                MV_EPI_DROP_CASE(5, MV_F16, MV_EPI_GELU, 0, 0, 1, false)
+                MV_EPI_DROP_CASE(9, MV_F16, MV_EPI_GELU, 0, 1, 1, false)
+                default:   // every chunk takes the generic path with the mask
+                    walk([&](uint32_t, uint32_t, int, int) {});
+                    break;
+            }
+#undef MV_EPI_DROP_CASE
+        } else if constexpr (AUX == 1) {
             if (p.variant == 11)
                 walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2* aux2, const float4*) {
                     epi_chunk<MV_F16, MV_EPI_DGELU, 0, 0, 0, false, true>(p, w, taddr, release, mrow0, nc0, aux2);
@@ -1146,16 +1211,16 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
     }
 }
 
-template <int BN, int EW, int AUX = 0>
+template <int BN, int EW, int AUX = 0, bool kDrop = false>
 static int launch_gemm2(const CUtensorMap& ta, const CUtensorMap& tb, const GemmDev& p, int grid, cudaStream_t st,
                         const CUtensorMap* taux = nullptr) {
     using Cfg = Gemm2Cfg<BN, EW, AUX>;
     static bool attr_done = false;
     if (!attr_done) {
-        MV_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, EW, AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, EW, AUX, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
         attr_done = true;
     }
-    gemm2_kernel<BN, EW, AUX><<<grid, Cfg::kThreads, Cfg::kSmem, st>>>(ta, tb, taux != nullptr ? *taux : ta, p);
+    gemm2_kernel<BN, EW, AUX, kDrop><<<grid, Cfg::kThreads, Cfg::kSmem, st>>>(ta, tb, taux != nullptr ? *taux : ta, p);
     return 0;
 }
 
@@ -1226,6 +1291,11 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     p.rows_per_img = a->rows_per_img;
     p.colsum = a->accumulate ? nullptr : a->colsum;
     p.ovf = g_overflow;
+    const bool drop = a->drop_seed != nullptr;
+    MV_CHECK(!drop || (!a->accumulate && a->colsum == nullptr && a->out2 == nullptr),
+             "mv_gemm: dropout needs a plain output (no accumulate, colsum or out2)");
+    MV_CHECK(!drop || a->epilogue != MV_EPI_DGELU, "mv_gemm: the gelu' epilogue takes its mask from aux, not from drop_seed");
+    p.drop = DropDev{a->drop_seed, a->drop_thr, a->drop_scale, a->drop_site};
     // epilogue variant (epi_chunk<> instantiations in gemm2_kernel); anything else runs the generic path
     {
         auto al = [](const void* q, int bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) == 0; };
@@ -1249,6 +1319,9 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
         else if (ok)
             for (const Row& r : table)
                 if (r.out == a->out_dtype && r.epi == a->epilogue && r.res == res && r.qo == qo && r.qr == qr && r.cs == cs) v = r.id;
+        // the dropout kernels have compile-time epilogues for the residual and GELU variants; a lane's four columns must be
+        // half a Philox block (N % 8 == 0, epi_chunk), everything else takes the generic path with the mask
+        if (drop && !((v == 3 || v == 4 || v == 5 || v == 9) && a->N % 8 == 0)) v = 0;
         p.variant = v;
     }
 
@@ -1273,7 +1346,12 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     const bool out_tma = !heavy && (BN == 192 || BN == 128) && (p.variant == 1 || p.variant == 2) && (a->ld_out & 7) == 0 &&
                          (reinterpret_cast<uintptr_t>(a->out) & 15) == 0;
     if (out_tma && make_tmap_2d_plain(&taux, a->out, MV_F16, a->M, a->N, a->ld_out, 32, 32, 1)) return 1;
-    if (BN == 384) rc = launch_gemm2<384, 12>(ta, tb, p, grid, st);
+    if (drop) {
+        if (res_tma) rc = launch_gemm2<192, 12, 2, true>(ta, tb, p, grid, st, &taux);
+        else if (BN == 256) rc = heavy ? launch_gemm2<256, 16, 0, true>(ta, tb, p, grid, st) : launch_gemm2<256, 12, 0, true>(ta, tb, p, grid, st);
+        else if (BN == 192) rc = launch_gemm2<192, 12, 0, true>(ta, tb, p, grid, st);
+        else rc = launch_gemm2<128, 12, 0, true>(ta, tb, p, grid, st);
+    } else if (BN == 384) rc = launch_gemm2<384, 12>(ta, tb, p, grid, st);
     else if (out_tma) rc = BN == 192 ? launch_gemm2<192, 12, 3>(ta, tb, p, grid, st, &taux) : launch_gemm2<128, 12, 3>(ta, tb, p, grid, st, &taux);
     else if (aux_tma) rc = launch_gemm2<256, 16, 1>(ta, tb, p, grid, st, &taux);
     else if (res_tma) rc = launch_gemm2<192, 12, 2>(ta, tb, p, grid, st, &taux);
@@ -1297,6 +1375,8 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     if (a->epilogue == MV_EPI_GELU || a->epilogue == MV_EPI_DGELU) MV_CHECK(a->aux != nullptr, "mv_gemm: GELU epilogues need aux");
     if (!tf32 && a->cluster == 0) return gemm2_host(a, stream);      // CTA-pair kernel (default)
     MV_CHECK(a->colsum == nullptr, "mv_gemm: colsum is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
+    MV_CHECK(a->drop_seed == nullptr, "mv_gemm: dropout is only fused into the CTA-pair kernel (16-bit operands, cluster == 0); "
+                                      "apply mv_dropout to the output instead");
     const int esz = tf32 ? 4 : 2;
     const int BK = 128 / esz;
     static bool attr_done = false;
@@ -1348,6 +1428,7 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     p.accumulate = a->accumulate;
     p.rows_per_img = a->rows_per_img;
     p.variant = 0; p.colsum = nullptr; p.idesc2 = 0; p.transpose_out = 0; p.ovf = g_overflow;
+    p.drop = DropDev{nullptr, 0u, 0.f, 0};
 
     // CTA pairs sharing B through TMA multicast: measured no faster on B200 (the bound is the per-SM
     // L2->SM ingest, which multicast does not reduce), so it is opt-in (cluster == 2)

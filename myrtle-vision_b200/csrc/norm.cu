@@ -164,14 +164,19 @@ __device__ __forceinline__ float4 unpack_dy(const uint2& u) {
 
 // kGQ: the gradient quantiser of the LayerNorm's input stub (QPyTorch backward_number; mv_set_grad_format) rounds the
 // LayerNorm-input gradient before the residual gradient is added to it
-template <int NV, typename DyT, bool kGQ = false>
+// kDrop: dropout mask `drop` on dx_lp and dbias_prev (and on dx when mask_dx): the gradient of the dropped branch that the
+// residual stream's producer receives.  A lane owns float4 c = lane + 32 i; with D % 8 == 0 lanes 2k / 2k+1 hold the two
+// halves of one Philox block, so vectors i and i+1 take one call per lane (drop_keep4_pair).  Separate instantiations:
+// the kernels without it keep their register allocation.
+template <int NV, typename DyT, bool kGQ = false, bool kDrop = false>
 __global__ void __launch_bounds__(kLnWarps * 32, 2)
 ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ld_x,
               const float* __restrict__ dres, int64_t ld_dres, const float* __restrict__ gamma,
               const float* __restrict__ mean_in, const float* __restrict__ rstd_in,
               float* __restrict__ dx, int64_t ld_dx, __half* __restrict__ dx_lp, int64_t ld_lp,
               float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ dbias_prev,
-              int rows, int D, FloatFmt q_in, int* __restrict__ ovf, FloatFmt q_grad = FloatFmt{0, 0}) {
+              int rows, int D, FloatFmt q_in, int* __restrict__ ovf, FloatFmt q_grad = FloatFmt{0, 0},
+              DropDev drop = DropDev{nullptr, 0u, 0.f, 0}, int mask_dx = 0) {
     // Column sums (dgamma, dbeta, previous bias grad) are kept per warp in shared memory — each
     // lane owns its columns, so plain read-modify-write — which frees ~36 registers per thread for
     // occupancy; the next row's loads are issued before the current row is reduced.
@@ -205,6 +210,7 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
         }
     };
     int row = blockIdx.x * kLnWarps + warp;
+    const uint64_t seed = kDrop ? __ldg(reinterpret_cast<const unsigned long long*>(drop.seed)) : 0ull;
     LnBwdRow<NV, DyT> cur;
     float amax = 0.f;                   // largest |dx| rounded into the fp16 operand copy (overflow sink)
     if (row < rows) load_row(row, cur);
@@ -251,6 +257,21 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
         // dx = rstd * (gy - mean(gy) - xhat * mean(gy * xhat))  as two FMAs per value
         const float cb = -rstd * (s2 * inv_d), cc = -rstd * (s1 * inv_d);
         float* dxr = dx + int64_t(row) * ld_dx;
+        uint32_t keep = 0;                  // bits 4 i .. 4 i + 3: the four columns of float4 i
+        if (kDrop) {
+            const bool odd = lane & 1;
+            const uint64_t rbase = uint64_t(row) * uint64_t(D);
+#pragma unroll
+            for (int i = 0; i < NV; i += 2) {
+                if (i + 1 < NV && (D & 7) == 0) {
+                    const uint64_t e = rbase + 4ull * uint64_t(lane + 32 * (i + (odd ? 1 : 0)));
+                    keep |= drop_keep4_pair(seed, drop, e >> 3, odd) << (4 * i);
+                } else {
+                    keep |= drop_keep4(seed, drop, rbase + 4ull * uint64_t(lane + 32 * i)) << (4 * i);
+                    if (i + 1 < NV) keep |= drop_keep4(seed, drop, rbase + 4ull * uint64_t(lane + 32 * (i + 1))) << (4 * (i + 1));
+                }
+            }
+        }
 #pragma unroll
         for (int i = 0; i < NV; i++) {
             const int c = lane + 32 * i;
@@ -266,14 +287,20 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
                     const float4 r = cur.dres[i];
                     o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w;
                 }
+                float4 om = o;              // what the dropped branch receives
+                if (kDrop) {
+                    om.x *= drop_mul(keep, 4 * i, drop.scale); om.y *= drop_mul(keep, 4 * i + 1, drop.scale);
+                    om.z *= drop_mul(keep, 4 * i + 2, drop.scale); om.w *= drop_mul(keep, 4 * i + 3, drop.scale);
+                    if (mask_dx) o = om;
+                }
                 float4 ps = acc[2 * nvec + c];
-                ps.x += o.x; ps.y += o.y; ps.z += o.z; ps.w += o.w;
+                ps.x += om.x; ps.y += om.y; ps.z += om.z; ps.w += om.w;
                 acc[2 * nvec + c] = ps;
                 __stcs(reinterpret_cast<float4*>(dxr) + c, o);
                 if (dx_lp != nullptr) {
-                    amax = fmaxf(amax, fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fmaxf(fabsf(o.z), fabsf(o.w))));
+                    amax = fmaxf(amax, fmaxf(fmaxf(fabsf(om.x), fabsf(om.y)), fmaxf(fabsf(om.z), fabsf(om.w))));
                     __stcs(reinterpret_cast<uint2*>(dx_lp + int64_t(row) * ld_lp) + c,
-                           make_uint2(pack_h2_sat(o.x, o.y), pack_h2_sat(o.z, o.w)));
+                           make_uint2(pack_h2_sat(om.x, om.y), pack_h2_sat(om.z, om.w)));
                 }
             }
         }
@@ -499,11 +526,32 @@ template <int NV>
 static int launch_ln_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
                          int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
                          float* dx, int64_t ld_dx, void* dx_lp, int64_t ld_lp, float* dgamma, float* dbeta,
-                         float* dbias_prev, int rows, int D, FloatFmt q_in, cudaStream_t st) {
+                         float* dbias_prev, int rows, int D, FloatFmt q_in, cudaStream_t st,
+                         const DropDev* drop = nullptr, int mask_dx = 0) {
     int grid = (rows + kLnWarps - 1) / kLnWarps;
     const int cap = persistent_sms() * 2;
     if (grid > cap) grid = cap;
     const size_t smem = size_t(kLnWarps) * 3 * D * sizeof(float);
+    if (drop != nullptr) {
+        // dropout variants: fp16 dy (the dgrad GEMM's output), with or without the gradient quantiser
+        static bool attr_drop = false;
+        if (!attr_drop) {
+            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
+            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
+            attr_drop = true;
+        }
+        if (dy_dtype != MV_F16) { set_error("mv_layernorm_q_bwd_drop: dy must be fp16"); return 1; }
+        if (g_grad_fmt.exp_bits != 0)
+            ln_bwd_kernel<NV, __half, true, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
+                                                                                   dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
+                                                                                   q_in, g_overflow, g_grad_fmt, *drop, mask_dx);
+        else
+            ln_bwd_kernel<NV, __half, false, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
+                                                                                    dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
+                                                                                    q_in, g_overflow, FloatFmt{0, 0}, *drop, mask_dx);
+        g_launches++;
+        return check_cuda(cudaGetLastError(), "ln bwd (dropout) launch");
+    }
     static bool attr_done = false;
     if (!attr_done) {
         cudaFuncSetAttribute(ln_bwd_kernel<NV, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
@@ -527,6 +575,70 @@ static int launch_ln_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const floa
                                                                    (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D, q_in, g_overflow);
     g_launches++;
     return check_cuda(cudaGetLastError(), "ln bwd launch");
+}
+
+// mv_dropout: out = in * keep * scale over [rows, cols] with row pitches.  A thread takes eight consecutive elements of
+// the flat (pitch-free) index, i.e. one Philox block; with cols, both pitches and both bases multiples of eight elements /
+// 16 bytes it moves them as 16-byte vectors, otherwise element by element.
+__device__ __forceinline__ float ld_elem(const float* p) { return *p; }
+__device__ __forceinline__ float ld_elem(const __half* p) { return __half2float(*p); }
+__device__ __forceinline__ void st_elem(float* p, float v) { *p = v; }
+__device__ __forceinline__ void st_elem(__half* p, float v) { *p = __float2half_rn(sat16(v)); }
+__device__ __forceinline__ void ld8(const float* p, float (&v)[8]) {
+    const float4 a = __ldcs(reinterpret_cast<const float4*>(p)), b = __ldcs(reinterpret_cast<const float4*>(p) + 1);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void ld8(const __half* p, float (&v)[8]) {
+    const uint4 u = __ldcs(reinterpret_cast<const uint4*>(p));
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w[j]));
+        v[2 * j] = f.x; v[2 * j + 1] = f.y;
+    }
+}
+__device__ __forceinline__ void st8(float* p, const float (&v)[8]) {
+    reinterpret_cast<float4*>(p)[0] = make_float4(v[0], v[1], v[2], v[3]);
+    reinterpret_cast<float4*>(p)[1] = make_float4(v[4], v[5], v[6], v[7]);
+}
+__device__ __forceinline__ void st8(__half* p, const float (&v)[8]) {
+    *reinterpret_cast<uint4*>(p) = make_uint4(pack_h2_sat(v[0], v[1]), pack_h2_sat(v[2], v[3]), pack_h2_sat(v[4], v[5]),
+                                              pack_h2_sat(v[6], v[7]));
+}
+template <typename InT, typename OutT>
+__global__ void __launch_bounds__(256)
+dropout_kernel(const InT* in, int64_t ld_in, OutT* out, int64_t ld_out, int rows, int cols, DropDev d, int vec,
+               int* __restrict__ ovf) {
+    const uint64_t seed = __ldg(reinterpret_cast<const unsigned long long*>(d.seed));
+    const uint64_t n = uint64_t(rows) * uint64_t(cols), blocks = (n + 7) >> 3;
+    float amax = 0.f;
+    for (uint64_t g = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x; g < blocks; g += uint64_t(gridDim.x) * blockDim.x) {
+        const uint4 w = philox4x32_10(seed, g, uint64_t(uint32_t(d.site)));
+        const uint32_t ws[4] = {w.x, w.y, w.z, w.w};
+        float v[8];
+        if (vec) {
+            const uint64_t r = (g * 8) / uint64_t(cols), c = (g * 8) % uint64_t(cols);
+            ld8(in + r * ld_in + c, v);
+#pragma unroll
+            for (int j = 0; j < 8; j++) {
+                const uint32_t h = (j & 1) ? (ws[j >> 1] >> 16) : (ws[j >> 1] & 0xFFFFu);
+                v[j] *= h >= d.thr ? d.scale : 0.f;
+                amax = fmaxf(amax, fabsf(v[j]));
+            }
+            st8(out + r * ld_out + c, v);
+        } else {
+            for (int j = 0; j < 8; j++) {
+                const uint64_t i = g * 8 + j;
+                if (i >= n) break;
+                const uint64_t r = i / uint64_t(cols), c = i % uint64_t(cols);
+                const uint32_t h = (j & 1) ? (ws[j >> 1] >> 16) : (ws[j >> 1] & 0xFFFFu);
+                const float x = ld_elem(in + r * ld_in + c) * (h >= d.thr ? d.scale : 0.f);
+                amax = fmaxf(amax, fabsf(x));
+                st_elem(out + r * ld_out + c, x);
+            }
+        }
+    }
+    if (sizeof(OutT) == 2) raise_overflow(ovf, amax);
 }
 
 // fp16 / fp32 [rows, cols] (row pitch ld) -> fp32 copy and / or fp32 transpose [cols, rows], 32x32 tiles
@@ -619,6 +731,61 @@ extern "C" int mv_layernorm_q_bwd(const void* dy, int dy_dtype, int64_t ld_dy, c
         case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
         default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
     }
+}
+
+extern "C" int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x,
+                                       const float* dres, int64_t ld_dres, const float* gamma, const float* mean,
+                                       const float* rstd, float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp,
+                                       float* dgamma, float* dbeta, float* dbias_prev, int rows, int D,
+                                       int q_in_exp, int q_in_man, const uint64_t* seed_dev, int site, uint32_t thr,
+                                       float scale, int mask_dx, void* stream) {
+    if (seed_dev == nullptr)
+        return mv_layernorm_q_bwd(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp,
+                                  dgamma, dbeta, dbias_prev, rows, D, q_in_exp, q_in_man, stream);
+    MV_CHECK(rows >= 0 && D > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd_drop: D=%d unsupported", D);
+    MV_CHECK(ld_dy % 4 == 0 && ld_x % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_lp % 4 == 0, "mv_layernorm_q_bwd_drop: row pitches must be multiples of 4");
+    MV_CHECK(thr <= 65536u, "mv_layernorm_q_bwd_drop: threshold %u above 65536", thr);
+    if (rows == 0) return 0;
+    const FloatFmt qi{q_in_exp, q_in_man};
+    const DropDev d{seed_dev, thr, scale, site};
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int nv = (D / 4 + 31) / 32;
+    switch (nv) {
+        case 1: return launch_ln_bwd<1>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+        case 2: return launch_ln_bwd<2>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+        case 3: return launch_ln_bwd<3>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+        case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+        case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+        default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+    }
+}
+
+extern "C" int mv_dropout(const void* in, int in_dtype, int64_t ld_in, void* out, int out_dtype, int64_t ld_out, int rows,
+                          int cols, const uint64_t* seed_dev, int site, uint32_t thr, float scale, void* stream) {
+    MV_CHECK(in && out && seed_dev, "mv_dropout: null pointer");
+    MV_CHECK(rows >= 0 && cols > 0 && ld_in >= cols && ld_out >= cols, "mv_dropout: bad shape %d x %d (pitches %lld, %lld)", rows, cols,
+             (long long)ld_in, (long long)ld_out);
+    MV_CHECK((in_dtype == MV_F32 || in_dtype == MV_F16) && (out_dtype == MV_F32 || out_dtype == MV_F16), "mv_dropout: fp32 or fp16 only");
+    MV_CHECK(thr <= 65536u, "mv_dropout: threshold %u above 65536", thr);
+    MV_CHECK(in != out || (in_dtype == out_dtype && ld_in == ld_out), "mv_dropout: in place needs one dtype and one pitch");
+    if (rows == 0) return 0;
+    const DropDev d{seed_dev, thr, scale, site};
+    const uint64_t blocks8 = (uint64_t(rows) * uint64_t(cols) + 7) / 8;
+    const int vec = cols % 8 == 0 && ld_in % 8 == 0 && ld_out % 8 == 0 && reinterpret_cast<uintptr_t>(in) % 16 == 0 &&
+                    reinterpret_cast<uintptr_t>(out) % 16 == 0;
+    int64_t grid = int64_t((blocks8 + 255) / 256);
+    if (grid > kNumSMs * 8) grid = kNumSMs * 8;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (in_dtype == MV_F32 && out_dtype == MV_F32)
+        dropout_kernel<float, float><<<int(grid), 256, 0, st>>>((const float*)in, ld_in, (float*)out, ld_out, rows, cols, d, vec, g_overflow);
+    else if (in_dtype == MV_F32)
+        dropout_kernel<float, __half><<<int(grid), 256, 0, st>>>((const float*)in, ld_in, (__half*)out, ld_out, rows, cols, d, vec, g_overflow);
+    else if (out_dtype == MV_F32)
+        dropout_kernel<__half, float><<<int(grid), 256, 0, st>>>((const __half*)in, ld_in, (float*)out, ld_out, rows, cols, d, vec, g_overflow);
+    else
+        dropout_kernel<__half, __half><<<int(grid), 256, 0, st>>>((const __half*)in, ld_in, (__half*)out, ld_out, rows, cols, d, vec, g_overflow);
+    g_launches++;
+    return check_cuda(cudaGetLastError(), "dropout launch");
 }
 
 extern "C" int mv_colsum(const void* in, int in_dtype, int64_t ld, int rows, int cols, float* out, void* stream) {

@@ -174,6 +174,38 @@ __device__ __forceinline__ uint32_t philox_half16(uint64_t seed, uint64_t i, uin
     const uint32_t word = ws[(i & 7) >> 1];
     return (i & 1) ? (word >> 16) : (word & 0xFFFFu);
 }
+
+// ---- dropout mask (include/mv_b200.h "dropout mask"): keep(i) = bits16(seed, site, i) >= thr ----
+struct DropDev {
+    const uint64_t* seed;       // device pointer; NULL: off
+    uint32_t thr;
+    float scale;
+    int site;
+};
+// keep bits of elements i .. i+3 (i % 4 == 0: one half of a Philox block) from that half's two words: bit j = element i+j
+__device__ __forceinline__ uint32_t drop_bits4(uint2 h, uint32_t thr) {
+    return uint32_t((h.x & 0xFFFFu) >= thr) | (uint32_t((h.x >> 16) >= thr) << 1) |
+           (uint32_t((h.y & 0xFFFFu) >= thr) << 2) | (uint32_t((h.y >> 16) >= thr) << 3);
+}
+// the half of element i's Philox block that holds i .. i+3 (i % 4 == 0), computed by this lane alone
+__device__ __forceinline__ uint32_t drop_keep4(uint64_t seed, const DropDev& d, uint64_t i) {
+    const uint4 w = philox4x32_10(seed, i >> 3, uint64_t(uint32_t(d.site)));
+    return drop_bits4((i & 4) ? make_uint2(w.z, w.w) : make_uint2(w.x, w.y), d.thr);
+}
+// One Philox call serves eight elements, i.e. two lanes that own four each.  Lanes 2k and 2k+1 each need their half of two
+// blocks A and B (the even lane elements 0..3 of a block, the odd lane 4..7): the even lane computes A, the odd lane B
+// (`ctr` = that block's counter), and each hands the other the half it needs — one call per lane instead of two.
+// Returns the keep bits of this lane's half of A (bits 0..3) and of B (bits 4..7).
+__device__ __forceinline__ uint32_t drop_keep4_pair(uint64_t seed, const DropDev& d, uint64_t ctr, bool odd) {
+    const uint4 w = philox4x32_10(seed, ctr, uint64_t(uint32_t(d.site)));
+    const uint2 mine = odd ? make_uint2(w.z, w.w) : make_uint2(w.x, w.y);
+    const uint2 give = odd ? make_uint2(w.x, w.y) : make_uint2(w.z, w.w);
+    const uint2 got = make_uint2(__shfl_xor_sync(0xffffffffu, give.x, 1), __shfl_xor_sync(0xffffffffu, give.y, 1));
+    const uint32_t a = drop_bits4(odd ? got : mine, d.thr), b = drop_bits4(odd ? mine : got, d.thr);
+    return a | (b << 4);
+}
+__device__ __forceinline__ float drop_mul(uint32_t bits, int j, float scale) { return ((bits >> j) & 1u) ? scale : 0.f; }
+
 __device__ __forceinline__ float bits_to_uniform(uint32_t b) {
     return float(b >> 8) * (1.0f / 16777216.0f);
 }

@@ -14,6 +14,11 @@ backward, with the fake-quantisers of SURVEY.md Appendix A folded into the neigh
     xn2  = H(LN(H(x1)))                                  mv_layernorm_q_fwd      -> fp16
     u,h  = o(xn2 . H(W1)^T + b),  H(gelu(u))             mv_gemm (GELU epilogue) -> fp16, fp16
     x2   = f(o(h . H(W2)^T + b) + x1)                    mv_gemm (+residual)     -> fp32
+  dropout (EngineConfig.dropout / emb_dropout, training forwards only): D(y) = y * keep * s with the mask stream of
+  include/mv_b200.h, fused where the tensor is produced — x0 = D_emb(embedding) (mv_dropout after mv_cls_rows),
+  x1 = f(D(o(att . Wo^T + b)) + x) and x2 = f(D(o(h . W2^T + b)) + x1) in the residual epilogues, h = H(D(gelu(u)))
+  with the saved gelu'(u) masked alike; the backward masks the gradient entering each dropped branch where the
+  LayerNorm backward writes its fp16 operand copy and bias column sums.
   backward: straight-through quantisers (utils/quantize.py:87-89); dgrad / wgrad on the same GEMM
   kernel (wgrad reads dY and X in place as MN-major operands, split-K red.add into a flat fp32
   gradient buffer), GELU' in the dgrad epilogue, LN backward fused with the residual-gradient add,
@@ -52,12 +57,38 @@ class _Range:
 
 
 class EngineConfig:
-    def __init__(self, dim, heads, mlp_dim, depth, patch, plan):
+    def __init__(self, dim, heads, mlp_dim, depth, patch, plan, dropout=0.0, emb_dropout=0.0):
         self.dim, self.heads, self.mlp_dim, self.depth, self.patch, self.plan = (
             dim, heads, mlp_dim, depth, patch, plan)
+        mv.drop_params(dropout), mv.drop_params(emb_dropout)        # ValueError outside [0, 1], as nn.Dropout
+        self.dropout, self.emb_dropout = float(dropout), float(emb_dropout)
 
 
 PER_LAYER = 12   # ln1.w ln1.b qkv.w qkv.b out.w out.b ln2.w ln2.b fc1.w fc1.b fc2.w fc2.b
+
+
+class _Drops:
+    """The dropout sites of one training forward and its backward: site ids of include/mv_b200.h ("dropout mask") and
+    the seed tensor drawn for that forward.  Each method returns the `drop` argument of the mv_native calls, or None
+    where the probability is 0 (the site is the identity and runs no mask code)."""
+
+    def __init__(self, cfg, seed):
+        self.p, self.pe, self.depth, self.seed = cfg.dropout, cfg.emb_dropout, cfg.depth, seed
+
+    def _site(self, p, site):
+        return (self.seed, p, site) if p > 0.0 else None
+
+    def proj(self, l):
+        return self._site(self.p, 3 * l)
+
+    def fc1(self, l):
+        return self._site(self.p, 3 * l + 1)
+
+    def fc2(self, l):
+        return self._site(self.p, 3 * l + 2)
+
+    def emb(self):
+        return self._site(self.pe, 3 * self.depth)
 
 
 class EncoderEngine:
@@ -119,6 +150,13 @@ class EncoderEngine:
         # True once an optimizer (utils/fused_adamw.FusedAdamW) emits q(W) / q(W)^T itself after every
         # update: a CUDA-graph capture then leaves the re-quantisation out of the graph
         self.external_requant = False
+        # nn.Module.training of the owning model (ViT.forward sets it): dropout acts in training forwards only
+        self.training = True
+        # seed of the last forward that applied dropout: int64 [1] on the device (its 64 bits are the Philox key)
+        self.last_dropout_seed = None
+        # None, or an int64 [1] device tensor that training forwards use instead of a fresh draw (reproduces the masks of
+        # an earlier step, e.g. one replayed from a CUDA graph, given its last_dropout_seed)
+        self.fixed_dropout_seed = None
 
     # ------------------------------------------------------------------ weights
     def _weight_indices(self):
@@ -230,14 +268,28 @@ class EncoderEngine:
         q, k = qkv.view(B, N, 3, H, 64).float().permute(2, 0, 3, 1, 4)[:2]
         m(torch.softmax(torch.matmul(q, k.transpose(-2, -1)) * 0.125, dim=-1))
 
+    def _draw_drops(self):
+        """A fresh seed per training forward with dropout, drawn on the device from torch's default CUDA generator: a
+        captured CUDA graph replays the draw with a new philox offset, so every replay gets new masks, and
+        torch.manual_seed makes runs repeatable.  None when dropout is off (no draw: the generator is not advanced)."""
+        cfg = self.cfg
+        if not self.training or (cfg.dropout == 0.0 and cfg.emb_dropout == 0.0):
+            return None
+        seed = self.fixed_dropout_seed
+        if seed is None:
+            seed = torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=self.dev)
+        self.last_dropout_seed = seed
+        return _Drops(cfg, seed)
+
     def forward(self, img, pos_full, cls_token, save):
         # a training forward opens an overflow window that its backward closes (mv_overflow_update); inference
         # forwards report nothing
         mv.set_overflow_flag(self.overflow if save else None)
         if save:
             self.overflow.zero_()
+        drops = self._draw_drops()
         if self.wide:
-            return self._forward_wide(img, pos_full, cls_token, save)
+            return self._forward_wide(img, pos_full, cls_token, save, drops)
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
@@ -255,8 +307,10 @@ class EncoderEngine:
             mv.gemm(patches, wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                     rows_per_img=N)
             mv.cls_rows(cls_token.detach().reshape(D).contiguous(), pos32, x, B, N, D, q_ff=plan.ff)
+            if drops and drops.emb():
+                mv.dropout(x, drops.emb(), out=x)
 
-        saved = {"B": B, "N": N, "patches": patches, "layers": []} if save else None
+        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops} if save else None
         with self._range("transformer"):
             for l in range(cfg.depth):
                 b0 = 2 + PER_LAYER * l
@@ -268,16 +322,16 @@ class EncoderEngine:
                     att, lse = mv.attention_fwd(qkv, B, H, N, scale=0.125, q_out=fmt)
                     x1 = torch.empty(M, D, dtype=torch.float32, device=dev)
                     mv.gemm(att, wq[b0 + 4][0], x1, bias=prm[b0 + 5], q_out=plan.out, residual=x,
-                            q_res=plan.ff)
+                            q_res=plan.ff, drop=drops and drops.proj(l))
                 with self._range("transformer:feedforward"):
                     xn2, mean2, rstd2 = mv.layernorm_q_fwd(x1, prm[b0 + 6], prm[b0 + 7], q_in=fmt, q_post=fmt)
                     u = torch.empty(M, Mm, dtype=f16, device=dev)
                     h = torch.empty(M, Mm, dtype=f16, device=dev)
                     mv.gemm(xn2, wq[b0 + 8][0], h, bias=prm[b0 + 9], q_out=plan.out, aux=u,
-                            epilogue=mv.EPI_GELU, q_res=fmt)
+                            epilogue=mv.EPI_GELU, q_res=fmt, drop=drops and drops.fc1(l))
                     x2 = torch.empty(M, D, dtype=torch.float32, device=dev)
                     mv.gemm(h, wq[b0 + 10][0], x2, bias=prm[b0 + 11], q_out=plan.out, residual=x1,
-                            q_res=plan.ff)
+                            q_res=plan.ff, drop=drops and drops.fc2(l))
                 if save:
                     saved["layers"].append((x, xn1, mean1, rstd1, qkv, att, lse, x1, xn2, mean2, rstd2, u, h))
                 x = x2
@@ -299,10 +353,21 @@ class EncoderEngine:
         # power-of-two gradient scale chosen on the device (no host sync)
         gx = gx.reshape(M, D)
         S = self._gradient_scale(gx)
-        dx, dx_h = mv.scale_f32(gx, S, want_f16=True)                             # fp32 master and fp16 operand in one pass
-        self.gflat.zero_()
+        drops = saved["drops"]
         last = cfg.depth - 1
-        mv.colsum(dx, g[2 + PER_LAYER * last + 11].view(-1))               # fc2 bias of the last block
+        if drops and drops.fc2(last):
+            # the last block's fc2 branch receives the masked gradient (its dgrad / wgrad operand and bias column sums);
+            # the residual stream keeps the unmasked fp32 one
+            dx, _ = mv.scale_f32(gx, S)
+            dxm = mv.dropout(dx, drops.fc2(last))
+            self.gflat.zero_()
+            mv.colsum(dxm, g[2 + PER_LAYER * last + 11].view(-1))
+            _, dx_h = mv.scale_f32(dxm, self._one(), want_f32=False, want_f16=True)
+            del dxm
+        else:
+            dx, dx_h = mv.scale_f32(gx, S, want_f16=True)                         # fp32 master and fp16 operand in one pass
+            self.gflat.zero_()
+            mv.colsum(dx, g[2 + PER_LAYER * last + 11].view(-1))           # fc2 bias of the last block
 
         # Gradient quantiser G (QuantPlan.grad, normally None): the backward of every QuantStub in front of a Linear is
         # the q_out of that Linear's dgrad GEMM (before the gelu' multiply for fc2's), of every stub in front of a
@@ -331,8 +396,10 @@ class EncoderEngine:
             mv.gemm(du, xn2, g[b0 + 8], a_major=1, b_major=1, accumulate=True)
             wq_grad(b0 + 8)
             del du
+            # dx1_h and to_out's bias gradient: the masked gradient of the to_out branch (dropout site of to_out)
             dx1, dx1_h = mv.layernorm_q_bwd(dxn2, x1, prm[b0 + 6], mean2, rstd2, dres=dx, q_in=fmt,
-                                            dgamma=g[b0 + 6], dbeta=g[b0 + 7], dbias_prev=g[b0 + 5])
+                                            dgamma=g[b0 + 6], dbeta=g[b0 + 7], dbias_prev=g[b0 + 5],
+                                            drop=drops and drops.proj(l))
             # ---- Attention
             datt = torch.empty(M, D, dtype=f16, device=dev)
             mv.gemm(dx1_h, wq[b0 + 4][1], datt, tag="dgrad", q_out=gq)
@@ -345,9 +412,12 @@ class EncoderEngine:
             mv.gemm(dqkv, xn1, g[b0 + 2], a_major=1, b_major=1, accumulate=True)
             wq_grad(b0 + 2)
             prev_bias = g[b0 - 1] if l > 0 else None                       # fc2 bias of block l-1
+            # dx_h (and prev_bias): masked with block l-1's fc2 site; below block 0 everything (dx too) with the embedding
+            # site — the patch wgrad, dpos / dcls and the patch bias all lie behind that dropout
+            drop = (drops.fc2(l - 1) if l > 0 else drops.emb()) if drops else None
             dx, dx_h = mv.layernorm_q_bwd(dxn1, x, prm[b0], mean1, rstd1, dres=dx1, q_in=fmt,
                                           dgamma=g[b0], dbeta=g[b0 + 1], dbias_prev=prev_bias,
-                                          dx=dx, dx_f16=dx_h)
+                                          dx=dx, dx_f16=dx_h, drop=drop, mask_dx=l == 0)
             if self.reducer is not None and l % self.bucket_blocks == 0:
                 # one all-reduce per bucket of `bucket_blocks` encoder blocks (their gradient slices are contiguous),
                 # issued as soon as the bucket's last wgrad is enqueued
@@ -402,7 +472,7 @@ class EncoderEngine:
     # wgrad therefore takes explicit transposes (mv_widen_transpose) instead of the in-place MN-major
     # reads of the 16-bit path.  Attention keeps the fp16 tcgen05 kernels: qkv / attention output /
     # their gradients carry 11 significant bits, the same as a tf32 operand.
-    def _forward_wide(self, img, pos_full, cls_token, save):
+    def _forward_wide(self, img, pos_full, cls_token, save, drops):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
@@ -421,8 +491,22 @@ class EncoderEngine:
         mv.gemm(A_(patches), wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                 rows_per_img=N)
         mv.cls_rows(cls_token.detach().reshape(D).contiguous(), pos32, x, B, N, D, q_ff=plan.ff)
+        if drops and drops.emb():
+            mv.dropout(x, drops.emb(), out=x)
 
-        saved = {"B": B, "N": N, "patches": patches, "layers": []} if save else None
+        def linear_res(a, w, bias, res, drop):
+            # x + D(Linear(a)): the single-CTA kind::tf32 kernel has no dropout epilogue, so the mask is a pass of its own
+            y = torch.empty(M, D, dtype=f32, device=dev)
+            if drop is None:
+                return mv.gemm(a, w, y, bias=bias, q_out=plan.out, residual=res, q_res=plan.ff)
+            mv.gemm(a, w, y, bias=bias, q_out=plan.out)
+            mv.dropout(y, drop, out=y)
+            y.add_(res)
+            if plan.ff:
+                mv.float_quantize(y, plan.ff[0], plan.ff[1], out=y)
+            return y
+
+        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops} if save else None
         for l in range(cfg.depth):
             b0 = 2 + PER_LAYER * l
             xn1, mean1, rstd1 = mv.layernorm_q_fwd(x, prm[b0], prm[b0 + 1], q_in=fmt, q_post=fmt,
@@ -436,21 +520,27 @@ class EncoderEngine:
             else:
                 att16, lse = mv.attention_fwd(qkv, B, H, N, scale=0.125, q_out=fmt)
                 att, _ = mv.widen_transpose(att16, want_copy=True, want_t=False)
-            x1 = torch.empty(M, D, dtype=f32, device=dev)
-            mv.gemm(A_(att), wq[b0 + 4][0], x1, bias=prm[b0 + 5], q_out=plan.out, residual=x, q_res=plan.ff)
+            x1 = linear_res(A_(att), wq[b0 + 4][0], prm[b0 + 5], x, drops and drops.proj(l))
             xn2, mean2, rstd2 = mv.layernorm_q_fwd(x1, prm[b0 + 6], prm[b0 + 7], q_in=fmt, q_post=fmt,
                                                    out_dtype=f32)
             h = torch.empty(M, Mm, dtype=f32, device=dev)
+            d1 = drops and drops.fc1(l)
             if ex:
                 gd = torch.empty(M, Mm, dtype=f32, device=dev)               # u (pre-GELU), fp32
                 mv.gemm(A_(xn2), wq[b0 + 8][0], gd, bias=prm[b0 + 9])
                 h = torch.nn.functional.gelu(gd)
+                if d1:
+                    mv.dropout(h, d1, out=h)
             else:
-                gd = torch.empty(M, Mm, dtype=f16, device=dev)               # gelu'(u)
+                # gelu'(u); with dropout the backward applies the mask after the gelu' multiply (mv_dropout on du)
+                gd = torch.empty(M, Mm, dtype=f16, device=dev)
                 mv.gemm(xn2, wq[b0 + 8][0], h, bias=prm[b0 + 9], q_out=plan.out, aux=gd,
-                        epilogue=mv.EPI_GELU, q_res=fmt)
-            x2 = torch.empty(M, D, dtype=f32, device=dev)
-            mv.gemm(A_(h), wq[b0 + 10][0], x2, bias=prm[b0 + 11], q_out=plan.out, residual=x1, q_res=plan.ff)
+                        epilogue=mv.EPI_GELU, q_res=None if d1 else fmt)
+                if d1:
+                    mv.dropout(h, d1, out=h)
+                    if fmt:
+                        mv.float_quantize(h, fmt[0], fmt[1], out=h)
+            x2 = linear_res(A_(h), wq[b0 + 10][0], prm[b0 + 11], x1, drops and drops.fc2(l))
             if save:
                 saved["layers"].append((x, xn1, mean1, rstd1, qkv, att16, lse, x1, xn2, mean2, rstd2, gd, h))
             x = x2
@@ -499,33 +589,49 @@ class EncoderEngine:
         dx, _ = mv.scale_f32(gx, S)
         self.gflat.zero_()
         last = cfg.depth - 1
-        mv.colsum(dx, g[2 + PER_LAYER * last + 11].view(-1))
+        drops = saved["drops"]
+        # with dropout each masked branch gradient is a pass of its own (mv_dropout) and its bias gradient a colsum of it
+        dropping = bool(drops and drops.p > 0.0)
+        if not dropping:
+            mv.colsum(dx, g[2 + PER_LAYER * last + 11].view(-1))
 
         for l in range(last, -1, -1):
             b0 = 2 + PER_LAYER * l
             x, xn1, mean1, rstd1, qkv, att16, lse, x1, xn2, mean2, rstd2, gd, h = saved["layers"][l]
             # ---- FeedForward
+            dxm = dx
+            if dropping:
+                dxm = mv.dropout(dx, drops.fc2(l))
+                mv.colsum(dxm, g[b0 + 11].view(-1))
             du = torch.empty(M, Mm, dtype=f32, device=dev)
             if ex:
-                mv.gemm(A_(dx), wq[b0 + 10][1], du)
+                mv.gemm(A_(dxm), wq[b0 + 10][1], du)
                 u = gd                                                       # gelu'(u) = Phi(u) + u phi(u)
                 du.mul_(0.5 * (1.0 + torch.erf(u * 0.7071067811865476))
                         + u * torch.exp(-0.5 * u * u) * 0.3989422804014327)
             else:
-                mv.gemm(dx, wq[b0 + 10][1], du, aux=gd, epilogue=mv.EPI_DGELU)
-            wgrad(dx, h, g[b0 + 10])
+                mv.gemm(dxm, wq[b0 + 10][1], du, aux=gd, epilogue=mv.EPI_DGELU)
+            if dropping:
+                mv.dropout(du, drops.fc1(l), out=du)
+            wgrad(dxm, h, g[b0 + 10])
+            del dxm
             dxn2 = torch.empty(M, D, dtype=f32, device=dev)
             mv.gemm(A_(du), wq[b0 + 8][1], dxn2, tag="dgrad")
             wgrad(du, xn2, g[b0 + 8])
             mv.colsum(du, g[b0 + 9].view(-1))
             del du
             dx1, _ = mv.layernorm_q_bwd(dxn2, x1, prm[b0 + 6], mean2, rstd2, dres=dx, q_in=fmt,
-                                        dgamma=g[b0 + 6], dbeta=g[b0 + 7], dbias_prev=g[b0 + 5],
-                                        want_f16=False)
+                                        dgamma=g[b0 + 6], dbeta=g[b0 + 7],
+                                        dbias_prev=None if dropping else g[b0 + 5], want_f16=False)
             # ---- Attention
+            dx1m = dx1
+            if dropping:
+                dx1m = mv.dropout(dx1, drops.proj(l))
+                mv.colsum(dx1m, g[b0 + 5].view(-1))
             datt = torch.empty(M, D, dtype=f32 if ex else f16, device=dev)
-            mv.gemm(A_(dx1), wq[b0 + 4][1], datt, tag="dgrad")
-            wgrad(dx1, att16, g[b0 + 4])
+            mv.gemm(A_(dx1m), wq[b0 + 4][1], datt, tag="dgrad")
+            wgrad(dx1m, att16, g[b0 + 4])
+            del dx1m
             if ex:
                 dqkv16 = dqkv = self._attention_exact_bwd(qkv, lse, datt, B, H, N)
                 _, dqkv_t = mv.widen_transpose(dqkv, padded=True)
@@ -540,7 +646,7 @@ class EncoderEngine:
             mv.gemm(dqkv_t, xn1_t, g[b0 + 2], accumulate=True)
             if ex:
                 mv.colsum(dqkv16, g[b0 + 3].view(-1))
-            prev_bias = g[b0 - 1] if l > 0 else None
+            prev_bias = g[b0 - 1] if l > 0 and not dropping else None
             dx, _ = mv.layernorm_q_bwd(dxn1, x, prm[b0], mean1, rstd1, dres=dx1, q_in=fmt,
                                        dgamma=g[b0], dbeta=g[b0 + 1], dbias_prev=prev_bias,
                                        want_f16=False, dx=dx)
@@ -550,6 +656,8 @@ class EncoderEngine:
                 top = min(cfg.depth, l + self.bucket_blocks)
                 lo, hi = self.offsets[b0], self.offsets[2 + PER_LAYER * top]
                 self.reducer.reduce_slice(self.gflat[lo:hi], 1.0 / S)
+        if drops and drops.emb():
+            mv.dropout(dx, drops.emb(), out=dx)
         wgrad(dx, saved["patches"], g[0])
         return self._finish_backward(dx, S, B, N, D)
 

@@ -6,6 +6,7 @@ missing or a call fails.  PyTorch is used only for device memory and streams.
 import ctypes
 import os
 
+import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -42,6 +43,8 @@ class GemmArgs(ctypes.Structure):
         ("colsum", ctypes.c_void_p),
         ("transpose_out", ctypes.c_int),
         ("cluster", ctypes.c_int),
+        ("drop_seed", ctypes.c_void_p), ("drop_thr", ctypes.c_uint32), ("drop_scale", ctypes.c_float),
+        ("drop_site", ctypes.c_int),
     ]
 
 
@@ -159,6 +162,42 @@ def launch_count():
     return int(lib().mv_launch_count())
 
 
+# ------------------------------------------------------------------ dropout
+def drop_params(p):
+    """(thr, scale) of nn.Dropout(p) in the mask stream of include/mv_b200.h: keep = bits16 >= thr with
+    thr = nearbyint(p * 65536), scale = 1 / (1 - p) in fp32 (0 for p == 1)."""
+    p = float(p)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError("dropout probability has to be between 0 and 1, but got %r" % (p,))
+    thr = int(round(p * 65536.0))                  # round half to even, as nearbyint
+    scale = 0.0 if p == 1.0 else float(np.float32(1.0) / np.float32(1.0 - p))
+    return thr, scale
+
+
+def _drop_args(drop):
+    """drop = (seed, p, site): seed a 1-element int64 CUDA tensor holding the 64-bit seed."""
+    seed, p, site = drop
+    _need_cuda(seed)
+    assert seed.dtype == torch.int64 and seed.numel() == 1
+    thr, scale = drop_params(p)
+    return ctypes.c_void_p(seed.data_ptr()), int(site), ctypes.c_uint32(thr), ctypes.c_float(scale)   # C argument order
+
+
+def dropout(x, drop, *, out=None, out_dtype=None, tag="dropout"):
+    """mv_dropout: out = x * keep * scale over a 2-D fp32 / fp16 tensor (row pitch honoured); out may be x."""
+    _need_cuda(x)
+    assert x.dim() == 2 and x.stride(1) == 1 and x.dtype in (torch.float32, torch.float16)
+    if out is None:
+        out = torch.empty(x.shape, dtype=out_dtype or x.dtype, device=x.device)
+    assert out.dim() == 2 and out.stride(1) == 1 and out.shape == x.shape
+    seed, site, thr, scale = _drop_args(drop)
+    with _timed(tag, 0.0, x.numel() * (x.element_size() + out.element_size())):
+        _check(lib().mv_dropout(_ptr(x), _DT[x.dtype], ctypes.c_int64(x.stride(0)), _ptr(out), _DT[out.dtype],
+                                ctypes.c_int64(out.stride(0)), x.shape[0], x.shape[1], seed, site, thr, scale,
+                                _stream()), "mv_dropout")
+    return out
+
+
 # ------------------------------------------------------------------ fake-quant
 def float_quantize(x, exp, man, rounding="nearest", seed=0, offset=0, out=None,
                    out_dtype=torch.float32):
@@ -244,9 +283,10 @@ def quantize_weight(w, exp, man, out_dtype=torch.float16, transpose=True, out=No
 # ------------------------------------------------------------------------ GEMM
 def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None, out2=None,
          epilogue=EPI_NONE, q_out=None, q_res=None, accumulate=False, rows_per_img=0,
-         M=None, N=None, K=None, tag=None, tile_n=0, cluster=0, colsum=None, transpose_out=False):
+         M=None, N=None, K=None, tag=None, tile_n=0, cluster=0, colsum=None, transpose_out=False, drop=None):
     """out[M,N] = A . B^T over K with the fused epilogue of mv_gemm (include/mv_b200.h).
-    a_major/b_major = 0: operand is [M|N, K] (K contiguous); 1: operand is [K, M|N]."""
+    a_major/b_major = 0: operand is [M|N, K] (K contiguous); 1: operand is [K, M|N].
+    drop = (seed, p, site): dropout of the output after q_out (seed: int64 [1] CUDA tensor), None: off."""
     _need_cuda(A, B, out)
     assert A.dim() == 2 and B.dim() == 2 and A.stride(1) == 1 and B.stride(1) == 1
     if M is None:
@@ -282,6 +322,9 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
     if colsum is not None:
         assert colsum.dtype == torch.float32 and colsum.is_contiguous() and colsum.numel() == N
         a.colsum = colsum.data_ptr()
+    if drop is not None:
+        seed, site, thr, scale = _drop_args(drop)
+        a.drop_seed, a.drop_thr, a.drop_scale, a.drop_site = seed.value, thr.value, scale.value, site
     kind = "gemm_wgrad" if accumulate else ("gemm_dgrad" if epilogue == EPI_DGELU or tag == "dgrad"
                                             else "gemm_fwd")
     flop = nbytes = 0.0
@@ -327,7 +370,9 @@ def layernorm_q_fwd(x, gamma, beta, *, q_in=None, q_post=None, out_dtype=torch.f
 
 
 def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=None, dbeta=None,
-                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None):
+                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None, drop=None, mask_dx=False):
+    """drop = (seed, p, site): mv_layernorm_q_bwd_drop — dx_f16 and dbias_prev see the masked gradient, dx too when
+    mask_dx."""
     _need_cuda(dy, x)
     D = x.shape[-1]
     x2, dy2 = x.reshape(-1, D), dy.reshape(-1, D)
@@ -342,13 +387,16 @@ def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=No
     # x 4 + dy + dres 4 read, dx 4 + fp16 copy 2 written
     with _timed(tag or "ln_bwd", 0.0, rows * D * (4 + dy2.element_size() + (4 if dres is not None else 0) + 4
                                             + (2 if dx_f16 is not None else 0))):
-        rc = lib().mv_layernorm_q_bwd(_ptr(dy2), _DT[dy2.dtype], ctypes.c_int64(dy2.stride(0)), _ptr(x2),
-                                      ctypes.c_int64(x2.stride(0)), _ptr(dres2),
-                                      ctypes.c_int64(dres2.stride(0) if dres2 is not None else D),
-                                      _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dx),
-                                      ctypes.c_int64(dx.stride(0)), _ptr(dx_f16), ctypes.c_int64(D),
-                                      _ptr(dgamma), _ptr(dbeta), _ptr(dbias_prev), rows, D, qi[0], qi[1],
-                                      _stream())
+        args = (_ptr(dy2), _DT[dy2.dtype], ctypes.c_int64(dy2.stride(0)), _ptr(x2),
+                ctypes.c_int64(x2.stride(0)), _ptr(dres2),
+                ctypes.c_int64(dres2.stride(0) if dres2 is not None else D),
+                _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dx),
+                ctypes.c_int64(dx.stride(0)), _ptr(dx_f16), ctypes.c_int64(D),
+                _ptr(dgamma), _ptr(dbeta), _ptr(dbias_prev), rows, D, qi[0], qi[1])
+        if drop is None:
+            rc = lib().mv_layernorm_q_bwd(*args, _stream())
+        else:
+            rc = lib().mv_layernorm_q_bwd_drop(*args, *_drop_args(drop), int(bool(mask_dx)), _stream())
     _check(rc, "mv_layernorm_q_bwd")
     return dx, dx_f16
 

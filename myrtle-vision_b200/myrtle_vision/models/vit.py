@@ -231,7 +231,8 @@ class ViT(nn.Module):
     def engine(self):
         if self._engine is None:
             cfg = mv_engine.EngineConfig(self.dim, self.heads, self.mlp_dim, self.depth,
-                                         self.patch_size, self.quantizer.plan)
+                                         self.patch_size, self.quantizer.plan, dropout=self.dropout_p,
+                                         emb_dropout=self.emb_dropout_p)
             self._engine = mv_engine.EncoderEngine(cfg, self._engine_params())
             self._engine.profile = self.profile
             self._engine.probes = [block[0].fn.fn.attn_output for block in self.transformer.layers]
@@ -295,12 +296,10 @@ class ViT(nn.Module):
         if not img.is_cuda:
             raise RuntimeError("myrtle-vision_b200 runs on CUDA (sm_100a) only; there is no CPU "
                                "fallback — move the model and the batch to a B200")
-        if self.training and (self.dropout_p > 0 or self.emb_dropout_p > 0):
-            raise NotImplementedError("dropout > 0 is not supported by the fused path "
-                                      "(all shipped configs use 0.0)")
         b, c, h, w = img.shape
         p = self.patch_size
         engine = self.engine()
+        engine.training = self.training          # dropout (self.dropout_p, self.emb_dropout_p) in training mode only
         pos_full = self._pos_full(h // p, w // p)
         x = mv_engine.EncoderFunction.apply(engine, img, pos_full, self.cls_token,
                                             *engine.params)
