@@ -138,8 +138,12 @@ int mv_gemm(const mv_gemm_args* args, void* stream);
  *     mv_gemm that carry no quantiser (dgrad / gelu' outputs; the unquantised qkv of FP16_32), dqkv of
  *     mv_attention_bwd;
  *   - mv_scale_f32 meets a non-finite result (the un-scale pass over the parameter gradients sees every NaN / inf
- *     the backward produced).
- * The caller clears it at the start of a step and hands it to mv_adamw_step's found_inf (no host sync). */
+ *     the backward produced; each element is tested, so a finite FLT_MAX does not raise it).
+ * The caller clears it at the start of a step and hands it to mv_adamw_step's found_inf (no host sync).
+ * The library does not own the int: it keeps the one pointer process-wide and every later launch of the kernels
+ * above, by any caller, writes through it.  Register it only around the launches that should report into it, and
+ * unregister it (NULL) before the int is freed.  A launch captured into a CUDA graph keeps the pointer it was
+ * captured with. */
 int mv_set_overflow_flag(int* flag_dev);
 /* End-of-step bookkeeping, GradScaler.update() on the device: state_dev = {found_inf, scale_target, good_steps}
  * (3 floats).  found_inf <- found_inf (sticky until the caller clears it) or flag != 0 or *shared_slot != 0 (shared_slot, nullable: a float that went through the

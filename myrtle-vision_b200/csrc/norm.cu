@@ -475,14 +475,14 @@ scale_kernel(const float* __restrict__ in, const float* __restrict__ scale_dev, 
     const float s = invert ? 1.0f / __ldg(scale_dev) : __ldg(scale_dev);
     const int64_t stride = int64_t(gridDim.x) * blockDim.x;
     // overflow sink: a non-finite result anywhere (the final un-scale of the parameter gradients: GradScaler's
-    // inf / NaN test), or a value that does not fit the fp16 copy
-    const float limit = out16 != nullptr ? kHalfOverflow : 3.4028234664e38f;
+    // inf / NaN test, element by element like its isfinite), or a value that does not fit the fp16 copy.  One test per
+    // element, !(|v| < limit), is true for NaN as well; fp32 only, the limit is +inf, so FLT_MAX passes.
+    const float limit = out16 != nullptr ? kHalfOverflow : __int_as_float(0x7f800000);
     bool bad = false;
     for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n4; i += stride) {
         float4 v = __ldcs(reinterpret_cast<const float4*>(in) + i);
         v.x *= s; v.y *= s; v.z *= s; v.w *= s;
-        const float m = fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w)));
-        bad |= !(m < limit) | !((v.x + v.y) + (v.z + v.w) == (v.x + v.y) + (v.z + v.w));     // too large, inf, or NaN
+        bad |= !(fabsf(v.x) < limit) | !(fabsf(v.y) < limit) | !(fabsf(v.z) < limit) | !(fabsf(v.w) < limit);
         if (out32 != nullptr) reinterpret_cast<float4*>(out32)[i] = v;
         if (out16 != nullptr) {
             __half2 lo = __floats2half2_rn(sat16(v.x), sat16(v.y)), hi = __floats2half2_rn(sat16(v.z), sat16(v.w));

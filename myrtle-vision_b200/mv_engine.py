@@ -246,7 +246,6 @@ class EncoderEngine:
 
     def _gradient_scale(self, gx):
         """Power-of-two operand scale S chosen on the device: max |gx| * S lands in [target / 2, target]."""
-        mv.set_overflow_flag(self.overflow)        # (cleared by the training forward this backward belongs to)
         if self.gfmt is not None:
             # the gradient quantisers must see the gradient as autograd presents it (what QPyTorch's would see under
             # the reference's GradScaler): no rescaling here, loss scaling is the caller's
@@ -282,14 +281,23 @@ class EncoderEngine:
         return _Drops(cfg, seed)
 
     def forward(self, img, pos_full, cls_token, save):
-        # a training forward opens an overflow window that its backward closes (mv_overflow_update); inference
-        # forwards report nothing
+        # A training forward clears self.overflow and its backward closes the window (mv_overflow_update); inference
+        # forwards report nothing.  The library keeps one process-wide flag pointer, so it is registered only while
+        # this engine's own kernels run and cleared on the way out, exception or not: launches outside the step (other
+        # models, standalone calls) never write into this engine's flag, nor into it after it is freed.  A captured
+        # CUDA graph keeps the pointer its kernels were captured with.
         mv.set_overflow_flag(self.overflow if save else None)
-        if save:
-            self.overflow.zero_()
-        drops = self._draw_drops()
-        if self.wide:
-            return self._forward_wide(img, pos_full, cls_token, save, drops)
+        try:
+            if save:
+                self.overflow.zero_()
+            drops = self._draw_drops()
+            if self.wide:
+                return self._forward_wide(img, pos_full, cls_token, save, drops)
+            return self._forward_16(img, pos_full, cls_token, save, drops)
+        finally:
+            mv.set_overflow_flag(None)
+
+    def _forward_16(self, img, pos_full, cls_token, save, drops):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
@@ -339,8 +347,16 @@ class EncoderEngine:
 
     # ----------------------------------------------------------------- backward
     def backward(self, saved, gx):
-        if self.wide:
-            return self._backward_wide(saved, gx)
+        # the overflow window of the training forward, continued for this engine's backward launches only (see forward)
+        mv.set_overflow_flag(self.overflow)
+        try:
+            if self.wide:
+                return self._backward_wide(saved, gx)
+            return self._backward_16(saved, gx)
+        finally:
+            mv.set_overflow_flag(None)
+
+    def _backward_16(self, saved, gx):
         cfg, fmt = self.cfg, self.fmt
         B, N = saved["B"], saved["N"]
         M, D, Mm, H = B * N, cfg.dim, cfg.mlp_dim, cfg.heads
@@ -663,9 +679,17 @@ class EncoderEngine:
 
 
 class EncoderFunction(torch.autograd.Function):
+    @classmethod
+    def apply(cls, engine, img, pos_full, cls_token, *params):
+        # ctx.needs_input_grad follows requires_grad even under torch.no_grad(), and forward() itself always runs with
+        # grad mode off, so grad mode is read here: without it the forward saves nothing and reports into no flag
+        if not torch.is_grad_enabled():
+            return engine.forward(img, pos_full, cls_token, save=False)[0]
+        return super().apply(engine, img, pos_full, cls_token, *params)
+
     @staticmethod
     def forward(ctx, engine, img, pos_full, cls_token, *params):
-        need = any(ctx.needs_input_grad)      # False under torch.no_grad() / eval without grads
+        need = any(ctx.needs_input_grad)      # False when no input requires a gradient
         with torch.no_grad():
             x, saved = engine.forward(img, pos_full, cls_token, save=need)
         ctx.engine, ctx.saved = engine, saved
