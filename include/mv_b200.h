@@ -128,6 +128,13 @@ typedef struct {
 } mv_gemm_args;
 
 int mv_gemm(const mv_gemm_args* args, void* stream);
+/* mv_gemm with q_out rounded stochastically (see "gradient rounding stream" below): value (m, n) of the output [M, N] is
+ * element i = m*N + n of the site tensor, rounded to (q_out_exp, q_out_man) with the bits that mv_float_quantize(...,
+ * MV_ROUND_STOCHASTIC, *seed_dev, offset) uses for element i.  The rounding takes q_out's place in the epilogue
+ * (before the gelu' multiply of MV_EPI_DGELU).  An fp16 output raises the overflow flag where the value before or
+ * after rounding does not fit fp16.  CTA-pair kernel only (16-bit operands, cluster == 0), plain or MV_EPI_DGELU
+ * outputs (colsum allowed; no accumulate, out2, residual or dropout).  seed_dev NULL: exactly mv_gemm. */
+int mv_gemm_grad_round(const mv_gemm_args* args, const uint64_t* seed_dev, uint64_t offset, void* stream);
 
 /* ---------------------------------------------------------------- overflow sink
  * Replaces the inf / NaN test of torch.cuda.amp.GradScaler (classification/train.py:167, 259-277; the reference
@@ -179,6 +186,16 @@ int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_dy, const f
                             float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
                             float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
                             const uint64_t* seed_dev, int site, uint32_t thr, float scale, int mask_dx, void* stream);
+/* mv_layernorm_q_bwd_drop with the gradient quantiser's rounding per call: rounding MV_ROUND_STOCHASTIC rounds the
+ * LayerNorm-input gradient (format of mv_set_grad_format) with the "gradient rounding stream" (round_seed, a device
+ * pointer, and round_offset; element i = row*D + c).  MV_ROUND_NEAREST, or no gradient format set: exactly
+ * mv_layernorm_q_bwd_drop (seed_dev NULL: no dropout).  Stochastic: fp16 dy. */
+int mv_layernorm_q_bwd_round(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
+                             int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
+                             float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
+                             float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
+                             const uint64_t* seed_dev, int site, uint32_t thr, float scale, int mask_dx,
+                             int rounding, const uint64_t* round_seed, uint64_t round_offset, void* stream);
 /* Gradient quantiser (QPyTorch's Quantizer(backward_number=FloatingPoint(exp, man), backward_rounding="nearest"),
  * qtorch/quant/quant_module.py — an option the reference's NumberFormat.quantizer never sets, utils/quantize.py:47-72;
  * named by the north star).  Process-wide; (0, 0) = off, the default.  When on, mv_layernorm_q_bwd rounds the
@@ -216,6 +233,23 @@ int mv_scale_f32(const float* in, const float* scale_dev, int invert, float* out
  * output saturates and raises the overflow flag (mv_set_overflow_flag) where |value| does not fit. */
 int mv_dropout(const void* in, int in_dtype, int64_t ld_in, void* out, int out_dtype, int64_t ld_out, int rows, int cols,
                const uint64_t* seed_dev, int site, uint32_t thr, float scale, void* stream);
+/* ---------------------------------------------------------------- gradient rounding stream
+ * QPyTorch's Quantizer(backward_number=FloatingPoint(exp, man), backward_rounding="stochastic") at a gradient-quantiser
+ * site: element i of the site tensor (token-major gradient [rows = B*N, cols = C]: i = m*C + c; a weight gradient: its
+ * [out, in] layout) is rounded with the bits mv_float_quantize(x, exp, man, MV_ROUND_STOCHASTIC, seed, offset) uses for
+ * element i — the 16-bit stream for man >= 7, the 32-bit stream for man < 7 — with
+ *   offset = site + (rank << 32)   (rank: data-parallel rank, 0 on one GPU, so that ranks round independently)
+ *   sites of encoder block l: 10l + k, k = 0 LN1 input, 1 to_qkv input, 2 to_qkv weight, 3 to_out input, 4 to_out
+ *   weight, 5 LN2 input, 6 fc1 input, 7 fc1 weight, 8 fc2 input (before the gelu' multiply), 9 fc2 weight;
+ *   10 * depth: the patch-embedding weight; 10 * depth + 1 + j: the decoder's quantisers in the order its forward
+ *   applies them (the LayerNorm input first, then input and weight of each Linear).
+ * The 64-bit seed is read from device memory (drawn per training forward from torch's generator, separate from the
+ * dropout seed, whose sites use the same counter words).  The result is a pure function of (seed, offset, i): a fused
+ * site equals mv_float_quantize_dev applied to the unfused value, bit for bit. */
+/* mv_float_quantize with MV_ROUND_STOCHASTIC and the seed read from device memory (a captured CUDA graph rounds with
+ * whatever seed the step drew). */
+int mv_float_quantize_dev(const float* in, void* out, int out_dtype, int64_t n, int exp_bits, int man_bits,
+                          const uint64_t* seed_dev, uint64_t offset, void* stream);
 /* fp16 / fp32 in[rows, cols] (row pitch ld elements) times `mul` -> fp32 copy out[rows, cols] and / or
  * fp32 transpose out_t[cols, rows] with row pitch ld_t >= rows (either may be NULL).  The 32-bit formats (q_format TF32 / FP32) run
  * their contractions as kind::tf32 on K-major fp32 operands; this prepares dY^T / X^T for wgrad and

@@ -123,7 +123,7 @@ int make_tmap_3d(CUtensorMap* map, const void* ptr, int dtype, uint64_t d0, uint
 }  // namespace mv
 
 extern "C" const char* mv_last_error(void) { return mv::g_err; }
-extern "C" int mv_version(void) { return 101; }
+extern "C" int mv_version(void) { return 102; }
 extern "C" int mv_set_overflow_flag(int* flag_dev) { mv::g_overflow = flag_dev; return 0; }
 extern "C" int mv_set_grad_format(int exp_bits, int man_bits) {
     if (exp_bits != 0 && (exp_bits < 2 || exp_bits > 8 || man_bits < 1 || man_bits > 22)) {

@@ -67,6 +67,7 @@ struct GemmDev {
     float* colsum;              // CTA-pair kernel: fp32 [N] += column sums of the stored values (fused bias gradient)
     int* ovf;                   // overflow sink (mv_set_overflow_flag) or NULL
     DropDev drop;               // dropout mask of the output (CTA-pair kernel, kDrop instantiations); seed NULL: off
+    SrDev sr;                   // stochastic rounding of q_out (CTA-pair kernel, kSR instantiations); seed NULL: off
 };
 
 __device__ __forceinline__ float sat16(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
@@ -637,7 +638,10 @@ __device__ __forceinline__ void stage_chunk(const EpiWarp& w, uint32_t taddr, ui
 // loop is a few instructions per 4 outputs.  kRes: 0 none, 1 residual[m, n], 2 residual[m % rows_per_img, n].
 // kDrop: dropout after q_out (include/mv_b200.h "dropout mask"; the host guarantees N % 8 == 0, so the four columns of a
 // lane are one half of a Philox block and lanes 2k / 2k+1 share the block: drop_keep4_pair, rows 2j / 2j+1).
-template <int kOut, int kEpi, int kRes, int kQO, int kQR, bool kAcc, bool kCS = false, bool kDrop = false>
+// kSR: q_out rounds stochastically with the gradient rounding stream (p.sr; the host sets kQO = 0 and N % 8 == 0).  The
+// 16-bit stream shares each Philox block between lanes 2k / 2k+1 as kDrop does (rows 2j / 2j+1, sr_pair16); the 32-bit
+// stream takes one call per lane and row.
+template <int kOut, int kEpi, int kRes, int kQO, int kQR, bool kAcc, bool kCS = false, bool kDrop = false, bool kSR = false>
 __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, uint32_t taddr, uint32_t release,
                                           int mrow0, int nc0, const uint2* aux_pre = nullptr, const float4* res_pre = nullptr) {
     const int n = nc0 + w.lc;
@@ -682,6 +686,10 @@ __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, ui
     // unquantised values rounded into an fp16 container (gradient operands; qkv of FP16_32): report saturation
     constexpr bool kOvf = kOut == MV_F16 && kQO == 0 && kQR == 0 && kEpi != MV_EPI_GELU && !kAcc;
     float amax = 0.f;
+    uint64_t sr_s = 0;
+    bool s16 = false;
+    if (kSR) { sr_s = sr_seed(p.sr); s16 = p.q_out.man_bits >= 7; }
+    uint2 sr_next = make_uint2(0u, 0u);                // 16-bit stream: the odd row's half, computed with the even row
 #pragma unroll
     for (int it = 0; it < 8; it++) {
         const int m = m_first + it * 4;
@@ -698,6 +706,28 @@ __device__ __forceinline__ void epi_chunk(const GemmDev& p, const EpiWarp& w, ui
             v[0] += b4.x; v[1] += b4.y; v[2] += b4.z; v[3] += b4.w;
         }
         if (kQO == 1) fq_half4<false>(v);
+        if (kSR) {
+            uint4 r;
+            if (s16) {
+                if ((it & 1) == 0) {
+                    const bool odd = w.lane & 1;
+                    const uint64_t i = uint64_t(m_first + (it + (odd ? 1 : 0)) * 4) * uint64_t(p.N) + uint64_t(n);
+                    const uint4 ab = sr_pair16(sr_s, p.sr.offset, i >> 3, odd);
+                    r = sr_halves(make_uint2(ab.x, ab.y));
+                    sr_next = make_uint2(ab.z, ab.w);
+                } else {
+                    r = sr_halves(sr_next);
+                }
+            } else {
+                r = sr_bits4(sr_s, p.sr.offset, uint64_t(m) * uint64_t(p.N) + uint64_t(n), false);
+            }
+            const uint32_t rr[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                amax = fmaxf(amax, fabsf(v[j]));       // a value the format saturates beyond the fp16 range still raises the flag
+                v[j] = fq_stoch_elem(v[j], rr[j], p.q_out);
+            }
+        }
         if (kEpi == MV_EPI_GELU) {
             float d[4];
             gelu_both2(v[0], v[1], v[0], v[1], d[0], d[1]);
@@ -820,14 +850,15 @@ __device__ __forceinline__ void epi_chunk_acc_t(const GemmDev& p, const EpiWarp&
 }
 
 // Generic path: tails in M / N, unaligned pitches, bf16 / second outputs.  Same arithmetic, rolled loops.
-// kDrop: the dropout mask element by element (any N).
-template <bool kDrop = false>
+// kDrop: the dropout mask element by element (any N).  kSR: q_out rounds stochastically, element by element (any N).
+template <bool kDrop = false, bool kSR = false>
 __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWarp& w, uint32_t taddr, uint32_t release,
                                                int mrow0, int nc0) {
     stage_chunk(w, taddr, release);
     const int n = nc0 + w.lc;
     const int nvalid = min(4, p.N - n);
     if (nvalid > 0) {
+        const uint64_t sr_s = kSR ? sr_seed(p.sr) : 0ull;
         float cs[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll 1
         for (int it = 0; it < 8; it++) {
@@ -843,7 +874,14 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
                 continue;
             }
             if (p.bias != nullptr) for (int j = 0; j < 4; j++) if (j < nvalid) v[j] += __ldg(p.bias + n + j);
-            if (w.mode_out) for (int j = 0; j < 4; j++) v[j] = fq_apply(v[j], w.mode_out, p.q_out);
+            if (kSR) {
+                for (int j = 0; j < 4; j++)
+                    if (j < nvalid) {
+                        if (p.out_dtype == MV_F16) raise_overflow(p.ovf, fabsf(v[j]));
+                        const uint32_t r = sr_bits1(sr_s, p.sr.offset, uint64_t(m) * uint64_t(p.N) + uint64_t(n + j), p.q_out.man_bits >= 7);
+                        v[j] = float_quantize_elem<true>(v[j], r, p.q_out.exp_bits, p.q_out.man_bits);
+                    }
+            } else if (w.mode_out) for (int j = 0; j < 4; j++) v[j] = fq_apply(v[j], w.mode_out, p.q_out);
             float dm[4] = {1.f, 1.f, 1.f, 1.f};
             if (kDrop) {
                 const uint64_t seed = __ldg(reinterpret_cast<const unsigned long long*>(p.drop.seed));
@@ -872,7 +910,7 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
             }
             if (w.mode_res) for (int j = 0; j < 4; j++) v[j] = fq_apply(v[j], w.mode_res, p.q_res);
             for (int j = 0; j < 4; j++) cs[j] += v[j];
-            if (p.out_dtype == MV_F16 && !w.mode_out && !w.mode_res && p.epilogue != MV_EPI_GELU)
+            if (p.out_dtype == MV_F16 && (kSR || !w.mode_out) && !w.mode_res && p.epilogue != MV_EPI_GELU)
                 for (int j = 0; j < 4; j++) if (j < nvalid) raise_overflow(p.ovf, fabsf(v[j]));
             store_out4(p.out, p.out_dtype, m, p.ld_out, n, v, false, nvalid);
             if (p.out2 != nullptr) store_out4(p.out2, p.out2_dtype, m, p.ld_out2, n, v, false, nvalid);
@@ -885,7 +923,9 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
 
 // kDrop: the dropout instantiations (variants 3, 4, 5, 9 and the generic path with the mask).  Separate kernels so that
 // the register allocation of the kernels without dropout — the maximum over every epilogue a kernel contains — stays as it is.
-template <int BN, int EW, int AUX = 0, bool kDrop = false>
+// kSR: the stochastic gradient-rounding instantiations (variants 1, 6, 11 with q_out rounded by the stream of p.sr, and
+// the generic path with it), separate for the same reason.
+template <int BN, int EW, int AUX = 0, bool kDrop = false, bool kSR = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + 32 * EW, 1)
 gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
              const __grid_constant__ CUtensorMap tmap_aux, const __grid_constant__ GemmDev p) {
@@ -1058,7 +1098,7 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                             if (lane == 0) tma_store_wait_read();
                             __syncwarp();
                         }
-                        epi_chunk_generic<kDrop>(p, w, taddr, release, mrow0, nc0);
+                        epi_chunk_generic<kDrop, kSR>(p, w, taddr, release, mrow0, nc0);
                     }
                 }
                 GEMM_TRACE(lane == 0 && (warp == 2 || warp == 17), warp == 2 ? 1 : 2, 7, u);    // this warp's chunks done
@@ -1112,12 +1152,28 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
                     if (c + kStep < BN / 32) request(u, c + kStep);
                     else if (u + unit_stride < total_units) request(u + unit_stride, cg);
                     if (fast) chunk(taddr, release, mrow0, nc0, aux2, res4);
-                    else epi_chunk_generic<kDrop>(p, w, taddr, release, mrow0, nc0);
+                    else epi_chunk_generic<kDrop, kSR>(p, w, taddr, release, mrow0, nc0);
                 }
                 if (++acc == kAccBufs) { acc = 0; acc_phase ^= 1; }
             }
         };
-        if constexpr (kDrop && AUX == 2) {
+        if constexpr (kSR && AUX == 1) {
+            if (p.variant == 11)
+                walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2* aux2, const float4*) {
+                    epi_chunk<MV_F16, MV_EPI_DGELU, 0, 0, 0, false, true, false, true>(p, w, taddr, release, mrow0, nc0, aux2);
+                });
+            else
+                walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2* aux2, const float4*) {
+                    epi_chunk<MV_F16, MV_EPI_DGELU, 0, 0, 0, false, false, false, true>(p, w, taddr, release, mrow0, nc0, aux2);
+                });
+        } else if constexpr (kSR) {
+            if (p.variant == 1)
+                walk([&](uint32_t taddr, uint32_t release, int mrow0, int nc0) {
+                    epi_chunk<MV_F16, MV_EPI_NONE, 0, 0, 0, false, false, false, true>(p, w, taddr, release, mrow0, nc0);
+                });
+            else           // every chunk takes the generic path with stochastic rounding
+                walk([&](uint32_t, uint32_t, int, int) {});
+        } else if constexpr (kDrop && AUX == 2) {
             if (p.variant == 4)
                 walk_aux([&](uint32_t taddr, uint32_t release, int mrow0, int nc0, const uint2*, const float4* res4) {
                     epi_chunk<MV_F32, MV_EPI_NONE, 1, 1, 1, false, false, true>(p, w, taddr, release, mrow0, nc0, nullptr, res4);
@@ -1211,16 +1267,16 @@ gemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__
     }
 }
 
-template <int BN, int EW, int AUX = 0, bool kDrop = false>
+template <int BN, int EW, int AUX = 0, bool kDrop = false, bool kSR = false>
 static int launch_gemm2(const CUtensorMap& ta, const CUtensorMap& tb, const GemmDev& p, int grid, cudaStream_t st,
                         const CUtensorMap* taux = nullptr) {
     using Cfg = Gemm2Cfg<BN, EW, AUX>;
     static bool attr_done = false;
     if (!attr_done) {
-        MV_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, EW, AUX, kDrop>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm2_kernel<BN, EW, AUX, kDrop, kSR>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmem));
         attr_done = true;
     }
-    gemm2_kernel<BN, EW, AUX, kDrop><<<grid, Cfg::kThreads, Cfg::kSmem, st>>>(ta, tb, taux != nullptr ? *taux : ta, p);
+    gemm2_kernel<BN, EW, AUX, kDrop, kSR><<<grid, Cfg::kThreads, Cfg::kSmem, st>>>(ta, tb, taux != nullptr ? *taux : ta, p);
     return 0;
 }
 
@@ -1229,7 +1285,7 @@ static int launch_gemm2(const CUtensorMap& ta, const CUtensorMap& tb, const Gemm
 using namespace mv;
 
 // CTA-pair path: 16-bit operands, 256 x BN cluster tiles
-static int gemm2_host(const mv_gemm_args* a, void* stream) {
+static int gemm2_host(const mv_gemm_args* a, void* stream, const SrDev* sr = nullptr) {
     constexpr int BK = 64;
     // BN: least padding of N, ties to the wider tile; MN-major B is staged in 64-element chunks per CTA
     int BN = 128, best = -1;
@@ -1296,11 +1352,14 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
              "mv_gemm: dropout needs a plain output (no accumulate, colsum or out2)");
     MV_CHECK(!drop || a->epilogue != MV_EPI_DGELU, "mv_gemm: the gelu' epilogue takes its mask from aux, not from drop_seed");
     p.drop = DropDev{a->drop_seed, a->drop_thr, a->drop_scale, a->drop_site};
+    const bool srnd = sr != nullptr;
+    p.sr = srnd ? *sr : SrDev{nullptr, 0ull};
     // epilogue variant (epi_chunk<> instantiations in gemm2_kernel); anything else runs the generic path
     {
         auto al = [](const void* q, int bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) == 0; };
         auto qkind = [](int e, int m) { return e == 0 ? 0 : ((e == 5 && m == 10) ? 1 : 2); };
-        const int qo = qkind(a->q_out_exp, a->q_out_man), qr = qkind(a->q_res_exp, a->q_res_man);
+        // stochastic rounding replaces q_out in the kSR kernels: the variant is chosen as for an output without q_out
+        const int qo = srnd ? 0 : qkind(a->q_out_exp, a->q_out_man), qr = qkind(a->q_res_exp, a->q_res_man);
         const int res = a->residual == nullptr ? 0 : (a->rows_per_img > 0 ? 2 : 1);
         const int cs = a->colsum != nullptr ? 1 : 0;
         const bool ok = a->out2 == nullptr && (a->ld_out & 3) == 0 && (a->bias == nullptr || al(a->bias, 16)) &&
@@ -1322,6 +1381,9 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
         // the dropout kernels have compile-time epilogues for the residual and GELU variants; a lane's four columns must be
         // half a Philox block (N % 8 == 0, epi_chunk), everything else takes the generic path with the mask
         if (drop && !((v == 3 || v == 4 || v == 5 || v == 9) && a->N % 8 == 0)) v = 0;
+        // the kSR kernels have compile-time epilogues for the plain fp16 dgrad and the gelu' dgrad (its four columns per
+        // lane are half a 16-bit-stream block only with N % 8 == 0); everything else takes the generic path
+        if (srnd && !((v == 1 || v == 6 || v == 11) && a->N % 8 == 0)) v = 0;
         p.variant = v;
     }
 
@@ -1334,6 +1396,9 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     // gelu' epilogue on 256-wide tiles with a compile-time variant: its aux operand by TMA, a chunk ahead
     const bool aux_tma = heavy && BN == 256 && (p.variant == 6 || p.variant == 11) && (a->ld_aux & 7) == 0 &&
                          (reinterpret_cast<uintptr_t>(a->aux) & 15) == 0;
+    // the kSR kernels have the gelu' epilogue only with its aux operand by TMA (AUX = 1); without it (tiles narrower than
+    // 256: an mlp_dim that 256 does not divide, or a forced tile_n; an unaligned aux) every chunk takes the generic path
+    if (srnd && (p.variant == 6 || p.variant == 11) && !aux_tma) p.variant = 0;
     // x + Linear(...) epilogues with a row-for-row fp32 residual on 192-wide tiles (proj at D = 384): likewise, where the
     // epilogue and not the operand stream bounds the tile (short K: 56.5 -> 46.6 us at K = 384; at K = 1536 the two
     // operand stages it costs lose more than the prefetch gains, 93.3 -> 96.5 us)
@@ -1343,10 +1408,15 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     if (aux_tma && make_tmap_2d_plain(&taux, a->aux, MV_F16, a->M, a->N, a->ld_aux, 32, 32)) return 1;
     if (res_tma && make_tmap_2d_plain(&taux, a->residual, MV_F32, a->M, a->N, a->ld_res, 32, 32)) return 1;
     // plain fp16 outputs (variants 1, 2) on 192- / 128-wide tiles: TMA-store epilogue
-    const bool out_tma = !heavy && (BN == 192 || BN == 128) && (p.variant == 1 || p.variant == 2) && (a->ld_out & 7) == 0 &&
+    const bool out_tma = !srnd && !heavy && (BN == 192 || BN == 128) && (p.variant == 1 || p.variant == 2) && (a->ld_out & 7) == 0 &&
                          (reinterpret_cast<uintptr_t>(a->out) & 15) == 0;
     if (out_tma && make_tmap_2d_plain(&taux, a->out, MV_F16, a->M, a->N, a->ld_out, 32, 32, 1)) return 1;
-    if (drop) {
+    if (srnd) {
+        if (aux_tma) rc = launch_gemm2<256, 16, 1, false, true>(ta, tb, p, grid, st, &taux);
+        else if (BN == 256) rc = heavy ? launch_gemm2<256, 16, 0, false, true>(ta, tb, p, grid, st) : launch_gemm2<256, 12, 0, false, true>(ta, tb, p, grid, st);
+        else if (BN == 192) rc = launch_gemm2<192, 12, 0, false, true>(ta, tb, p, grid, st);
+        else rc = launch_gemm2<128, 12, 0, false, true>(ta, tb, p, grid, st);
+    } else if (drop) {
         if (res_tma) rc = launch_gemm2<192, 12, 2, true>(ta, tb, p, grid, st, &taux);
         else if (BN == 256) rc = heavy ? launch_gemm2<256, 16, 0, true>(ta, tb, p, grid, st) : launch_gemm2<256, 12, 0, true>(ta, tb, p, grid, st);
         else if (BN == 192) rc = launch_gemm2<192, 12, 0, true>(ta, tb, p, grid, st);
@@ -1429,6 +1499,7 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     p.rows_per_img = a->rows_per_img;
     p.variant = 0; p.colsum = nullptr; p.idesc2 = 0; p.transpose_out = 0; p.ovf = g_overflow;
     p.drop = DropDev{nullptr, 0u, 0.f, 0};
+    p.sr = SrDev{nullptr, 0ull};
 
     // CTA pairs sharing B through TMA multicast: measured no faster on B200 (the bound is the per-SM
     // L2->SM ingest, which multicast does not reduce), so it is opt-in (cluster == 2)
@@ -1463,4 +1534,22 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     else MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<128, 2, false>, ta, tb, p));
     g_launches++;
     return check_cuda(cudaGetLastError(), "gemm launch");
+}
+
+extern "C" int mv_gemm_grad_round(const mv_gemm_args* a, const uint64_t* seed_dev, uint64_t offset, void* stream) {
+    if (seed_dev == nullptr) return mv_gemm(a, stream);
+    MV_CHECK(a != nullptr, "mv_gemm_grad_round: null args");
+    MV_CHECK(a->a_dtype != MV_F32 && a->cluster == 0,
+             "mv_gemm_grad_round: stochastic rounding is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
+    MV_CHECK(a->q_out_exp >= 1 && a->q_out_exp <= 8 && a->q_out_man >= 1 && a->q_out_man <= 22,
+             "mv_gemm_grad_round: q_out (%d, %d) is not a float format", a->q_out_exp, a->q_out_man);
+    MV_CHECK(!a->accumulate && a->out2 == nullptr && a->drop_seed == nullptr && a->residual == nullptr &&
+             a->epilogue != MV_EPI_GELU,
+             "mv_gemm_grad_round: needs a plain or gelu' output (no accumulate, out2, dropout, residual or GELU)");
+    MV_CHECK(a->M > 0 && a->N > 0 && a->K > 0, "mv_gemm_grad_round: bad shape %dx%dx%d", a->M, a->N, a->K);
+    MV_CHECK(a->A && a->B && a->out, "mv_gemm_grad_round: null operand");
+    MV_CHECK(a->a_dtype == a->b_dtype, "mv_gemm_grad_round: A and B must share one element type");
+    if (a->epilogue == MV_EPI_DGELU) MV_CHECK(a->aux != nullptr, "mv_gemm_grad_round: the gelu' epilogue needs aux");
+    const SrDev sr{seed_dev, offset};
+    return gemm2_host(a, stream, &sr);
 }

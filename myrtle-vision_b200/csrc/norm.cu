@@ -168,7 +168,9 @@ __device__ __forceinline__ float4 unpack_dy(const uint2& u) {
 // residual stream's producer receives.  A lane owns float4 c = lane + 32 i; with D % 8 == 0 lanes 2k / 2k+1 hold the two
 // halves of one Philox block, so vectors i and i+1 take one call per lane (drop_keep4_pair).  Separate instantiations:
 // the kernels without it keep their register allocation.
-template <int NV, typename DyT, bool kGQ = false, bool kDrop = false>
+// kSR (with kGQ): the gradient quantiser rounds stochastically with the gradient rounding stream `sr` (element
+// row * D + c of the site tensor; one Philox call per lane and float4).  Separate instantiations likewise.
+template <int NV, typename DyT, bool kGQ = false, bool kDrop = false, bool kSR = false>
 __global__ void __launch_bounds__(kLnWarps * 32, 2)
 ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict__ x, int64_t ld_x,
               const float* __restrict__ dres, int64_t ld_dres, const float* __restrict__ gamma,
@@ -176,7 +178,7 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
               float* __restrict__ dx, int64_t ld_dx, __half* __restrict__ dx_lp, int64_t ld_lp,
               float* __restrict__ dgamma, float* __restrict__ dbeta, float* __restrict__ dbias_prev,
               int rows, int D, FloatFmt q_in, int* __restrict__ ovf, FloatFmt q_grad = FloatFmt{0, 0},
-              DropDev drop = DropDev{nullptr, 0u, 0.f, 0}, int mask_dx = 0) {
+              DropDev drop = DropDev{nullptr, 0u, 0.f, 0}, int mask_dx = 0, SrDev sr = SrDev{nullptr, 0ull}) {
     // Column sums (dgamma, dbeta, previous bias grad) are kept per warp in shared memory — each
     // lane owns its columns, so plain read-modify-write — which frees ~36 registers per thread for
     // occupancy; the next row's loads are issued before the current row is reduced.
@@ -211,6 +213,7 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
     };
     int row = blockIdx.x * kLnWarps + warp;
     const uint64_t seed = kDrop ? __ldg(reinterpret_cast<const unsigned long long*>(drop.seed)) : 0ull;
+    const uint64_t sr_s = kSR ? sr_seed(sr) : 0ull;
     LnBwdRow<NV, DyT> cur;
     float amax = 0.f;                   // largest |dx| rounded into the fp16 operand copy (overflow sink)
     if (row < rows) load_row(row, cur);
@@ -279,7 +282,13 @@ ln_bwd_kernel(const DyT* __restrict__ dy, int64_t ld_dy, const float* __restrict
                 float4 o;
                 o.x = fmaf(gy[i].x, rstd, fmaf(xh[i].x, cb, cc)); o.y = fmaf(gy[i].y, rstd, fmaf(xh[i].y, cb, cc));
                 o.z = fmaf(gy[i].z, rstd, fmaf(xh[i].z, cb, cc)); o.w = fmaf(gy[i].w, rstd, fmaf(xh[i].w, cb, cc));
-                if (kGQ) {
+                if (kGQ && kSR) {
+                    const uint4 r = sr_bits4(sr_s, sr.offset, uint64_t(row) * uint64_t(D) + 4ull * uint64_t(c), q_grad.man_bits >= 7);
+                    o.x = float_quantize_elem<true>(o.x, r.x, q_grad.exp_bits, q_grad.man_bits);
+                    o.y = float_quantize_elem<true>(o.y, r.y, q_grad.exp_bits, q_grad.man_bits);
+                    o.z = float_quantize_elem<true>(o.z, r.z, q_grad.exp_bits, q_grad.man_bits);
+                    o.w = float_quantize_elem<true>(o.w, r.w, q_grad.exp_bits, q_grad.man_bits);
+                } else if (kGQ) {
                     o.x = fq_nearest(o.x, q_grad); o.y = fq_nearest(o.y, q_grad);
                     o.z = fq_nearest(o.z, q_grad); o.w = fq_nearest(o.w, q_grad);
                 }
@@ -527,11 +536,32 @@ static int launch_ln_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const floa
                          int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
                          float* dx, int64_t ld_dx, void* dx_lp, int64_t ld_lp, float* dgamma, float* dbeta,
                          float* dbias_prev, int rows, int D, FloatFmt q_in, cudaStream_t st,
-                         const DropDev* drop = nullptr, int mask_dx = 0) {
+                         const DropDev* drop = nullptr, int mask_dx = 0, const SrDev* sr = nullptr) {
     int grid = (rows + kLnWarps - 1) / kLnWarps;
     const int cap = persistent_sms() * 2;
     if (grid > cap) grid = cap;
     const size_t smem = size_t(kLnWarps) * 3 * D * sizeof(float);
+    if (sr != nullptr) {
+        // stochastic gradient rounding: fp16 dy, with or without dropout
+        static bool attr_sr = false;
+        if (!attr_sr) {
+            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
+            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
+            attr_sr = true;
+        }
+        if (dy_dtype != MV_F16) { set_error("mv_layernorm_q_bwd_round: dy must be fp16"); return 1; }
+        const DropDev d = drop != nullptr ? *drop : DropDev{nullptr, 0u, 0.f, 0};
+        if (drop != nullptr)
+            ln_bwd_kernel<NV, __half, true, true, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
+                                                                                         dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
+                                                                                         q_in, g_overflow, g_grad_fmt, d, mask_dx, *sr);
+        else
+            ln_bwd_kernel<NV, __half, true, false, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
+                                                                                          dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
+                                                                                          q_in, g_overflow, g_grad_fmt, d, 0, *sr);
+        g_launches++;
+        return check_cuda(cudaGetLastError(), "ln bwd (stochastic rounding) launch");
+    }
     if (drop != nullptr) {
         // dropout variants: fp16 dy (the dgrad GEMM's output), with or without the gradient quantiser
         static bool attr_drop = false;
@@ -757,6 +787,39 @@ extern "C" int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_
         case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
         case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
         default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
+    }
+}
+
+extern "C" int mv_layernorm_q_bwd_round(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x,
+                                        const float* dres, int64_t ld_dres, const float* gamma, const float* mean,
+                                        const float* rstd, float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp,
+                                        float* dgamma, float* dbeta, float* dbias_prev, int rows, int D,
+                                        int q_in_exp, int q_in_man, const uint64_t* seed_dev, int site, uint32_t thr,
+                                        float scale, int mask_dx, int rounding, const uint64_t* round_seed,
+                                        uint64_t round_offset, void* stream) {
+    MV_CHECK(rounding == MV_ROUND_NEAREST || rounding == MV_ROUND_STOCHASTIC, "mv_layernorm_q_bwd_round: rounding %d", rounding);
+    if (rounding == MV_ROUND_NEAREST || g_grad_fmt.exp_bits == 0)
+        return mv_layernorm_q_bwd_drop(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp,
+                                       dgamma, dbeta, dbias_prev, rows, D, q_in_exp, q_in_man, seed_dev, site, thr, scale,
+                                       mask_dx, stream);
+    MV_CHECK(round_seed != nullptr, "mv_layernorm_q_bwd_round: stochastic rounding needs round_seed");
+    MV_CHECK(rows >= 0 && D > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd_round: D=%d unsupported", D);
+    MV_CHECK(ld_dy % 4 == 0 && ld_x % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_lp % 4 == 0, "mv_layernorm_q_bwd_round: row pitches must be multiples of 4");
+    MV_CHECK(thr <= 65536u, "mv_layernorm_q_bwd_round: threshold %u above 65536", thr);
+    if (rows == 0) return 0;
+    const FloatFmt qi{q_in_exp, q_in_man};
+    const DropDev d{seed_dev, thr, scale, site};
+    const DropDev* dp = seed_dev != nullptr ? &d : nullptr;
+    const SrDev sr{round_seed, round_offset};
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int nv = (D / 4 + 31) / 32;
+    switch (nv) {
+        case 1: return launch_ln_bwd<1>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+        case 2: return launch_ln_bwd<2>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+        case 3: return launch_ln_bwd<3>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+        case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+        case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+        default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
     }
 }
 

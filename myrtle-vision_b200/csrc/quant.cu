@@ -101,10 +101,13 @@ __device__ __forceinline__ float4 float_quantize_stoch4(float4 v, uint32_t r0, u
 // kStoch = false: nearest rounding on the same access pattern (a thread owns 32 contiguous input bytes, four such
 // groups in flight): every tail word is half a step of the tail, no Philox (5.57 -> TB/s on randn against
 // 16 bytes per thread and load in quant_vec_kernel)
-template <typename OutT, bool kStoch = true>
+// kDevSeed (every kernel of this file that has it): the seed is read from device memory, seed_dev, not the `seed` argument —
+// a captured CUDA graph then rounds with whatever seed the step drew (mv_float_quantize_dev)
+template <typename OutT, bool kStoch = true, bool kDevSeed = false>
 __global__ void __launch_bounds__(kQThreads)
 quant_vec16_kernel(const float* __restrict__ in, OutT* __restrict__ out, int64_t n, int exp_bits, int man_bits,
-                   uint64_t seed, uint64_t offset) {
+                   uint64_t seed, uint64_t offset, const uint64_t* __restrict__ seed_dev = nullptr) {
+    if (kDevSeed) seed = __ldg(reinterpret_cast<const unsigned long long*>(seed_dev));
     const int64_t n8 = n >> 3;
     constexpr int kU = 4;                                   // 4 x 32 B in flight per thread
     const uint32_t mask = (1u << (23 - man_bits)) - 1u;
@@ -148,20 +151,23 @@ quant_vec16_kernel(const float* __restrict__ in, OutT* __restrict__ out, int64_t
     }
 }
 // scalar companion (tails, unaligned buffers): the same 16-bit stream
-template <typename OutT>
+template <typename OutT, bool kDevSeed = false>
 __global__ void quant_scalar16_kernel(const float* __restrict__ in, OutT* __restrict__ out, int64_t begin, int64_t n,
-                                      int exp_bits, int man_bits, uint64_t seed, uint64_t offset) {
+                                      int exp_bits, int man_bits, uint64_t seed, uint64_t offset,
+                                      const uint64_t* __restrict__ seed_dev = nullptr) {
+    if (kDevSeed) seed = __ldg(reinterpret_cast<const unsigned long long*>(seed_dev));
     const int64_t stride = int64_t(gridDim.x) * blockDim.x;
     for (int64_t i = begin + int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride)
         out[i] = cvt_out<OutT>(float_quantize_elem<true>(in[i], philox_half16(seed, uint64_t(i), offset), exp_bits, man_bits));
 }
 
 // MODE 0: float_quantize ; MODE 1: fixed_point_quantize
-template <int MODE, bool STOCH, typename OutT>
+template <int MODE, bool STOCH, typename OutT, bool kDevSeed = false>
 __global__ void __launch_bounds__(kQThreads)
 quant_vec_kernel(const float* __restrict__ in, OutT* __restrict__ out, uint8_t* __restrict__ mask,
                  int64_t n, int exp_bits, int man_bits, FixedParams fp, uint64_t seed,
-                 uint64_t offset) {
+                 uint64_t offset, const uint64_t* __restrict__ seed_dev = nullptr) {
+    if (kDevSeed) seed = __ldg(reinterpret_cast<const unsigned long long*>(seed_dev));
     const int64_t n4 = n >> 2;
     const int64_t stride = int64_t(gridDim.x) * kQThreads * kQUnroll;
     // MODE 0: the format's tail mask, half a step of it, its lowest normal and largest finite magnitudes
@@ -221,11 +227,12 @@ quant_vec_kernel(const float* __restrict__ in, OutT* __restrict__ out, uint8_t* 
 }
 
 // scalar path: tails (n % 4) and unaligned buffers.  Element index i keeps its RNG word.
-template <int MODE, bool STOCH, typename OutT>
+template <int MODE, bool STOCH, typename OutT, bool kDevSeed = false>
 __global__ void quant_scalar_kernel(const float* __restrict__ in, OutT* __restrict__ out,
                                     uint8_t* __restrict__ mask, int64_t begin, int64_t n,
                                     int exp_bits, int man_bits, FixedParams fp, uint64_t seed,
-                                    uint64_t offset) {
+                                    uint64_t offset, const uint64_t* __restrict__ seed_dev = nullptr) {
+    if (kDevSeed) seed = __ldg(reinterpret_cast<const unsigned long long*>(seed_dev));
     const int64_t stride = int64_t(gridDim.x) * blockDim.x;
     for (int64_t i = begin + int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += stride) {
         uint32_t r = 0;
@@ -259,20 +266,22 @@ static inline int grid_for(int64_t work_items, int per_block) {
     return int(blocks);
 }
 
-template <typename OutT>
+template <typename OutT, bool kDevSeed = false>
 static int launch_quant16(const float* in, OutT* out, int64_t n, int exp_bits, int man_bits, uint64_t seed,
-                          uint64_t offset, cudaStream_t st) {
+                          uint64_t offset, cudaStream_t st, const uint64_t* seed_dev = nullptr) {
     if (n == 0) return 0;
     const bool aligned = (reinterpret_cast<uintptr_t>(in) % 16 == 0) && (reinterpret_cast<uintptr_t>(out) % 16 == 0);
     int64_t done = 0;
     if (aligned && n >= 8) {
         const int64_t n8 = n >> 3;
-        quant_vec16_kernel<OutT><<<grid_for(n8, kQThreads * 4), kQThreads, 0, st>>>(in, out, n, exp_bits, man_bits, seed, offset);
+        quant_vec16_kernel<OutT, true, kDevSeed><<<grid_for(n8, kQThreads * 4), kQThreads, 0, st>>>(in, out, n, exp_bits, man_bits, seed, offset,
+                                                                                                  seed_dev);
         g_launches++;
         done = n8 << 3;
     }
     if (done < n) {
-        quant_scalar16_kernel<OutT><<<grid_for(n - done, 256), 256, 0, st>>>(in, out, done, n, exp_bits, man_bits, seed, offset);
+        quant_scalar16_kernel<OutT, kDevSeed><<<grid_for(n - done, 256), 256, 0, st>>>(in, out, done, n, exp_bits, man_bits, seed, offset,
+                                                                                        seed_dev);
         g_launches++;
     }
     return check_cuda(cudaGetLastError(), "quant launch");
@@ -298,10 +307,10 @@ static int launch_quant_nearest8(const float* in, OutT* out, int64_t n, int exp_
     return check_cuda(cudaGetLastError(), "quant launch");
 }
 
-template <int MODE, bool STOCH, typename OutT>
+template <int MODE, bool STOCH, typename OutT, bool kDevSeed = false>
 static int launch_quant(const float* in, OutT* out, uint8_t* mask, int64_t n, int exp_bits,
                         int man_bits, FixedParams fp, uint64_t seed, uint64_t offset,
-                        cudaStream_t st) {
+                        cudaStream_t st, const uint64_t* seed_dev = nullptr) {
     if (n == 0) return 0;
     const bool aligned = (reinterpret_cast<uintptr_t>(in) % 16 == 0) &&
                          (reinterpret_cast<uintptr_t>(out) % (4 * sizeof(OutT)) == 0) &&
@@ -309,14 +318,14 @@ static int launch_quant(const float* in, OutT* out, uint8_t* mask, int64_t n, in
     int64_t done = 0;
     if (aligned && n >= 4) {
         const int64_t n4 = n >> 2;
-        quant_vec_kernel<MODE, STOCH, OutT><<<grid_for(n4, kQThreads * kQUnroll), kQThreads, 0, st>>>(
-            in, out, mask, n, exp_bits, man_bits, fp, seed, offset);
+        quant_vec_kernel<MODE, STOCH, OutT, kDevSeed><<<grid_for(n4, kQThreads * kQUnroll), kQThreads, 0, st>>>(
+            in, out, mask, n, exp_bits, man_bits, fp, seed, offset, seed_dev);
         g_launches++;
         done = n4 << 2;
     }
     if (done < n) {
-        quant_scalar_kernel<MODE, STOCH, OutT><<<grid_for(n - done, 256), 256, 0, st>>>(
-            in, out, mask, done, n, exp_bits, man_bits, fp, seed, offset);
+        quant_scalar_kernel<MODE, STOCH, OutT, kDevSeed><<<grid_for(n - done, 256), 256, 0, st>>>(
+            in, out, mask, done, n, exp_bits, man_bits, fp, seed, offset, seed_dev);
         g_launches++;
     }
     return check_cuda(cudaGetLastError(), "quant launch");
@@ -519,6 +528,26 @@ extern "C" int mv_float_quantize(const float* in, void* out, int out_dtype, int6
     return rounding == MV_ROUND_STOCHASTIC
                ? launch_quant<0, true, __half>(in, (__half*)out, nullptr, n, exp_bits, man_bits, fp, seed, offset, st)
                : launch_quant_nearest8<__half>(in, (__half*)out, n, exp_bits, man_bits, st);
+}
+
+extern "C" int mv_float_quantize_dev(const float* in, void* out, int out_dtype, int64_t n, int exp_bits, int man_bits,
+                                     const uint64_t* seed_dev, uint64_t offset, void* stream) {
+    MV_CHECK(n >= 0, "mv_float_quantize_dev: negative n");
+    MV_CHECK(exp_bits >= 1 && exp_bits <= 8, "mv_float_quantize_dev: exp_bits %d not in [1,8]", exp_bits);
+    MV_CHECK(man_bits >= 1 && man_bits <= 22, "mv_float_quantize_dev: man_bits %d not in [1,22]", man_bits);
+    MV_CHECK(n == 0 || (in && out && seed_dev), "mv_float_quantize_dev: null buffer");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    FixedParams fp{};
+    const bool s16 = man_bits >= 7;             // the streams of mv_float_quantize, MV_ROUND_STOCHASTIC
+    if (out_dtype == MV_F32) {
+        if (s16) return launch_quant16<float, true>(in, (float*)out, n, exp_bits, man_bits, 0, offset, st, seed_dev);
+        return launch_quant<0, true, float, true>(in, (float*)out, nullptr, n, exp_bits, man_bits, fp, 0, offset, st, seed_dev);
+    }
+    MV_CHECK(out_dtype == MV_F16, "mv_float_quantize_dev: unsupported out_dtype %d", out_dtype);
+    MV_CHECK(exp_bits <= 5 && man_bits <= 10,
+             "mv_float_quantize_dev: (exp=%d, man=%d) is not exactly representable in an fp16 container", exp_bits, man_bits);
+    if (s16) return launch_quant16<__half, true>(in, (__half*)out, n, exp_bits, man_bits, 0, offset, st, seed_dev);
+    return launch_quant<0, true, __half, true>(in, (__half*)out, nullptr, n, exp_bits, man_bits, fp, 0, offset, st, seed_dev);
 }
 
 extern "C" int mv_fixed_point_quantize(const float* in, float* out, uint8_t* mask, int64_t n, int wl,

@@ -206,6 +206,60 @@ __device__ __forceinline__ uint32_t drop_keep4_pair(uint64_t seed, const DropDev
 }
 __device__ __forceinline__ float drop_mul(uint32_t bits, int j, float scale) { return ((bits >> j) & 1u) ? scale : 0.f; }
 
+// ---- stochastic gradient rounding (include/mv_b200.h "gradient rounding stream"): element i of a site tensor is rounded
+// with the bits mv_float_quantize(..., MV_ROUND_STOCHASTIC, seed, offset) gives element i ----
+struct SrDev {
+    const uint64_t* seed;       // device pointer; NULL: off
+    uint64_t offset;            // site + (rank << 32)
+};
+__device__ __forceinline__ uint64_t sr_seed(const SrDev& s) { return __ldg(reinterpret_cast<const unsigned long long*>(s.seed)); }
+// the four half-words of one half of a 16-bit-stream block, element order
+__device__ __forceinline__ uint4 sr_halves(uint2 h) {
+    return make_uint4(h.x & 0xFFFFu, h.x >> 16, h.y & 0xFFFFu, h.y >> 16);
+}
+// random bits of elements i .. i+3 (i % 4 == 0), computed by this lane alone: half (i & 4) of the 16-bit block i >> 3
+// (s16, man_bits >= 7) or the whole 32-bit block i >> 2
+__device__ __forceinline__ uint4 sr_bits4(uint64_t seed, uint64_t offset, uint64_t i, bool s16) {
+    if (s16) {
+        const uint4 w = philox4x32_10(seed, i >> 3, offset);
+        return sr_halves((i & 4) ? make_uint2(w.z, w.w) : make_uint2(w.x, w.y));
+    }
+    return philox4x32_10(seed, i >> 2, offset);
+}
+// random bits of element i alone (word selects, not an indexed array: that would live in local memory)
+__device__ __forceinline__ uint32_t sr_bits1(uint64_t seed, uint64_t offset, uint64_t i, bool s16) {
+    const uint4 w = philox4x32_10(seed, s16 ? (i >> 3) : (i >> 2), offset);
+    const uint64_t k = s16 ? ((i & 7) >> 1) : (i & 3);
+    const uint32_t word = (k & 2) ? ((k & 1) ? w.w : w.z) : ((k & 1) ? w.y : w.x);
+    return s16 ? ((i & 1) ? (word >> 16) : (word & 0xFFFFu)) : word;
+}
+// float_quantize_elem<true> with the normal range inline ("add the tail bits, clear the tail, clip to the largest finite
+// value") and everything else (below the lowest normal binade, inf / NaN) out of line, so that the rare branch does not hold
+// registers across an unrolled epilogue.  Same results.
+static __device__ __noinline__ float fq_stoch_rare(float a, uint32_t r, int exp_bits, int man_bits) {
+    return float_quantize_elem<true>(a, r, exp_bits, man_bits);
+}
+__device__ __forceinline__ float fq_stoch_elem(float a, uint32_t r, FloatFmt f) {
+    const uint32_t t = __float_as_uint(a), mag = t & 0x7FFFFFFFu;
+    const uint32_t mask = (1u << (23 - f.man_bits)) - 1u;
+    const uint32_t lo_bits = uint32_t(127 - ((1 << (f.exp_bits - 1)) - 2)) << 23;
+    const uint32_t hi_bits = (uint32_t((1 << (f.exp_bits - 1)) - 1 + 127) << 23) | (0x007FFFFFu & ~mask);
+    if (mag < lo_bits || mag > hi_bits) return fq_stoch_rare(a, r, f.exp_bits, f.man_bits);
+    const uint32_t q = (t + (r & mask)) & ~mask;
+    return __uint_as_float((q & 0x7FFFFFFFu) > hi_bits ? ((t & 0x80000000u) | hi_bits) : q);
+}
+
+// 16-bit stream shared by a lane pair, as drop_keep4_pair: the even lane computes block `ctr` for its row A, the odd lane
+// for its row B; returns this lane's half of A (.x) and of B (.y), each as the two words of four half-words
+__device__ __forceinline__ uint4 sr_pair16(uint64_t seed, uint64_t offset, uint64_t ctr, bool odd) {
+    const uint4 w = philox4x32_10(seed, ctr, offset);
+    const uint2 mine = odd ? make_uint2(w.z, w.w) : make_uint2(w.x, w.y);
+    const uint2 give = odd ? make_uint2(w.x, w.y) : make_uint2(w.z, w.w);
+    const uint2 got = make_uint2(__shfl_xor_sync(0xffffffffu, give.x, 1), __shfl_xor_sync(0xffffffffu, give.y, 1));
+    const uint2 a = odd ? got : mine, b = odd ? mine : got;
+    return make_uint4(a.x, a.y, b.x, b.y);
+}
+
 __device__ __forceinline__ float bits_to_uniform(uint32_t b) {
     return float(b >> 8) * (1.0f / 16777216.0f);
 }

@@ -66,6 +66,15 @@ class EngineConfig:
 
 PER_LAYER = 12   # ln1.w ln1.b qkv.w qkv.b out.w out.b ln2.w ln2.b fc1.w fc1.b fc2.w fc2.b
 
+# Gradient-quantiser sites of encoder block l (include/mv_b200.h "gradient rounding stream"): 10 l + k; 10 depth is the
+# patch-embedding weight, 10 depth + 1 + j the decoder's stubs (models/vit.py ViT._gfmt)
+GS_LN1, GS_QKV_IN, GS_QKV_W, GS_OUT_IN, GS_OUT_W, GS_LN2, GS_FC1_IN, GS_FC1_W, GS_FC2_IN, GS_FC2_W = range(10)
+
+
+def grad_round_offset(site, rank=0):
+    """The stream offset of a gradient-quantiser site on data-parallel rank `rank`: site + (rank << 32)."""
+    return int(site) + (int(rank) << 32)
+
 
 class _Drops:
     """The dropout sites of one training forward and its backward: site ids of include/mv_b200.h ("dropout mask") and
@@ -157,6 +166,13 @@ class EncoderEngine:
         # None, or an int64 [1] device tensor that training forwards use instead of a fresh draw (reproduces the masks of
         # an earlier step, e.g. one replayed from a CUDA graph, given its last_dropout_seed)
         self.fixed_dropout_seed = None
+        # stochastic gradient rounding (QuantPlan.grad_rounding == "stochastic" with a gradient format): the seed of the
+        # last forward that drew one, an override like fixed_dropout_seed, and the seed of the running step (None when
+        # this forward drew none; the decoder's stubs read it)
+        self.grad_round = self.gfmt is not None and getattr(plan, "grad_rounding", "nearest") == "stochastic"
+        self.last_grad_round_seed = None
+        self.fixed_grad_round_seed = None
+        self.step_grad_round_seed = None
 
     # ------------------------------------------------------------------ weights
     def _weight_indices(self):
@@ -240,6 +256,14 @@ class EncoderEngine:
             self.params[i].data_ptr() for i in idx)
 
     @property
+    def rank(self):
+        """Data-parallel rank (0 without parallel.DataParallel): the high word of the gradient rounding offsets."""
+        if self.reducer is None or getattr(self.reducer, "world", 1) <= 1:
+            return 0
+        import torch.distributed as dist
+        return dist.get_rank(self.reducer.group)
+
+    @property
     def found_inf(self):
         """fp32 [1] on the device: 1.0 when the last backward overflowed (identical on every data-parallel rank)."""
         return self.scaler_state[0:1]
@@ -280,6 +304,18 @@ class EncoderEngine:
         self.last_dropout_seed = seed
         return _Drops(cfg, seed)
 
+    def _draw_grad_round(self, save):
+        """A fresh 64-bit seed per forward that may be followed by a backward, when stochastic gradient rounding is on
+        (drawn after the dropout seed, on the device, like it).  None otherwise: no draw, the generator is not
+        advanced."""
+        if not (save and self.grad_round):
+            return None
+        seed = self.fixed_grad_round_seed
+        if seed is None:
+            seed = torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=self.dev)
+        self.last_grad_round_seed = seed
+        return seed
+
     def forward(self, img, pos_full, cls_token, save):
         # A training forward clears self.overflow and its backward closes the window (mv_overflow_update); inference
         # forwards report nothing.  The library keeps one process-wide flag pointer, so it is registered only while
@@ -291,9 +327,13 @@ class EncoderEngine:
             if save:
                 self.overflow.zero_()
             drops = self._draw_drops()
+            self.step_grad_round_seed = self._draw_grad_round(save)
             if self.wide:
                 return self._forward_wide(img, pos_full, cls_token, save, drops)
-            return self._forward_16(img, pos_full, cls_token, save, drops)
+            x, saved = self._forward_16(img, pos_full, cls_token, save, drops)
+            if saved is not None:
+                saved["grad_round"] = self.step_grad_round_seed
+            return x, saved
         finally:
             mv.set_overflow_flag(None)
 
@@ -392,48 +432,58 @@ class EncoderEngine:
         # would apply it to the local gradient)
         gq = self.gfmt
         mv.set_grad_format(gq)
+        # stochastic rounding (QuantPlan.grad_rounding): every site rounds with the stream of include/mv_b200.h under
+        # the seed its forward drew; gr(site) is the grad_round argument of the mv_native calls, None: nearest
+        seed, rank = saved.get("grad_round"), self.rank
 
-        def wq_grad(i):
-            if gq is not None:
+        def gr(site):
+            return None if seed is None else (seed, grad_round_offset(site, rank))
+
+        def wq_grad(i, site):
+            if gq is not None and seed is not None:
+                mv.float_quantize_dev(g[i], gq[0], gq[1], gr(site), out=g[i])
+            elif gq is not None:
                 mv.float_quantize(g[i], gq[0], gq[1], out=g[i])
 
         for l in range(last, -1, -1):
             b0 = 2 + PER_LAYER * l
             x, xn1, mean1, rstd1, qkv, att, lse, x1, xn2, mean2, rstd2, u, h = saved["layers"][l]
+            s0 = 10 * l                                                     # this block's gradient-quantiser sites
             # ---- FeedForward
             du = torch.empty(M, Mm, dtype=f16, device=dev)
             # fc1's bias gradient (column sums of du) rides in the epilogue
-            mv.gemm(dx_h, wq[b0 + 10][1], du, aux=u, epilogue=mv.EPI_DGELU, colsum=g[b0 + 9].view(-1), q_out=gq)
+            mv.gemm(dx_h, wq[b0 + 10][1], du, aux=u, epilogue=mv.EPI_DGELU, colsum=g[b0 + 9].view(-1), q_out=gq,
+                    grad_round=gr(s0 + GS_FC2_IN))
             # fc2's [D, 4D] gradient as its transpose h^T dx: 256 x 384 tiles over 4D rows instead of 1.5 padded 256-row tiles
             mv.gemm(h, dx_h, g[b0 + 10], a_major=1, b_major=1, accumulate=True, transpose_out=True)
-            wq_grad(b0 + 10)
+            wq_grad(b0 + 10, s0 + GS_FC2_W)
             dxn2 = torch.empty(M, D, dtype=f16, device=dev)
-            mv.gemm(du, wq[b0 + 8][1], dxn2, tag="dgrad", q_out=gq)
+            mv.gemm(du, wq[b0 + 8][1], dxn2, tag="dgrad", q_out=gq, grad_round=gr(s0 + GS_FC1_IN))
             mv.gemm(du, xn2, g[b0 + 8], a_major=1, b_major=1, accumulate=True)
-            wq_grad(b0 + 8)
+            wq_grad(b0 + 8, s0 + GS_FC1_W)
             del du
             # dx1_h and to_out's bias gradient: the masked gradient of the to_out branch (dropout site of to_out)
             dx1, dx1_h = mv.layernorm_q_bwd(dxn2, x1, prm[b0 + 6], mean2, rstd2, dres=dx, q_in=fmt,
                                             dgamma=g[b0 + 6], dbeta=g[b0 + 7], dbias_prev=g[b0 + 5],
-                                            drop=drops and drops.proj(l))
+                                            drop=drops and drops.proj(l), grad_round=gr(s0 + GS_LN2))
             # ---- Attention
             datt = torch.empty(M, D, dtype=f16, device=dev)
-            mv.gemm(dx1_h, wq[b0 + 4][1], datt, tag="dgrad", q_out=gq)
+            mv.gemm(dx1_h, wq[b0 + 4][1], datt, tag="dgrad", q_out=gq, grad_round=gr(s0 + GS_OUT_IN))
             mv.gemm(dx1_h, att, g[b0 + 4], a_major=1, b_major=1, accumulate=True)
-            wq_grad(b0 + 4)
+            wq_grad(b0 + 4, s0 + GS_OUT_W)
             dqkv = mv.attention_bwd(qkv, att, datt, lse, B, H, N, scale=0.125,
                                     dbias=g[b0 + 3].view(-1))          # to_qkv's bias gradient fused
             dxn1 = dxn2      # reuse
-            mv.gemm(dqkv, wq[b0 + 2][1], dxn1, tag="dgrad", q_out=gq)
+            mv.gemm(dqkv, wq[b0 + 2][1], dxn1, tag="dgrad", q_out=gq, grad_round=gr(s0 + GS_QKV_IN))
             mv.gemm(dqkv, xn1, g[b0 + 2], a_major=1, b_major=1, accumulate=True)
-            wq_grad(b0 + 2)
+            wq_grad(b0 + 2, s0 + GS_QKV_W)
             prev_bias = g[b0 - 1] if l > 0 else None                       # fc2 bias of block l-1
             # dx_h (and prev_bias): masked with block l-1's fc2 site; below block 0 everything (dx too) with the embedding
             # site — the patch wgrad, dpos / dcls and the patch bias all lie behind that dropout
             drop = (drops.fc2(l - 1) if l > 0 else drops.emb()) if drops else None
             dx, dx_h = mv.layernorm_q_bwd(dxn1, x, prm[b0], mean1, rstd1, dres=dx1, q_in=fmt,
                                           dgamma=g[b0], dbeta=g[b0 + 1], dbias_prev=prev_bias,
-                                          dx=dx, dx_f16=dx_h, drop=drop, mask_dx=l == 0)
+                                          dx=dx, dx_f16=dx_h, drop=drop, mask_dx=l == 0, grad_round=gr(s0 + GS_LN1))
             if self.reducer is not None and l % self.bucket_blocks == 0:
                 # one all-reduce per bucket of `bucket_blocks` encoder blocks (their gradient slices are contiguous),
                 # issued as soon as the bucket's last wgrad is enqueued
@@ -445,7 +495,7 @@ class EncoderEngine:
                     mv.set_option("sm_limit_launches", self.dp_limit_launches)
         # ---- patch embedding: dW = dx^T patches (cls rows of `patches` are zero)
         mv.gemm(dx_h, saved["patches"], g[0], a_major=1, b_major=1, accumulate=True)
-        wq_grad(0)
+        wq_grad(0, 10 * cfg.depth)
         mv.set_grad_format(None)
         return self._finish_backward(dx, S, B, N, D)
 

@@ -198,6 +198,32 @@ def dropout(x, drop, *, out=None, out_dtype=None, tag="dropout"):
     return out
 
 
+# ------------------------------------------------------------------ gradient rounding
+def _round_args(grad_round):
+    """grad_round = (seed, offset): seed a 1-element int64 CUDA tensor holding the 64-bit seed, offset the stream's
+    site + (rank << 32) (include/mv_b200.h "gradient rounding stream")."""
+    seed, offset = grad_round
+    _need_cuda(seed)
+    assert seed.dtype == torch.int64 and seed.numel() == 1
+    return ctypes.c_void_p(seed.data_ptr()), ctypes.c_uint64(int(offset))
+
+
+def float_quantize_dev(x, exp, man, grad_round, out=None, out_dtype=torch.float32):
+    """mv_float_quantize_dev: stochastic float_quantize with the seed read from device memory."""
+    _need_cuda(x)
+    x = x.contiguous()
+    if x.dtype != torch.float32:
+        x = x.float()
+    if out is None:
+        out = torch.empty(x.shape, dtype=out_dtype, device=x.device)
+    assert out.is_contiguous() and out.numel() == x.numel()
+    seed, offset = _round_args(grad_round)
+    with _timed("quant_grad", 0.0, x.numel() * (4 + out.element_size())):
+        _check(lib().mv_float_quantize_dev(_ptr(x), _ptr(out), _DT[out.dtype], ctypes.c_int64(x.numel()), int(exp),
+                                           int(man), seed, offset, _stream()), "mv_float_quantize_dev")
+    return out
+
+
 # ------------------------------------------------------------------ fake-quant
 def float_quantize(x, exp, man, rounding="nearest", seed=0, offset=0, out=None,
                    out_dtype=torch.float32):
@@ -283,10 +309,12 @@ def quantize_weight(w, exp, man, out_dtype=torch.float16, transpose=True, out=No
 # ------------------------------------------------------------------------ GEMM
 def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None, out2=None,
          epilogue=EPI_NONE, q_out=None, q_res=None, accumulate=False, rows_per_img=0,
-         M=None, N=None, K=None, tag=None, tile_n=0, cluster=0, colsum=None, transpose_out=False, drop=None):
+         M=None, N=None, K=None, tag=None, tile_n=0, cluster=0, colsum=None, transpose_out=False, drop=None,
+         grad_round=None):
     """out[M,N] = A . B^T over K with the fused epilogue of mv_gemm (include/mv_b200.h).
     a_major/b_major = 0: operand is [M|N, K] (K contiguous); 1: operand is [K, M|N].
-    drop = (seed, p, site): dropout of the output after q_out (seed: int64 [1] CUDA tensor), None: off."""
+    drop = (seed, p, site): dropout of the output after q_out (seed: int64 [1] CUDA tensor), None: off.
+    grad_round = (seed, offset): q_out rounds stochastically (mv_gemm_grad_round), None: nearest."""
     _need_cuda(A, B, out)
     assert A.dim() == 2 and B.dim() == 2 and A.stride(1) == 1 and B.stride(1) == 1
     if M is None:
@@ -341,7 +369,10 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
         if out2 is not None:
             nbytes += M * N * out2.element_size()
     with _timed(kind, flop, nbytes):
-        _check(lib().mv_gemm(ctypes.byref(a), _stream()), "mv_gemm")
+        if grad_round is None:
+            _check(lib().mv_gemm(ctypes.byref(a), _stream()), "mv_gemm")
+        else:
+            _check(lib().mv_gemm_grad_round(ctypes.byref(a), *_round_args(grad_round), _stream()), "mv_gemm_grad_round")
     return out
 
 
@@ -370,9 +401,11 @@ def layernorm_q_fwd(x, gamma, beta, *, q_in=None, q_post=None, out_dtype=torch.f
 
 
 def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=None, dbeta=None,
-                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None, drop=None, mask_dx=False):
+                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None, drop=None, mask_dx=False,
+                    grad_round=None):
     """drop = (seed, p, site): mv_layernorm_q_bwd_drop — dx_f16 and dbias_prev see the masked gradient, dx too when
-    mask_dx."""
+    mask_dx.  grad_round = (seed, offset): the gradient quantiser (set_grad_format) rounds stochastically
+    (mv_layernorm_q_bwd_round)."""
     _need_cuda(dy, x)
     D = x.shape[-1]
     x2, dy2 = x.reshape(-1, D), dy.reshape(-1, D)
@@ -393,7 +426,11 @@ def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=No
                 _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dx),
                 ctypes.c_int64(dx.stride(0)), _ptr(dx_f16), ctypes.c_int64(D),
                 _ptr(dgamma), _ptr(dbeta), _ptr(dbias_prev), rows, D, qi[0], qi[1])
-        if drop is None:
+        if grad_round is not None:
+            dargs = _drop_args(drop) if drop is not None else (None, 0, ctypes.c_uint32(0), ctypes.c_float(0.0))
+            rc = lib().mv_layernorm_q_bwd_round(*args, *dargs, int(bool(mask_dx)), ROUND_STOCHASTIC,
+                                                *_round_args(grad_round), _stream())
+        elif drop is None:
             rc = lib().mv_layernorm_q_bwd(*args, _stream())
         else:
             rc = lib().mv_layernorm_q_bwd_drop(*args, *_drop_args(drop), int(bool(mask_dx)), _stream())

@@ -96,8 +96,9 @@ class DetectionDecoder(nn.Module):
 
 
 class _STEQuant(torch.autograd.Function):
-    """float_quantize (nearest) on the GPU; backward straight-through, or float_quantize (nearest) of the incoming
-    gradient with the plan's gradient format (QPyTorch's backward_number; utils.quantize.QuantPlan.grad)."""
+    """float_quantize (nearest) on the GPU; backward straight-through, or float_quantize of the incoming gradient with
+    the plan's gradient format (QPyTorch's backward_number; utils.quantize.QuantPlan.grad): gfmt = (exp, man) rounds to
+    nearest, (exp, man, seed, offset) stochastically with the gradient rounding stream (mv_float_quantize_dev)."""
 
     @staticmethod
     def forward(ctx, x, exp, man, gfmt):
@@ -106,7 +107,10 @@ class _STEQuant(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        if ctx.gfmt is not None:
+        if ctx.gfmt is not None and len(ctx.gfmt) == 4:
+            e, m, seed, offset = ctx.gfmt
+            g = mv_native.float_quantize_dev(g, e, m, (seed, offset)).to(g.dtype).view(g.shape)
+        elif ctx.gfmt is not None:
             g = mv_native.float_quantize(g, ctx.gfmt[0], ctx.gfmt[1]).to(g.dtype)
         return g, None, None, None
 
@@ -171,6 +175,7 @@ class ViT(nn.Module):
         profile: bool = False,
         q_format: Optional[Union[str, QFormat]] = None,
         backward_format=None,      # extension: (exp, man) gradient format, see ModelQuantizer.prepare_qat
+        backward_rounding: str = "nearest",    # its rounding, "nearest" or "stochastic" (QPyTorch's backward_rounding)
     ):
         super().__init__()
         assert image_size % patch_size == 0, "Image dimensions must be divisible by the patch size."
@@ -204,8 +209,10 @@ class ViT(nn.Module):
             self.decoder = DetectionDecoder(dim, num_classes, num_det_tokens)
 
         self._engine = None
+        self._grad_round_seed = None     # stochastic gradient rounding: the seed of the last encoder forward that drew one
         self.quantizer = ModelQuantizer(self)
-        self.quantizer.prepare_qat(q_format if q_format is not None else QFormat.FP32, backward_format=backward_format)
+        self.quantizer.prepare_qat(q_format if q_format is not None else QFormat.FP32, backward_format=backward_format,
+                                   backward_rounding=backward_rounding)
 
     # ------------------------------------------------------------------ plumbing
     def _invalidate_engine(self):
@@ -258,28 +265,39 @@ class ViT(nn.Module):
             cache[key] = w.view(14 * 14, gh * gw).t().contiguous().to(device)
         return cache[key]
 
-    def _linear(self, holder, x):
+    def _gfmt(self, j):
+        """Gradient format of the decoder's j-th gradient-quantiser site (DECODER_GRAD_SITES): (exp, man), or with
+        stochastic rounding (exp, man, seed, offset) — the seed of this forward, offset = the stream's site of stub j."""
+        plan = self.quantizer.plan
+        seed = self._grad_round_seed
+        if plan.grad is None or seed is None:
+            return plan.grad
+        engine = self._engine
+        return plan.grad + (seed, mv_engine.grad_round_offset(10 * self.depth + 1 + j, engine.rank))
+
+    def _linear(self, holder, x, j=0):
+        """j: gradient-quantiser site of the input stub; the weight's is j + 1."""
         plan = self.quantizer.plan
         lin = _unwrap(holder)
-        y = F.linear(_fq(x, plan.inp, plan.grad), _fq(lin.weight, plan.inp, plan.grad), lin.bias)
+        y = F.linear(_fq(x, plan.inp, self._gfmt(j)), _fq(lin.weight, plan.inp, self._gfmt(j + 1)), lin.bias)
         return _fq(y, plan.out)
 
-    def _norm(self, holder, x):
+    def _norm(self, holder, x, j=0):
         plan = self.quantizer.plan
         ln = _unwrap(holder)
         d = x.shape[-1]
         if (x.is_cuda and x.dtype == torch.float32 and plan.grad is None and ln.elementwise_affine and d % 4 == 0
                 and d <= 1024 and len(ln.normalized_shape) == 1):
             return _FusedNorm.apply(x, ln.weight, ln.bias, plan.inp, plan.out, ln.eps)
-        y = F.layer_norm(_fq(x, plan.inp, plan.grad), ln.normalized_shape, ln.weight, ln.bias, ln.eps)
+        y = F.layer_norm(_fq(x, plan.inp, self._gfmt(j)), ln.normalized_shape, ln.weight, ln.bias, ln.eps)
         return _fq(y, plan.out)
 
     def _decode(self, x, img_hw):
         dec = self.decoder
         if self.task == "classification":                               # vit.py:335-342
-            return self._linear(dec.linear, self._norm(dec.norm, x[:, 0]))
+            return self._linear(dec.linear, self._norm(dec.norm, x[:, 0], 0), 1)
         if self.task == "segmentation":                                 # vit.py:359-374
-            y = self._linear(dec.linear, self._norm(dec.norm, x[:, 1:]))
+            y = self._linear(dec.linear, self._norm(dec.norm, x[:, 1:], 0), 1)
             if self.training and getattr(dec, "fused_loss", False):
                 return y                 # [B, gh*gw, C] for models.losses.upsampled_cross_entropy
             b, hw, c = y.size()
@@ -289,8 +307,8 @@ class ViT(nn.Module):
         # always False (the attribute holds a Module), so det tokens never enter the sequence and
         # the heads read the last num_det_tokens *patch* tokens; reproduced here for parity.
         t = x[:, -dec.num_det_tokens:, :]
-        return {"pred_logits": self._linear(dec.class_embed, t),
-                "pred_boxes": self._linear(dec.bbox_embed, t).sigmoid()}
+        return {"pred_logits": self._linear(dec.class_embed, t, 0),
+                "pred_boxes": self._linear(dec.bbox_embed, t, 2).sigmoid()}
 
     def forward(self, img: torch.Tensor):
         if not img.is_cuda:
@@ -303,6 +321,7 @@ class ViT(nn.Module):
         pos_full = self._pos_full(h // p, w // p)
         x = mv_engine.EncoderFunction.apply(engine, img, pos_full, self.cls_token,
                                             *engine.params)
+        self._grad_round_seed = engine.step_grad_round_seed      # the decoder's stubs round with the encoder's seed
         with engine._range("mlp_head"):
             return self._decode(x, (h, w))
 

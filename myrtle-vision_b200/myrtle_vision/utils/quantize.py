@@ -111,7 +111,9 @@ _FLOAT_FMT = {
 #   gelu: QuantStub in front of GELU
 #   grad: gradient format of the `inp` quantisers (QPyTorch's backward_number; None = straight-through, the only
 #         thing the reference configures, utils/quantize.py:47-72 — see ModelQuantizer.prepare_qat)
-QuantPlan = namedtuple("QuantPlan", ["inp", "out", "ff", "gelu", "grad"], defaults=[None])
+#   grad_rounding: QPyTorch's backward_rounding of those quantisers, "nearest" or "stochastic"
+QuantPlan = namedtuple("QuantPlan", ["inp", "out", "ff", "gelu", "grad", "grad_rounding"], defaults=[None, "nearest"])
+GRAD_ROUNDINGS = ("nearest", "stochastic")
 
 _PLANS = {
     QFormat.FP32: QuantPlan(None, None, None, None),
@@ -155,7 +157,7 @@ class ModelQuantizer:
     def __init__(self, model):
         self.model = model
 
-    def prepare_qat(self, q_format, backward_format=None):
+    def prepare_qat(self, q_format, backward_format=None, backward_rounding="nearest"):
         """Make the model simulate `q_format`.
 
         backward_format (extension; the reference builds every QPyTorch quantiser without a backward_number):
@@ -163,7 +165,14 @@ class ModelQuantizer:
         nearest rounding, to the gradient flowing back through it — qtorch.quant.Quantizer(forward_number,
         backward_number) at the QuantStubs in front of Linear / LayerNorm and at the weight fake-quant.  The
         quantiser sees the gradient as autograd presents it (loss scaling is the caller's, as with the reference's
-        GradScaler): the engine's own power-of-two operand scale is switched off.  FP16_32 only."""
+        GradScaler): the engine's own power-of-two operand scale is switched off.  FP16_32 only.
+
+        backward_rounding: QPyTorch's backward_rounding of those quantisers.  "stochastic" (QPyTorch's default) rounds
+        every gradient-quantiser site with the Philox stream of include/mv_b200.h ("gradient rounding stream") under a
+        seed drawn per training forward; "nearest" (the default here) rounds to nearest.  No effect without
+        backward_format."""
+        if backward_rounding not in GRAD_ROUNDINGS:
+            raise ValueError("backward_rounding must be one of %s, got %r" % (GRAD_ROUNDINGS, backward_rounding))
         if hasattr(self, "q_format") and self.q_format != QFormat.FP32:
             raise ValueError("model already quantized")
         if isinstance(q_format, str):
@@ -181,7 +190,7 @@ class ModelQuantizer:
             e, m = (int(v) for v in backward_format)
             if not (2 <= e <= 8 and 1 <= m <= 22):
                 raise ValueError("backward_format must be (exp_bits in 2..8, man_bits in 1..22)")
-            plan = plan._replace(grad=(e, m))
+            plan = plan._replace(grad=(e, m), grad_rounding=backward_rounding)
         if q_format != QFormat.FP32:
             self._wrap_modules(plan)
         self.plan = plan
