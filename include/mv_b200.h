@@ -114,8 +114,7 @@ typedef struct {
                                    * gradient this GEMM produces, without a second pass over it.  CTA-pair kernel only. */
     int transpose_out;            /* accumulate only: out is [N, M] (pitch ld_out) and receives out[n, m] += acc[m, n] */
     int cluster;                  /* 0 = CTA-pair kernel (tcgen05 cta_group::2, 256 x tile_n cluster tiles; 16-bit operands);
-                                   * 1 = single-CTA kernel (always used for tf32); 2 = single-CTA MMAs with the B tile
-                                   * TMA-multicast across a CTA pair (kept for comparison) */
+                                   * 1 = single-CTA kernel (always used for tf32); any other value is an error */
     /* Dropout (see "dropout mask" below); drop_seed == NULL: off.  The output [M, N] is the site tensor (C = N):
      * value (m, n) is multiplied by keep(seed, site, m*N + n) * drop_scale right after q_out — before the residual
      * add and q_res; in MV_EPI_GELU both gelu(u) and the stored gelu'(u) are multiplied before they are rounded, so the
@@ -125,16 +124,18 @@ typedef struct {
     uint32_t drop_thr;            /* keep when bits16 >= drop_thr; drop_thr = nearbyint(p * 65536) */
     float drop_scale;             /* 1 / (1 - p) in fp32 (0 for p == 1) */
     int drop_site;
+    /* q_out rounded stochastically (see "gradient rounding stream" below); round_seed == NULL: nearest.  Value (m, n) of
+     * the output [M, N] is element i = m*N + n of the site tensor, rounded to (q_out_exp, q_out_man), which must be a
+     * float format, with the bits that mv_float_quantize(..., MV_ROUND_STOCHASTIC, *round_seed, round_offset) uses for
+     * element i.  The rounding takes q_out's place in the epilogue (before the gelu' multiply of MV_EPI_DGELU).  An fp16
+     * output raises the overflow flag where the value before or after rounding does not fit fp16.  CTA-pair kernel only
+     * (16-bit operands, cluster == 0), plain or MV_EPI_DGELU outputs (colsum allowed; no accumulate, out2, residual or
+     * dropout). */
+    const uint64_t* round_seed;   /* device pointer to the 64-bit seed */
+    uint64_t round_offset;
 } mv_gemm_args;
 
 int mv_gemm(const mv_gemm_args* args, void* stream);
-/* mv_gemm with q_out rounded stochastically (see "gradient rounding stream" below): value (m, n) of the output [M, N] is
- * element i = m*N + n of the site tensor, rounded to (q_out_exp, q_out_man) with the bits that mv_float_quantize(...,
- * MV_ROUND_STOCHASTIC, *seed_dev, offset) uses for element i.  The rounding takes q_out's place in the epilogue
- * (before the gelu' multiply of MV_EPI_DGELU).  An fp16 output raises the overflow flag where the value before or
- * after rounding does not fit fp16.  CTA-pair kernel only (16-bit operands, cluster == 0), plain or MV_EPI_DGELU
- * outputs (colsum allowed; no accumulate, out2, residual or dropout).  seed_dev NULL: exactly mv_gemm. */
-int mv_gemm_grad_round(const mv_gemm_args* args, const uint64_t* seed_dev, uint64_t offset, void* stream);
 
 /* ---------------------------------------------------------------- overflow sink
  * Replaces the inf / NaN test of torch.cuda.amp.GradScaler (classification/train.py:167, 259-277; the reference
@@ -169,40 +170,34 @@ int mv_overflow_update(const int* flag_dev, const float* shared_slot_dev, float*
 int mv_layernorm_q_fwd(const float* x, int64_t ld_x, const float* gamma, const float* beta, void* y,
                        int64_t ld_y, int y_dtype, float* mean, float* rstd, int rows, int D, float eps,
                        int q_in_exp, int q_in_man, int q_post_exp, int q_post_man, void* stream);
-/* dy: MV_F32 or MV_F16 (the dgrad GEMM's output).  dx = LN'(dy; q_in(x)) + dres (dres nullable); dx_f16 (nullable) gets an fp16 copy of dx (the next
- * GEMM operand).  dgamma/dbeta/dbias_prev (fp32 [D], nullable) are ACCUMULATED (+=): sum dy*xhat,
- * sum dy, sum dx. */
-int mv_layernorm_q_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
-                       int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
-                       float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
-                       float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
-                       void* stream);
-/* mv_layernorm_q_bwd with a dropout mask (site, see "dropout mask") applied to what feeds the Linear in front of the
- * residual stream: dx_f16 and the dbias_prev column sums get keep * scale times dx; the fp32 dx (the residual
- * gradient) stays unmasked unless mask_dx != 0 (then every output is masked: the embedding site).  seed_dev NULL:
- * exactly mv_layernorm_q_bwd. */
-int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
-                            int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
-                            float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
-                            float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
-                            const uint64_t* seed_dev, int site, uint32_t thr, float scale, int mask_dx, void* stream);
-/* mv_layernorm_q_bwd_drop with the gradient quantiser's rounding per call: rounding MV_ROUND_STOCHASTIC rounds the
- * LayerNorm-input gradient (format of mv_set_grad_format) with the "gradient rounding stream" (round_seed, a device
- * pointer, and round_offset; element i = row*D + c).  MV_ROUND_NEAREST, or no gradient format set: exactly
- * mv_layernorm_q_bwd_drop (seed_dev NULL: no dropout).  Stochastic: fp16 dy. */
-int mv_layernorm_q_bwd_round(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
-                             int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
-                             float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp, float* dgamma,
-                             float* dbeta, float* dbias_prev, int rows, int D, int q_in_exp, int q_in_man,
-                             const uint64_t* seed_dev, int site, uint32_t thr, float scale, int mask_dx,
-                             int rounding, const uint64_t* round_seed, uint64_t round_offset, void* stream);
-/* Gradient quantiser (QPyTorch's Quantizer(backward_number=FloatingPoint(exp, man), backward_rounding="nearest"),
- * qtorch/quant/quant_module.py — an option the reference's NumberFormat.quantizer never sets, utils/quantize.py:47-72;
- * named by the north star).  Process-wide; (0, 0) = off, the default.  When on, mv_layernorm_q_bwd rounds the
- * LayerNorm-input gradient (the backward of the QuantStub in front of the LayerNorm) before it adds dres; the
- * stubs in front of the Linears are the q_out of their dgrad mv_gemm, the weight quantisers a mv_float_quantize over
- * the accumulated weight gradient (the caller passes them: mv_engine.EncoderEngine.backward). */
-int mv_set_grad_format(int exp_bits, int man_bits);
+/* dx = LN'(dy; q_in(x)) [-> q_grad] + dres (dres nullable); dx_f16 (nullable) gets an fp16 copy of dx (the next GEMM
+ * operand).  dgamma/dbeta/dbias_prev (fp32 [D], nullable) are ACCUMULATED (+=): sum dy*xhat, sum dy, sum dx. */
+typedef struct {
+    const void* dy; int dy_dtype; int64_t ld_dy;   /* MV_F32 or MV_F16 (the dgrad GEMM's output) */
+    const float* x; int64_t ld_x;
+    const float* dres; int64_t ld_dres;
+    const float* gamma; const float* mean; const float* rstd;
+    float* dx; int64_t ld_dx;
+    void* dx_f16; int64_t ld_lp;
+    float* dgamma; float* dbeta; float* dbias_prev;
+    int rows, D;
+    int q_in_exp, q_in_man;
+    /* Gradient quantiser (QPyTorch's Quantizer(backward_number=FloatingPoint(exp, man)), qtorch/quant/quant_module.py — an
+     * option the reference's NumberFormat.quantizer never sets, utils/quantize.py:47-72): exp == 0: off; otherwise exp
+     * 2..8, man 1..22.  It rounds the LayerNorm-input gradient (the backward of the QuantStub in front of the LayerNorm)
+     * before dres is added; the stubs in front of the Linears are the q_out of their dgrad mv_gemm, the weight quantisers
+     * a mv_float_quantize over the accumulated weight gradient (the caller passes them: mv_engine.EncoderEngine.backward). */
+    int q_grad_exp, q_grad_man;
+    /* round_seed (device pointer) != NULL: the gradient quantiser rounds stochastically with the "gradient rounding
+     * stream" (element i = row*D + c; see below); NULL: nearest.  No effect without a gradient format. */
+    const uint64_t* round_seed; uint64_t round_offset;
+    /* Dropout (see "dropout mask"); drop_seed == NULL: off.  The mask (site drop_site) is applied to what feeds the Linear
+     * in front of the residual stream: dx_f16 and the dbias_prev column sums get keep * drop_scale times dx; the fp32 dx
+     * (the residual gradient) stays unmasked unless mask_dx != 0 (then every output is masked: the embedding site). */
+    const uint64_t* drop_seed; uint32_t drop_thr; float drop_scale; int drop_site; int mask_dx;
+} mv_layernorm_bwd_args;
+/* The gradient quantiser and dropout take fp16 dy. */
+int mv_layernorm_q_bwd(const mv_layernorm_bwd_args* args, void* stream);
 /* out[c] += sum_r in[r,c]   (bias gradients); in_dtype MV_F16 or MV_F32 */
 int mv_colsum(const void* in, int in_dtype, int64_t ld, int rows, int cols, float* out, void* stream);
 /* img NCHW fp32 -> q(patches) [B*(H/P)*(W/P), P*P*C], (ph,pw,c) minor order (models/vit.py:271-275).

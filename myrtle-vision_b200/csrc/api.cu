@@ -12,7 +12,6 @@ int64_t g_launches = 0;
 int g_opt_quant_ctas = 8;       // grid cap of the elementwise quant kernels, CTAs per SM
 int g_opt_sm_limit = 148, g_opt_sm_limit_launches = 0;   // see persistent_sms() (common.cuh)
 int g_opt_attn_sn = 1;          // short-sequence attention kernels (attention_sn.cu) when N fits
-FloatFmt g_grad_fmt = {0, 0};
 int* g_overflow = nullptr;      // device int registered with mv_set_overflow_flag (NULL: no overflow reporting)
 
 void set_error(const char* fmt, ...) {
@@ -123,16 +122,8 @@ int make_tmap_3d(CUtensorMap* map, const void* ptr, int dtype, uint64_t d0, uint
 }  // namespace mv
 
 extern "C" const char* mv_last_error(void) { return mv::g_err; }
-extern "C" int mv_version(void) { return 102; }
+extern "C" int mv_version(void) { return 103; }
 extern "C" int mv_set_overflow_flag(int* flag_dev) { mv::g_overflow = flag_dev; return 0; }
-extern "C" int mv_set_grad_format(int exp_bits, int man_bits) {
-    if (exp_bits != 0 && (exp_bits < 2 || exp_bits > 8 || man_bits < 1 || man_bits > 22)) {
-        mv::set_error("mv_set_grad_format: unsupported format (%d, %d)", exp_bits, man_bits);
-        return 1;
-    }
-    mv::g_grad_fmt = mv::FloatFmt{exp_bits, exp_bits == 0 ? 0 : man_bits};
-    return 0;
-}
 extern "C" int64_t mv_launch_count(void) { return mv::g_launches; }
 
 extern "C" int mv_set_option(const char* name, int value) {

@@ -44,7 +44,6 @@ inline int persistent_sms() {
 // |value| they convert and raise the flag when it would not fit (>= 65520 rounds past 65504: the container
 // saturates; +-inf included.  NaNs are caught by the final un-scale pass, which tests every parameter gradient).
 extern int* g_overflow;
-extern FloatFmt g_grad_fmt;     // mv_set_grad_format: gradient quantiser of the LayerNorm input stubs ({0, 0} = off)
 constexpr float kHalfOverflow = 65520.0f;
 __device__ __forceinline__ void raise_overflow(int* flag, float amax) {
     if (flag != nullptr && amax >= kHalfOverflow) *flag = 1;
@@ -161,17 +160,6 @@ __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk
 __device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 // ... and written (before the kernel ends)
 __device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-
-// multicast: the tile lands at the same smem offset of every CTA in cta_mask and completes the
-// mbarrier at the same offset in each of them
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const void* tmap, uint64_t* bar, int c0,
-                                               int c1, uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(smem_u32(smem_dst)),
-        "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-        : "memory");
-}
 
 // --------------------------------------------------------------- clusters
 __device__ __forceinline__ uint32_t cluster_ctarank() {
@@ -290,14 +278,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile(
         "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(
             smem_u32(bar))
-        : "memory");
-}
-// same, arriving on the barrier at this offset in every CTA of cta_mask
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile(
-        "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-            smem_u32(bar)),
-        "h"(cta_mask)
         : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() {

@@ -248,11 +248,7 @@ __device__ __forceinline__ void store_out(void* base, int dtype, int64_t row, in
 }
 
 // kEsz: operand element size (2: f16/bf16, kind::f16; 4: tf32-in-fp32, kind::tf32)
-// kCluster: CTA pairs (cluster 2x1x1) work on vertically adjacent tiles that share the B tile; each CTA
-// fetches half of it and TMA-multicasts it into both CTAs' shared memory (halves the L2->SM traffic
-// of B, the bound of these small-K GEMMs).  MMAs stay per-CTA (cta_group::1); a stage is recycled
-// when both CTAs' MMAs have released it (multicast tcgen05.commit onto both empty barriers).
-template <int BN, int kEsz, bool kCluster>
+template <int BN, int kEsz>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
             const GemmDev p) {
@@ -278,22 +274,19 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmap_a);
         tma_prefetch_desc(&tmap_b);
-        for (int s = 0; s < kStages; s++) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], kCluster ? 2 : 1); }
+        for (int s = 0; s < kStages; s++) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
         for (int a = 0; a < 2; a++) { mbar_init(&tmem_full[a], 1); mbar_init(&tmem_empty[a], kEpiWarps); }
         fence_barrier_init();
     }
     if (warp == 1) tmem_alloc<2 * BN>(tmem_slot);
     tc_fence_before();
     __syncthreads();
-    if (kCluster) cluster_sync_all();          // the peer's barriers exist before anything lands on them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
 
-    // work units: (tile pair, k split); both CTAs of a cluster walk the same unit sequence
-    const int ncta = kCluster ? 2 : 1;
-    const int cta_rank = kCluster ? int(cluster_ctarank()) : 0;
-    const int unit0 = blockIdx.x / ncta, unit_stride = gridDim.x / ncta;
-    const int total_units = ((p.m_tiles + ncta - 1) / ncta) * p.n_tiles * p.splits;
+    // work units: (tile, k split)
+    const int unit0 = blockIdx.x, unit_stride = gridDim.x;
+    const int total_units = p.m_tiles * p.n_tiles * p.splits;
 
     if (warp == 0) {
         // ================================ TMA producer ================================
@@ -302,7 +295,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
             for (int u = unit0; u < total_units; u += unit_stride) {
                 const int split = u % p.splits;
                 const int tile = u / p.splits;
-                const int m0 = ((tile / p.n_tiles) * ncta + cta_rank) * BM, n0 = (tile % p.n_tiles) * BN;
+                const int m0 = (tile / p.n_tiles) * BM, n0 = (tile % p.n_tiles) * BN;
                 const int kb0 = split * p.kb_per_split;
                 const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
                 for (int kb = kb0; kb < kb1; kb++) {
@@ -318,21 +311,14 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                             tma_load_2d(sa + c * kMnBoxBytes, &tmap_a, &full_bar[stage], m0 + c * kMnChunk, kb * BK);
                     }
                     if (p.b_major == 0) {
-                        // two half-tiles of BN/2 rows; in cluster mode each CTA fetches one and multicasts it
+                        // two half-tiles of BN/2 rows
 #pragma unroll
-                        for (int c = 0; c < 2; c++) {
-                            uint8_t* dst = sb + c * (BN / 2) * 128;
-                            if (!kCluster) tma_load_2d(dst, &tmap_b, &full_bar[stage], kb * BK, n0 + c * (BN / 2));
-                            else if (c == cta_rank) tma_load_2d_mc(dst, &tmap_b, &full_bar[stage], kb * BK, n0 + c * (BN / 2), 3);
-                        }
+                        for (int c = 0; c < 2; c++)
+                            tma_load_2d(sb + c * (BN / 2) * 128, &tmap_b, &full_bar[stage], kb * BK, n0 + c * (BN / 2));
                     } else {
-                        constexpr int kChunks = BN / kMnChunk;
 #pragma unroll
-                        for (int c = 0; c < kChunks; c++) {
-                            uint8_t* dst = sb + c * kMnBoxBytes;
-                            if (!kCluster) tma_load_2d(dst, &tmap_b, &full_bar[stage], n0 + c * kMnChunk, kb * BK);
-                            else if (c / (kChunks / 2) == cta_rank) tma_load_2d_mc(dst, &tmap_b, &full_bar[stage], n0 + c * kMnChunk, kb * BK, 3);
-                        }
+                        for (int c = 0; c < BN / kMnChunk; c++)
+                            tma_load_2d(sb + c * kMnBoxBytes, &tmap_b, &full_bar[stage], n0 + c * kMnChunk, kb * BK);
                     }
                     if (++stage == kStages) { stage = 0; phase ^= 1; }
                 }
@@ -368,8 +354,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                         if (kEsz == 2) umma_f16(tmem_d, adesc, bdesc, p.idesc, accum);
                         else umma_tf32(tmem_d, adesc, bdesc, p.idesc, accum);
                     }
-                    if (kCluster) umma_commit_mc(&empty_bar[stage], 3);    // both CTAs' producers wait for both MMAs
-                    else umma_commit(&empty_bar[stage]);       // frees the smem slot when the MMAs retire
+                    umma_commit(&empty_bar[stage]);            // frees the smem slot when the MMAs retire
                     if (++stage == kStages) { stage = 0; phase ^= 1; }
                 }
                 umma_commit(&tmem_full[acc]);                  // accumulator ready for the epilogue
@@ -388,7 +373,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
         int acc = 0; uint32_t acc_phase = 0;
         for (int u = unit0; u < total_units; u += unit_stride) {
             const int tile = u / p.splits;
-            const int m0 = ((tile / p.n_tiles) * ncta + cta_rank) * BM, n0 = (tile % p.n_tiles) * BN;
+            const int m0 = (tile / p.n_tiles) * BM, n0 = (tile % p.n_tiles) * BN;
             mbar_wait(&tmem_full[acc], acc_phase);
             tc_fence_after();
             const int m = m0 + quad * 32 + lane;
@@ -511,7 +496,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
     }
     tc_fence_before();
     __syncthreads();
-    if (kCluster) cluster_sync_all();          // no CTA exits while its peer may still write into it
     if (warp == 1) {
         tc_fence_after();
         tmem_dealloc<2 * BN>(tmem_base);
@@ -1285,7 +1269,7 @@ static int launch_gemm2(const CUtensorMap& ta, const CUtensorMap& tb, const Gemm
 using namespace mv;
 
 // CTA-pair path: 16-bit operands, 256 x BN cluster tiles
-static int gemm2_host(const mv_gemm_args* a, void* stream, const SrDev* sr = nullptr) {
+static int gemm2_host(const mv_gemm_args* a, void* stream) {
     constexpr int BK = 64;
     // BN: least padding of N, ties to the wider tile; MN-major B is staged in 64-element chunks per CTA
     int BN = 128, best = -1;
@@ -1352,8 +1336,8 @@ static int gemm2_host(const mv_gemm_args* a, void* stream, const SrDev* sr = nul
              "mv_gemm: dropout needs a plain output (no accumulate, colsum or out2)");
     MV_CHECK(!drop || a->epilogue != MV_EPI_DGELU, "mv_gemm: the gelu' epilogue takes its mask from aux, not from drop_seed");
     p.drop = DropDev{a->drop_seed, a->drop_thr, a->drop_scale, a->drop_site};
-    const bool srnd = sr != nullptr;
-    p.sr = srnd ? *sr : SrDev{nullptr, 0ull};
+    const bool srnd = a->round_seed != nullptr;
+    p.sr = SrDev{a->round_seed, a->round_offset};
     // epilogue variant (epi_chunk<> instantiations in gemm2_kernel); anything else runs the generic path
     {
         auto al = [](const void* q, int bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) == 0; };
@@ -1440,9 +1424,19 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     const bool tf32 = a->a_dtype == MV_F32;
     MV_CHECK(a->a_dtype == a->b_dtype, "mv_gemm: A and B must share one element type (tcgen05 kind::f16 rejects f16 x bf16)");
     if (a->accumulate) MV_CHECK(a->out_dtype == MV_F32, "mv_gemm: accumulate needs an fp32 output");
+    MV_CHECK(a->cluster == 0 || a->cluster == 1, "mv_gemm: cluster %d (0: CTA-pair kernel, 1: single-CTA kernel)", a->cluster);
     MV_CHECK(!a->transpose_out || (a->accumulate && !tf32 && a->cluster == 0),
              "mv_gemm: transpose_out needs accumulate on the CTA-pair kernel (16-bit operands, cluster == 0)");
     if (a->epilogue == MV_EPI_GELU || a->epilogue == MV_EPI_DGELU) MV_CHECK(a->aux != nullptr, "mv_gemm: GELU epilogues need aux");
+    if (a->round_seed != nullptr) {
+        MV_CHECK(!tf32 && a->cluster == 0,
+                 "mv_gemm: stochastic rounding is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
+        MV_CHECK(a->q_out_exp >= 1 && a->q_out_exp <= 8 && a->q_out_man >= 1 && a->q_out_man <= 22,
+                 "mv_gemm: q_out (%d, %d) is not a float format to round stochastically", a->q_out_exp, a->q_out_man);
+        MV_CHECK(!a->accumulate && a->out2 == nullptr && a->drop_seed == nullptr && a->residual == nullptr &&
+                 a->epilogue != MV_EPI_GELU,
+                 "mv_gemm: stochastic rounding needs a plain or gelu' output (no accumulate, out2, dropout, residual or GELU)");
+    }
     if (!tf32 && a->cluster == 0) return gemm2_host(a, stream);      // CTA-pair kernel (default)
     MV_CHECK(a->colsum == nullptr, "mv_gemm: colsum is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
     MV_CHECK(a->drop_seed == nullptr, "mv_gemm: dropout is only fused into the CTA-pair kernel (16-bit operands, cluster == 0); "
@@ -1451,11 +1445,9 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     const int BK = 128 / esz;
     static bool attr_done = false;
     if (!attr_done) {
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<256, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<256>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<256, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<256>::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<256, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<256>::kSmem));
         attr_done = true;
     }
     // 128x256 tiles cut the L2->SM operand traffic per flop by a quarter; use them when N tiles evenly
@@ -1501,55 +1493,13 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     p.drop = DropDev{nullptr, 0u, 0.f, 0};
     p.sr = SrDev{nullptr, 0ull};
 
-    // CTA pairs sharing B through TMA multicast: measured no faster on B200 (the bound is the per-SM
-    // L2->SM ingest, which multicast does not reduce), so it is opt-in (cluster == 2)
-    const bool cluster = !tf32 && p.m_tiles >= 2 && a->cluster == 2;
-    const int ncta = cluster ? 2 : 1;
-    int splits2 = p.splits;
-    if (cluster && a->accumulate) {
-        // re-derive the k split for pair units
-        const int pairs = ((p.m_tiles + 1) / 2) * p.n_tiles;
-        int sp = (kNumSMs / 2) / pairs;
-        if (sp < 1) sp = 1;
-        if (sp > p.kb_total) sp = p.kb_total;
-        p.kb_per_split = (p.kb_total + sp - 1) / sp;
-        p.splits = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
-        splits2 = p.splits;
-    }
-    const int units = ((p.m_tiles + ncta - 1) / ncta) * p.n_tiles * splits2;
-    int grid = units * ncta < kNumSMs ? units * ncta : kNumSMs;
-    grid -= grid % ncta;
+    const int units = p.m_tiles * p.n_tiles * p.splits;
+    const int grid = units < kNumSMs ? units : kNumSMs;
+    const size_t smem = BN == 256 ? GemmCfg<256>::kSmem : GemmCfg<128>::kSmem;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kGemmThreads); cfg.stream = st;
-    cfg.dynamicSmemBytes = BN == 256 ? GemmCfg<256>::kSmem : GemmCfg<128>::kSmem;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = cluster ? 1 : 0;
-    if (tf32) MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<128, 4, false>, ta, tb, p));
-    else if (BN == 256 && cluster) MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<256, 2, true>, ta, tb, p));
-    else if (BN == 256) MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<256, 2, false>, ta, tb, p));
-    else if (cluster) MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<128, 2, true>, ta, tb, p));
-    else MV_CUDA(cudaLaunchKernelEx(&cfg, gemm_kernel<128, 2, false>, ta, tb, p));
+    if (tf32) gemm_kernel<128, 4><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
+    else if (BN == 256) gemm_kernel<256, 2><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
+    else gemm_kernel<128, 2><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
     g_launches++;
     return check_cuda(cudaGetLastError(), "gemm launch");
-}
-
-extern "C" int mv_gemm_grad_round(const mv_gemm_args* a, const uint64_t* seed_dev, uint64_t offset, void* stream) {
-    if (seed_dev == nullptr) return mv_gemm(a, stream);
-    MV_CHECK(a != nullptr, "mv_gemm_grad_round: null args");
-    MV_CHECK(a->a_dtype != MV_F32 && a->cluster == 0,
-             "mv_gemm_grad_round: stochastic rounding is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
-    MV_CHECK(a->q_out_exp >= 1 && a->q_out_exp <= 8 && a->q_out_man >= 1 && a->q_out_man <= 22,
-             "mv_gemm_grad_round: q_out (%d, %d) is not a float format", a->q_out_exp, a->q_out_man);
-    MV_CHECK(!a->accumulate && a->out2 == nullptr && a->drop_seed == nullptr && a->residual == nullptr &&
-             a->epilogue != MV_EPI_GELU,
-             "mv_gemm_grad_round: needs a plain or gelu' output (no accumulate, out2, dropout, residual or GELU)");
-    MV_CHECK(a->M > 0 && a->N > 0 && a->K > 0, "mv_gemm_grad_round: bad shape %dx%dx%d", a->M, a->N, a->K);
-    MV_CHECK(a->A && a->B && a->out, "mv_gemm_grad_round: null operand");
-    MV_CHECK(a->a_dtype == a->b_dtype, "mv_gemm_grad_round: A and B must share one element type");
-    if (a->epilogue == MV_EPI_DGELU) MV_CHECK(a->aux != nullptr, "mv_gemm_grad_round: the gelu' epilogue needs aux");
-    const SrDev sr{seed_dev, offset};
-    return gemm2_host(a, stream, &sr);
 }

@@ -162,7 +162,7 @@ __device__ __forceinline__ float4 unpack_dy(const uint2& u) {
     return make_float4(a.x, a.y, b.x, b.y);
 }
 
-// kGQ: the gradient quantiser of the LayerNorm's input stub (QPyTorch backward_number; mv_set_grad_format) rounds the
+// kGQ: the gradient quantiser of the LayerNorm's input stub (QPyTorch backward_number; q_grad) rounds the
 // LayerNorm-input gradient before the residual gradient is added to it
 // kDrop: dropout mask `drop` on dx_lp and dbias_prev (and on dx when mask_dx): the gradient of the dropped branch that the
 // residual stream's producer receives.  A lane owns float4 c = lane + 32 i; with D % 8 == 0 lanes 2k / 2k+1 hold the two
@@ -531,78 +531,44 @@ static int launch_ln_fwd(const float* x, int64_t ld_x, const float* gamma, const
     return check_cuda(cudaGetLastError(), "ln fwd launch");
 }
 
+// Every ln_bwd_kernel instantiation may take the shared memory of the widest row (D = 128 * kLnMaxVec); the attribute is
+// set on its first launch.
+template <auto kKernel>
+static decltype(kKernel) ln_bwd_ready() {
+    static const cudaError_t once = cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                         kLnWarps * 3 * 128 * kLnMaxVec * 4);
+    (void)once;
+    return kKernel;
+}
+
 template <int NV>
-static int launch_ln_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x, const float* dres,
-                         int64_t ld_dres, const float* gamma, const float* mean, const float* rstd,
-                         float* dx, int64_t ld_dx, void* dx_lp, int64_t ld_lp, float* dgamma, float* dbeta,
-                         float* dbias_prev, int rows, int D, FloatFmt q_in, cudaStream_t st,
-                         const DropDev* drop = nullptr, int mask_dx = 0, const SrDev* sr = nullptr) {
-    int grid = (rows + kLnWarps - 1) / kLnWarps;
+static int launch_ln_bwd(const mv_layernorm_bwd_args& a, cudaStream_t st) {
+    int grid = (a.rows + kLnWarps - 1) / kLnWarps;
     const int cap = persistent_sms() * 2;
     if (grid > cap) grid = cap;
-    const size_t smem = size_t(kLnWarps) * 3 * D * sizeof(float);
-    if (sr != nullptr) {
-        // stochastic gradient rounding: fp16 dy, with or without dropout
-        static bool attr_sr = false;
-        if (!attr_sr) {
-            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-            attr_sr = true;
-        }
-        if (dy_dtype != MV_F16) { set_error("mv_layernorm_q_bwd_round: dy must be fp16"); return 1; }
-        const DropDev d = drop != nullptr ? *drop : DropDev{nullptr, 0u, 0.f, 0};
-        if (drop != nullptr)
-            ln_bwd_kernel<NV, __half, true, true, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
-                                                                                         dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
-                                                                                         q_in, g_overflow, g_grad_fmt, d, mask_dx, *sr);
-        else
-            ln_bwd_kernel<NV, __half, true, false, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
-                                                                                          dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
-                                                                                          q_in, g_overflow, g_grad_fmt, d, 0, *sr);
-        g_launches++;
-        return check_cuda(cudaGetLastError(), "ln bwd (stochastic rounding) launch");
+    const size_t smem = size_t(kLnWarps) * 3 * a.D * sizeof(float);
+    const FloatFmt q_in{a.q_in_exp, a.q_in_man}, q_grad{a.q_grad_exp, a.q_grad_man};
+    const DropDev drop{a.drop_seed, a.drop_thr, a.drop_scale, a.drop_site};
+    const SrDev sr{a.round_seed, a.round_offset};
+    auto launch = [&](auto kernel, auto* dy) {
+        kernel<<<grid, kLnWarps * 32, smem, st>>>(dy, a.ld_dy, a.x, a.ld_x, a.dres, a.ld_dres, a.gamma, a.mean, a.rstd, a.dx,
+                                                  a.ld_dx, (__half*)a.dx_f16, a.ld_lp, a.dgamma, a.dbeta, a.dbias_prev, a.rows,
+                                                  a.D, q_in, g_overflow, q_grad, drop, a.mask_dx, sr);
+    };
+    // kGQ: gradient quantiser; kDrop: dropout; kSR: the quantiser rounds stochastically (a round_seed without a
+    // gradient format has no effect).  Only the plain kernel also takes fp32 dy.
+    const bool gq = a.q_grad_exp != 0, dp = a.drop_seed != nullptr, sr_on = gq && a.round_seed != nullptr;
+    if (a.dy_dtype == MV_F32) {
+        launch(ln_bwd_ready<ln_bwd_kernel<NV, float>>(), (const float*)a.dy);
+    } else {
+        const auto kernel = sr_on ? (dp ? ln_bwd_ready<ln_bwd_kernel<NV, __half, true, true, true>>()
+                                        : ln_bwd_ready<ln_bwd_kernel<NV, __half, true, false, true>>())
+                          : dp    ? (gq ? ln_bwd_ready<ln_bwd_kernel<NV, __half, true, true>>()
+                                        : ln_bwd_ready<ln_bwd_kernel<NV, __half, false, true>>())
+                          : gq    ? ln_bwd_ready<ln_bwd_kernel<NV, __half, true>>()
+                                  : ln_bwd_ready<ln_bwd_kernel<NV, __half>>();
+        launch(kernel, (const __half*)a.dy);
     }
-    if (drop != nullptr) {
-        // dropout variants: fp16 dy (the dgrad GEMM's output), with or without the gradient quantiser
-        static bool attr_drop = false;
-        if (!attr_drop) {
-            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-            attr_drop = true;
-        }
-        if (dy_dtype != MV_F16) { set_error("mv_layernorm_q_bwd_drop: dy must be fp16"); return 1; }
-        if (g_grad_fmt.exp_bits != 0)
-            ln_bwd_kernel<NV, __half, true, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
-                                                                                   dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
-                                                                                   q_in, g_overflow, g_grad_fmt, *drop, mask_dx);
-        else
-            ln_bwd_kernel<NV, __half, false, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd,
-                                                                                    dx, ld_dx, (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D,
-                                                                                    q_in, g_overflow, FloatFmt{0, 0}, *drop, mask_dx);
-        g_launches++;
-        return check_cuda(cudaGetLastError(), "ln bwd (dropout) launch");
-    }
-    static bool attr_done = false;
-    if (!attr_done) {
-        cudaFuncSetAttribute(ln_bwd_kernel<NV, __half>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-        cudaFuncSetAttribute(ln_bwd_kernel<NV, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-        attr_done = true;
-    }
-    if (g_grad_fmt.exp_bits != 0) {      // gradient quantiser on (never in the shipped configurations): fp16 dy only
-        static bool attr_gq = false;
-        if (!attr_gq) {
-            cudaFuncSetAttribute(ln_bwd_kernel<NV, __half, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLnWarps * 3 * 128 * kLnMaxVec * 4);
-            attr_gq = true;
-        }
-        if (dy_dtype != MV_F16) { set_error("mv_layernorm_q_bwd: the gradient quantiser (mv_set_grad_format) takes fp16 dy"); return 1; }
-        ln_bwd_kernel<NV, __half, true><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx,
-                                                                          (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D, q_in, g_overflow, g_grad_fmt);
-    } else if (dy_dtype == MV_F16)
-        ln_bwd_kernel<NV, __half><<<grid, kLnWarps * 32, smem, st>>>((const __half*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx,
-                                                                    (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D, q_in, g_overflow);
-    else
-        ln_bwd_kernel<NV, float><<<grid, kLnWarps * 32, smem, st>>>((const float*)dy, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx,
-                                                                   (__half*)dx_lp, ld_lp, dgamma, dbeta, dbias_prev, rows, D, q_in, g_overflow);
     g_launches++;
     return check_cuda(cudaGetLastError(), "ln bwd launch");
 }
@@ -741,85 +707,27 @@ extern "C" int mv_layernorm_q_fwd(const float* x, int64_t ld_x, const float* gam
     }
 }
 
-extern "C" int mv_layernorm_q_bwd(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x,
-                                  const float* dres, int64_t ld_dres, const float* gamma, const float* mean,
-                                  const float* rstd, float* dx, int64_t ld_dx, void* dx_bf16, int64_t ld_lp,
-                                  float* dgamma, float* dbeta, float* dbias_prev, int rows, int D,
-                                  int q_in_exp, int q_in_man, void* stream) {
-    MV_CHECK(rows >= 0 && D > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd: D=%d unsupported", D);
-    MV_CHECK(dy_dtype == MV_F16 || dy_dtype == MV_F32, "mv_layernorm_q_bwd: dy must be fp16 or fp32");
-    MV_CHECK(ld_dy % 4 == 0 && ld_x % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_lp % 4 == 0, "mv_layernorm_q_bwd: row pitches must be multiples of 4");
-    if (rows == 0) return 0;
-    const FloatFmt qi{q_in_exp, q_in_man};
+extern "C" int mv_layernorm_q_bwd(const mv_layernorm_bwd_args* args, void* stream) {
+    MV_CHECK(args != nullptr, "mv_layernorm_q_bwd: null args");
+    const mv_layernorm_bwd_args& a = *args;
+    MV_CHECK(a.rows >= 0 && a.D > 0 && a.D % 4 == 0 && a.D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd: D=%d unsupported", a.D);
+    MV_CHECK(a.dy_dtype == MV_F16 || a.dy_dtype == MV_F32, "mv_layernorm_q_bwd: dy must be fp16 or fp32");
+    MV_CHECK(a.ld_dy % 4 == 0 && a.ld_x % 4 == 0 && a.ld_dx % 4 == 0 && a.ld_dres % 4 == 0 && a.ld_lp % 4 == 0,
+             "mv_layernorm_q_bwd: row pitches must be multiples of 4");
+    MV_CHECK(a.q_grad_exp == 0 || (a.q_grad_exp >= 2 && a.q_grad_exp <= 8 && a.q_grad_man >= 1 && a.q_grad_man <= 22),
+             "mv_layernorm_q_bwd: unsupported gradient format (%d, %d)", a.q_grad_exp, a.q_grad_man);
+    MV_CHECK(a.drop_seed == nullptr || a.drop_thr <= 65536u, "mv_layernorm_q_bwd: dropout threshold %u above 65536", a.drop_thr);
+    MV_CHECK((a.q_grad_exp == 0 && a.drop_seed == nullptr) || a.dy_dtype == MV_F16,
+             "mv_layernorm_q_bwd: the gradient quantiser and dropout take fp16 dy");
+    if (a.rows == 0) return 0;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const int nv = (D / 4 + 31) / 32;
-    switch (nv) {
-        case 1: return launch_ln_bwd<1>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-        case 2: return launch_ln_bwd<2>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-        case 3: return launch_ln_bwd<3>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-        case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-        case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-        default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_bf16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st);
-    }
-}
-
-extern "C" int mv_layernorm_q_bwd_drop(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x,
-                                       const float* dres, int64_t ld_dres, const float* gamma, const float* mean,
-                                       const float* rstd, float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp,
-                                       float* dgamma, float* dbeta, float* dbias_prev, int rows, int D,
-                                       int q_in_exp, int q_in_man, const uint64_t* seed_dev, int site, uint32_t thr,
-                                       float scale, int mask_dx, void* stream) {
-    if (seed_dev == nullptr)
-        return mv_layernorm_q_bwd(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp,
-                                  dgamma, dbeta, dbias_prev, rows, D, q_in_exp, q_in_man, stream);
-    MV_CHECK(rows >= 0 && D > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd_drop: D=%d unsupported", D);
-    MV_CHECK(ld_dy % 4 == 0 && ld_x % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_lp % 4 == 0, "mv_layernorm_q_bwd_drop: row pitches must be multiples of 4");
-    MV_CHECK(thr <= 65536u, "mv_layernorm_q_bwd_drop: threshold %u above 65536", thr);
-    if (rows == 0) return 0;
-    const FloatFmt qi{q_in_exp, q_in_man};
-    const DropDev d{seed_dev, thr, scale, site};
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const int nv = (D / 4 + 31) / 32;
-    switch (nv) {
-        case 1: return launch_ln_bwd<1>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-        case 2: return launch_ln_bwd<2>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-        case 3: return launch_ln_bwd<3>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-        case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-        case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-        default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, &d, mask_dx);
-    }
-}
-
-extern "C" int mv_layernorm_q_bwd_round(const void* dy, int dy_dtype, int64_t ld_dy, const float* x, int64_t ld_x,
-                                        const float* dres, int64_t ld_dres, const float* gamma, const float* mean,
-                                        const float* rstd, float* dx, int64_t ld_dx, void* dx_f16, int64_t ld_lp,
-                                        float* dgamma, float* dbeta, float* dbias_prev, int rows, int D,
-                                        int q_in_exp, int q_in_man, const uint64_t* seed_dev, int site, uint32_t thr,
-                                        float scale, int mask_dx, int rounding, const uint64_t* round_seed,
-                                        uint64_t round_offset, void* stream) {
-    MV_CHECK(rounding == MV_ROUND_NEAREST || rounding == MV_ROUND_STOCHASTIC, "mv_layernorm_q_bwd_round: rounding %d", rounding);
-    if (rounding == MV_ROUND_NEAREST || g_grad_fmt.exp_bits == 0)
-        return mv_layernorm_q_bwd_drop(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp,
-                                       dgamma, dbeta, dbias_prev, rows, D, q_in_exp, q_in_man, seed_dev, site, thr, scale,
-                                       mask_dx, stream);
-    MV_CHECK(round_seed != nullptr, "mv_layernorm_q_bwd_round: stochastic rounding needs round_seed");
-    MV_CHECK(rows >= 0 && D > 0 && D % 4 == 0 && D <= 128 * kLnMaxVec, "mv_layernorm_q_bwd_round: D=%d unsupported", D);
-    MV_CHECK(ld_dy % 4 == 0 && ld_x % 4 == 0 && ld_dx % 4 == 0 && ld_dres % 4 == 0 && ld_lp % 4 == 0, "mv_layernorm_q_bwd_round: row pitches must be multiples of 4");
-    MV_CHECK(thr <= 65536u, "mv_layernorm_q_bwd_round: threshold %u above 65536", thr);
-    if (rows == 0) return 0;
-    const FloatFmt qi{q_in_exp, q_in_man};
-    const DropDev d{seed_dev, thr, scale, site};
-    const DropDev* dp = seed_dev != nullptr ? &d : nullptr;
-    const SrDev sr{round_seed, round_offset};
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const int nv = (D / 4 + 31) / 32;
-    switch (nv) {
-        case 1: return launch_ln_bwd<1>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
-        case 2: return launch_ln_bwd<2>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
-        case 3: return launch_ln_bwd<3>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
-        case 4: return launch_ln_bwd<4>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
-        case 5: case 6: return launch_ln_bwd<6>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
-        default: return launch_ln_bwd<8>(dy, dy_dtype, ld_dy, x, ld_x, dres, ld_dres, gamma, mean, rstd, dx, ld_dx, dx_f16, ld_lp, dgamma, dbeta, dbias_prev, rows, D, qi, st, dp, mask_dx, &sr);
+    switch ((a.D / 4 + 31) / 32) {
+        case 1: return launch_ln_bwd<1>(a, st);
+        case 2: return launch_ln_bwd<2>(a, st);
+        case 3: return launch_ln_bwd<3>(a, st);
+        case 4: return launch_ln_bwd<4>(a, st);
+        case 5: case 6: return launch_ln_bwd<6>(a, st);
+        default: return launch_ln_bwd<8>(a, st);
     }
 }
 

@@ -431,7 +431,6 @@ class EncoderEngine:
         # quantiser a pass over the accumulated weight gradient (before the data-parallel reduction, as autograd
         # would apply it to the local gradient)
         gq = self.gfmt
-        mv.set_grad_format(gq)
         # stochastic rounding (QuantPlan.grad_rounding): every site rounds with the stream of include/mv_b200.h under
         # the seed its forward drew; gr(site) is the grad_round argument of the mv_native calls, None: nearest
         seed, rank = saved.get("grad_round"), self.rank
@@ -465,7 +464,7 @@ class EncoderEngine:
             # dx1_h and to_out's bias gradient: the masked gradient of the to_out branch (dropout site of to_out)
             dx1, dx1_h = mv.layernorm_q_bwd(dxn2, x1, prm[b0 + 6], mean2, rstd2, dres=dx, q_in=fmt,
                                             dgamma=g[b0 + 6], dbeta=g[b0 + 7], dbias_prev=g[b0 + 5],
-                                            drop=drops and drops.proj(l), grad_round=gr(s0 + GS_LN2))
+                                            q_grad=gq, drop=drops and drops.proj(l), grad_round=gr(s0 + GS_LN2))
             # ---- Attention
             datt = torch.empty(M, D, dtype=f16, device=dev)
             mv.gemm(dx1_h, wq[b0 + 4][1], datt, tag="dgrad", q_out=gq, grad_round=gr(s0 + GS_OUT_IN))
@@ -483,7 +482,8 @@ class EncoderEngine:
             drop = (drops.fc2(l - 1) if l > 0 else drops.emb()) if drops else None
             dx, dx_h = mv.layernorm_q_bwd(dxn1, x, prm[b0], mean1, rstd1, dres=dx1, q_in=fmt,
                                           dgamma=g[b0], dbeta=g[b0 + 1], dbias_prev=prev_bias,
-                                          dx=dx, dx_f16=dx_h, drop=drop, mask_dx=l == 0, grad_round=gr(s0 + GS_LN1))
+                                          dx=dx, dx_f16=dx_h, q_grad=gq, drop=drop, mask_dx=l == 0,
+                                          grad_round=gr(s0 + GS_LN1))
             if self.reducer is not None and l % self.bucket_blocks == 0:
                 # one all-reduce per bucket of `bucket_blocks` encoder blocks (their gradient slices are contiguous),
                 # issued as soon as the bucket's last wgrad is enqueued
@@ -496,7 +496,6 @@ class EncoderEngine:
         # ---- patch embedding: dW = dx^T patches (cls rows of `patches` are zero)
         mv.gemm(dx_h, saved["patches"], g[0], a_major=1, b_major=1, accumulate=True)
         wq_grad(0, 10 * cfg.depth)
-        mv.set_grad_format(None)
         return self._finish_backward(dx, S, B, N, D)
 
     def _finish_backward(self, dx, S, B, N, D):

@@ -45,6 +45,25 @@ class GemmArgs(ctypes.Structure):
         ("cluster", ctypes.c_int),
         ("drop_seed", ctypes.c_void_p), ("drop_thr", ctypes.c_uint32), ("drop_scale", ctypes.c_float),
         ("drop_site", ctypes.c_int),
+        ("round_seed", ctypes.c_void_p), ("round_offset", ctypes.c_uint64),
+    ]
+
+
+class LayerNormBwdArgs(ctypes.Structure):
+    _fields_ = [
+        ("dy", ctypes.c_void_p), ("dy_dtype", ctypes.c_int), ("ld_dy", ctypes.c_int64),
+        ("x", ctypes.c_void_p), ("ld_x", ctypes.c_int64),
+        ("dres", ctypes.c_void_p), ("ld_dres", ctypes.c_int64),
+        ("gamma", ctypes.c_void_p), ("mean", ctypes.c_void_p), ("rstd", ctypes.c_void_p),
+        ("dx", ctypes.c_void_p), ("ld_dx", ctypes.c_int64),
+        ("dx_f16", ctypes.c_void_p), ("ld_lp", ctypes.c_int64),
+        ("dgamma", ctypes.c_void_p), ("dbeta", ctypes.c_void_p), ("dbias_prev", ctypes.c_void_p),
+        ("rows", ctypes.c_int), ("D", ctypes.c_int),
+        ("q_in_exp", ctypes.c_int), ("q_in_man", ctypes.c_int),
+        ("q_grad_exp", ctypes.c_int), ("q_grad_man", ctypes.c_int),
+        ("round_seed", ctypes.c_void_p), ("round_offset", ctypes.c_uint64),
+        ("drop_seed", ctypes.c_void_p), ("drop_thr", ctypes.c_uint32), ("drop_scale", ctypes.c_float),
+        ("drop_site", ctypes.c_int), ("mask_dx", ctypes.c_int),
     ]
 
 
@@ -140,12 +159,6 @@ def set_overflow_flag(flag):
         _need_cuda(flag)
         assert flag.dtype == torch.int32 and flag.numel() >= 1
     _check(lib().mv_set_overflow_flag(_ptr(flag)), "mv_set_overflow_flag")
-
-
-def set_grad_format(fmt):
-    """Gradient quantiser of the LayerNorm input stubs (mv_set_grad_format); None = off."""
-    e, m = (0, 0) if fmt is None else fmt
-    _check(lib().mv_set_grad_format(int(e), int(m)), "mv_set_grad_format")
 
 
 def overflow_update(flag, state, shared_slot=None, backoff=1.0 / 16, growth=2.0, growth_interval=2000,
@@ -313,8 +326,9 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
          grad_round=None):
     """out[M,N] = A . B^T over K with the fused epilogue of mv_gemm (include/mv_b200.h).
     a_major/b_major = 0: operand is [M|N, K] (K contiguous); 1: operand is [K, M|N].
+    cluster = 0: CTA-pair kernel (16-bit operands), 1: single-CTA kernel (always used for tf32).
     drop = (seed, p, site): dropout of the output after q_out (seed: int64 [1] CUDA tensor), None: off.
-    grad_round = (seed, offset): q_out rounds stochastically (mv_gemm_grad_round), None: nearest."""
+    grad_round = (seed, offset): q_out rounds stochastically, None: nearest."""
     _need_cuda(A, B, out)
     assert A.dim() == 2 and B.dim() == 2 and A.stride(1) == 1 and B.stride(1) == 1
     if M is None:
@@ -353,6 +367,9 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
     if drop is not None:
         seed, site, thr, scale = _drop_args(drop)
         a.drop_seed, a.drop_thr, a.drop_scale, a.drop_site = seed.value, thr.value, scale.value, site
+    if grad_round is not None:
+        seed, offset = _round_args(grad_round)
+        a.round_seed, a.round_offset = seed.value, offset.value
     kind = "gemm_wgrad" if accumulate else ("gemm_dgrad" if epilogue == EPI_DGELU or tag == "dgrad"
                                             else "gemm_fwd")
     flop = nbytes = 0.0
@@ -369,10 +386,7 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
         if out2 is not None:
             nbytes += M * N * out2.element_size()
     with _timed(kind, flop, nbytes):
-        if grad_round is None:
-            _check(lib().mv_gemm(ctypes.byref(a), _stream()), "mv_gemm")
-        else:
-            _check(lib().mv_gemm_grad_round(ctypes.byref(a), *_round_args(grad_round), _stream()), "mv_gemm_grad_round")
+        _check(lib().mv_gemm(ctypes.byref(a), _stream()), "mv_gemm")
     return out
 
 
@@ -401,11 +415,11 @@ def layernorm_q_fwd(x, gamma, beta, *, q_in=None, q_post=None, out_dtype=torch.f
 
 
 def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=None, dbeta=None,
-                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None, drop=None, mask_dx=False,
+                    dbias_prev=None, want_f16=True, dx=None, dx_f16=None, tag=None, q_grad=None, drop=None, mask_dx=False,
                     grad_round=None):
-    """drop = (seed, p, site): mv_layernorm_q_bwd_drop — dx_f16 and dbias_prev see the masked gradient, dx too when
-    mask_dx.  grad_round = (seed, offset): the gradient quantiser (set_grad_format) rounds stochastically
-    (mv_layernorm_q_bwd_round)."""
+    """mv_layernorm_q_bwd (include/mv_b200.h).  q_grad = (exp, man): the gradient quantiser rounds the LayerNorm-input
+    gradient, None: off.  drop = (seed, p, site): dx_f16 and dbias_prev see the masked gradient, dx too when mask_dx.
+    grad_round = (seed, offset): q_grad rounds stochastically, None: nearest.  q_grad and drop take fp16 dy."""
     _need_cuda(dy, x)
     D = x.shape[-1]
     x2, dy2 = x.reshape(-1, D), dy.reshape(-1, D)
@@ -416,24 +430,24 @@ def layernorm_q_bwd(dy, x, gamma, mean, rstd, *, dres=None, q_in=None, dgamma=No
     if want_f16 and dx_f16 is None:
         dx_f16 = torch.empty(rows, D, dtype=torch.float16, device=x.device)
     dres2 = dres.reshape(-1, D) if dres is not None else None
-    qi = _fmt(q_in)
     # x 4 + dy + dres 4 read, dx 4 + fp16 copy 2 written
     with _timed(tag or "ln_bwd", 0.0, rows * D * (4 + dy2.element_size() + (4 if dres is not None else 0) + 4
                                             + (2 if dx_f16 is not None else 0))):
-        args = (_ptr(dy2), _DT[dy2.dtype], ctypes.c_int64(dy2.stride(0)), _ptr(x2),
-                ctypes.c_int64(x2.stride(0)), _ptr(dres2),
-                ctypes.c_int64(dres2.stride(0) if dres2 is not None else D),
-                _ptr(gamma), _ptr(mean), _ptr(rstd), _ptr(dx),
-                ctypes.c_int64(dx.stride(0)), _ptr(dx_f16), ctypes.c_int64(D),
-                _ptr(dgamma), _ptr(dbeta), _ptr(dbias_prev), rows, D, qi[0], qi[1])
+        a = LayerNormBwdArgs(
+            dy=dy2.data_ptr(), dy_dtype=_DT[dy2.dtype], ld_dy=dy2.stride(0), x=x2.data_ptr(), ld_x=x2.stride(0),
+            dres=_ptr(dres2), ld_dres=dres2.stride(0) if dres2 is not None else D,
+            gamma=_ptr(gamma), mean=_ptr(mean), rstd=_ptr(rstd), dx=dx.data_ptr(), ld_dx=dx.stride(0),
+            dx_f16=_ptr(dx_f16), ld_lp=D, dgamma=_ptr(dgamma), dbeta=_ptr(dbeta), dbias_prev=_ptr(dbias_prev),
+            rows=rows, D=D, mask_dx=int(bool(mask_dx)))
+        a.q_in_exp, a.q_in_man = _fmt(q_in)
+        a.q_grad_exp, a.q_grad_man = _fmt(q_grad)
         if grad_round is not None:
-            dargs = _drop_args(drop) if drop is not None else (None, 0, ctypes.c_uint32(0), ctypes.c_float(0.0))
-            rc = lib().mv_layernorm_q_bwd_round(*args, *dargs, int(bool(mask_dx)), ROUND_STOCHASTIC,
-                                                *_round_args(grad_round), _stream())
-        elif drop is None:
-            rc = lib().mv_layernorm_q_bwd(*args, _stream())
-        else:
-            rc = lib().mv_layernorm_q_bwd_drop(*args, *_drop_args(drop), int(bool(mask_dx)), _stream())
+            seed, offset = _round_args(grad_round)
+            a.round_seed, a.round_offset = seed.value, offset.value
+        if drop is not None:
+            seed, site, thr, scale = _drop_args(drop)
+            a.drop_seed, a.drop_thr, a.drop_scale, a.drop_site = seed.value, thr.value, scale.value, site
+        rc = lib().mv_layernorm_q_bwd(ctypes.byref(a), _stream())
     _check(rc, "mv_layernorm_q_bwd")
     return dx, dx_f16
 

@@ -31,6 +31,23 @@ def test_header_declares_the_expected_surface():
         assert s in syms
 
 
+def declared_fields(struct):
+    text = open(os.path.join(ROOT, "include", "mv_b200.h")).read()
+    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+    body = re.search(r"typedef struct \{([^}]*)\} %s;" % struct, text).group(1)
+    names = []
+    for decl in filter(None, (d.strip() for d in body.split(";"))):
+        first, *rest = decl.split(",")
+        names += [re.findall(r"\w+", first)[-1]] + [r.strip() for r in rest]
+    return names
+
+
+@pytest.mark.parametrize("struct,cls", [("mv_gemm_args", "GemmArgs"), ("mv_layernorm_bwd_args", "LayerNormBwdArgs")])
+def test_ctypes_structs_mirror_the_header(struct, cls):
+    import mv_native
+    assert [f[0] for f in getattr(mv_native, cls)._fields_] == declared_fields(struct)
+
+
 def test_every_declared_symbol_is_exported(lib):
     for s in declared_symbols():
         assert hasattr(lib, s), "libmv_b200.so does not export " + s

@@ -25,11 +25,12 @@ def test_probability_range_and_stream_parameters():
             mv_engine.EngineConfig(128, 2, 256, 2, 16, None, dropout=bad)
 
 
-def test_gemm_args_carry_the_dropout_fields_last():
+def test_gemm_args_end_with_the_dropout_and_rounding_fields():
     import mv_native as mv
     names = [f[0] for f in mv.GemmArgs._fields_]
-    assert names[-4:] == ["drop_seed", "drop_thr", "drop_scale", "drop_site"]
+    assert names[-6:] == ["drop_seed", "drop_thr", "drop_scale", "drop_site", "round_seed", "round_offset"]
     assert mv.GemmArgs().drop_seed is None                      # zero-initialised: off
+    assert mv.GemmArgs().round_seed is None                     # zero-initialised: nearest
 
 
 def test_oracle_mask_is_the_declared_stream():

@@ -126,7 +126,7 @@ def test_fused_site_raises_the_overflow_flag_on_saturation():
 @pytest.mark.parametrize("fmt", FORMATS)
 @pytest.mark.parametrize("D", [384, 200])
 @pytest.mark.parametrize("dropout", [False, True])
-def test_layernorm_backward_site(fmt, D, dropout):
+def test_layernorm_backward_site_with_q_grad(fmt, D, dropout):
     """The LN-input stub rounds LN'(dy) before dres is added: dx = q(LN'(dy)) + dres, dx_f16 its (masked) copy."""
     import mv_native as mv
     torch.manual_seed(D)
@@ -140,18 +140,47 @@ def test_layernorm_backward_site(fmt, D, dropout):
     q = mv.float_quantize_dev(ln, fmt[0], fmt[1], gr)
     drop = (seed_tensor(55), 0.1, 9) if dropout else None
     bp = torch.zeros(D, device=dev)
-    mv.set_grad_format(fmt)
-    try:
-        dx, h = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10), dbias_prev=bp, drop=drop,
-                                   grad_round=gr)
-    finally:
-        mv.set_grad_format(None)
+    dx, h = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10), dbias_prev=bp, q_grad=fmt, drop=drop,
+                               grad_round=gr)
     want = q + dres
     assert torch.equal(dx, want)
     m = dropout_oracle.dropout_mask((rows, D), 0.1, 55, 9).to(dev) if dropout else torch.ones_like(want)
     assert torch.equal(h, (want * m).half())
     ws = (want.double() * m.double()).sum(0)
     assert float((bp.double() - ws).abs().max()) <= 1e-5 * float(ws.abs().max())
+
+
+def test_a_failed_backward_leaves_no_gradient_format_behind(monkeypatch):
+    """The gradient format is an argument of each LayerNorm-backward call, not process state: after a backward with
+    backward_format raises part-way, a LayerNorm backward without q_grad, on fp32 dy, runs and is unrounded."""
+    import mv_native as mv
+    case = CASES["classification"]
+    m, _ = build(case, 3, rounding="nearest")
+    img, tgt = make_inputs("classification", case, 3)
+    loss = F.cross_entropy(m(img.to(dev)), tgt.to(dev)) * 65536.0
+    gemm, calls = mv.gemm, []
+
+    def failing_gemm(*args, **kwargs):
+        calls.append(kwargs.get("tag"))
+        if len(calls) == 5:                              # to_out's dgrad: after the last block's LN2 backward
+            raise mv.MvError("injected failure")
+        return gemm(*args, **kwargs)
+
+    monkeypatch.setattr(mv, "gemm", failing_gemm)
+    with pytest.raises(mv.MvError, match="injected failure"):
+        loss.backward()
+    monkeypatch.undo()
+    assert len(calls) == 5
+    torch.manual_seed(4)
+    rows, D = 1003, 192
+    x = torch.randn(rows, D, device=dev) * 2
+    g = 1 + 0.1 * torch.randn(D, device=dev); b = 0.1 * torch.randn(D, device=dev)
+    _, mean, rstd = mv.layernorm_q_fwd(x, g, b, q_in=(5, 10), q_post=(5, 10))
+    dy = torch.randn(rows, D, device=dev)
+    dx, _ = mv.layernorm_q_bwd(dy, x, g, mean, rstd, q_in=(5, 10), want_f16=False)
+    xr = mv.float_quantize(x, 5, 10).double().requires_grad_(True)
+    F.layer_norm(xr, (D,), g.double(), b.double(), 1e-5).backward(dy.double())
+    assert float((dx.double() - xr.grad).abs().max()) <= 1e-6 * float(xr.grad.abs().max())
 
 
 # ------------------------------------------------------------------------------------------------ unbiasedness

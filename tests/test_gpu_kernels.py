@@ -184,8 +184,8 @@ def test_layernorm_q(D):
     assert relmax(dg, gr.grad) < 1e-5 and relmax(db, br.grad) < 1e-5 and relmax(dp, want.sum(0)) < 1e-5
 
 
-def test_gradient_quantiser_sites_of_the_kernels():
-    """QPyTorch's backward_number at the QuantStubs (mv_set_grad_format / the dgrad GEMM's q_out), kernel by kernel
+def test_gradient_quantiser_sites_per_call():
+    """QPyTorch's backward_number at the QuantStubs (mv_layernorm_q_bwd's q_grad / the dgrad GEMM's q_out), kernel by kernel
     against fp64 references: the fp32 arithmetic is within 1e-6 of them, so apart from a handful of near-tie flips the
     quantised values must be EQUAL (the model-level test can only bound the flips that fp16 containers add)."""
     import mv_native as mv
@@ -200,15 +200,11 @@ def test_gradient_quantiser_sites_of_the_kernels():
     xr = xq.double().requires_grad_(True)
     F.layer_norm(xr, (D,), g.double(), b.double(), 1e-5).backward(dy.double())
     dp = torch.zeros(D, device=dev)
-    mv.set_grad_format(G)
-    try:
-        dx, dx16 = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10), dbias_prev=dp)
-    finally:
-        mv.set_grad_format(None)
+    dx, dx16 = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10), dbias_prev=dp, q_grad=G)
     want = mv.float_quantize(xr.grad.float(), *G).double() + dres.double()       # the stub rounds BEFORE the residual add
     assert ((dx.double() - want).abs() > 1e-6 * want.abs().max()).float().mean().item() < 1e-3
     assert relmax(dp, want.sum(0)) < 1e-3
-    plain, _ = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10))  # and the option is off again
+    plain, _ = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10))  # and without q_grad, unrounded
     assert relmax(plain, xr.grad + dres.double()) < 1e-6
     # dgrad GEMMs: plain (stub in front of qkv / proj / fc1) and gelu' (stub in front of fc2: rounded BEFORE the multiply)
     M, N, K = 1000, 1536, 384

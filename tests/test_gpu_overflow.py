@@ -196,9 +196,9 @@ def test_gemm_outputs_that_never_raise(place):
 # -------------------------------------------------------------------------------------------- LayerNorm backward
 @pytest.mark.parametrize("kind", ["f16", "f32", "grad_fmt", "drop"])
 @pytest.mark.parametrize("D", [128, 192, 384, 768])
-def test_layernorm_bwd(D, kind):
+def test_layernorm_bwd_sites(D, kind):
     """dy = 0 makes dx = dres exactly; the value sits in the last row of a row count that is not a multiple of the eight
-    rows a CTA takes.  Plain (fp16 / fp32 dy), with the gradient quantiser (set_grad_format), and the dropout variant,
+    rows a CTA takes.  Plain (fp16 / fp32 dy), with the gradient quantiser (q_grad), and the dropout variant,
     whose fp16 copy is the masked gradient: 40000 raises at a kept element (x 2) and not at a dropped one."""
     import mv_native as mv
     torch.manual_seed(D)
@@ -219,13 +219,8 @@ def test_layernorm_bwd(D, kind):
         out = {}
 
         def call():
-            if kind == "grad_fmt":
-                mv.set_grad_format((5, 2))
-            try:
-                out["dx"], out["dx16"] = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10),
-                                                            want_f16=want_f16, drop=drop)
-            finally:
-                mv.set_grad_format(None)
+            out["dx"], out["dx16"] = mv.layernorm_q_bwd(dy, x, g, mean, rstd, dres=dres, q_in=(5, 10), want_f16=want_f16,
+                                                        q_grad=(5, 2) if kind == "grad_fmt" else None, drop=drop)
         return flag_after(call), out["dx"], out["dx16"]
 
     cases = [(col, v / float(mul[-1, col])) for v in VALUES]  # exact thresholds of the stored (masked) value
