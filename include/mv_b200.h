@@ -310,6 +310,44 @@ typedef struct {
 int mv_adamw_step(const mv_adamw_tensor* tensors_dev, int n_tensors, int total_chunks,
                   const float* hyper_dev, void* stream);
 
+/* ---------------------------------------------------------------- low-precision optimizer (qtorch.optim.OptimLP)
+ * mv_adamw_step with QPyTorch's OptimLP quantisers in the same single pass (DESIGN.md section 7).  For every element of
+ * a tensor, unless found_inf is set:
+ *   1. g = q_grad(grad * inv_scale * grad_scaling); grad_out (if not NULL) receives g
+ *   2. the AdamW update of mv_adamw_step runs on acc (if not NULL) or on param itself, with gradient g
+ *   3. exp_avg = q_exp_avg(exp_avg), exp_avg_sq = q_exp_avg_sq(exp_avg_sq)
+ *   4. w = q_acc(updated value); acc (if not NULL) receives w
+ *   5. param = q_weight(w); Linear weights (wq != NULL) emit q(W) / q(W)^T of this final param, as mv_adamw_step.
+ * found_inf non-zero: nothing is written but the operands (grad_out included).
+ * "Optimizer rounding stream": site s (0 grad, 1 exp_avg, 2 exp_avg_sq, 3 acc, 4 weight) of the tensor with `index` k
+ * rounds element i (the tensor's flat row-major index, also for tiled Linear weights) stochastically with the bits that
+ * mv_float_quantize(..., MV_ROUND_STOCHASTIC, seed, offset) (16-bit stream for man >= 7, else 32-bit stream) or
+ * mv_fixed_point_quantize(..., MV_ROUND_STOCHASTIC, seed, offset) (32-bit stream) give element i, with
+ *   offset = (step << 32) | (k << 3) | s,   step = hyper_dev[3] (1-based; a float, so exact below 2^24 steps).
+ * The offset has no rank term: data-parallel ranks holding the same gradients round alike. */
+#define MV_LPQ_NONE 0
+#define MV_LPQ_FLOAT 1      /* FloatingPoint(exp_bits, man_bits): exp 1..8, man 1..22 (as mv_float_quantize) */
+#define MV_LPQ_FIXED 2      /* FixedPoint(wl, fl, clamp, symmetric): wl 1..32, fl -100..100 (as mv_fixed_point_quantize) */
+typedef struct {
+    int kind;                     /* MV_LPQ_* */
+    int rounding;                 /* MV_ROUND_NEAREST or MV_ROUND_STOCHASTIC */
+    int exp_bits, man_bits;
+    int wl, fl, clamp, symmetric;
+} mv_lp_quant;
+typedef struct {
+    mv_lp_quant grad, exp_avg, exp_avg_sq, acc, weight;
+    float grad_scaling;           /* multiplies the un-scaled gradient before q_grad */
+    uint64_t seed;                /* Philox key of the optimizer rounding stream */
+} mv_optim_lp;
+/* per-tensor side table, one entry per mv_adamw_tensor (same order) */
+typedef struct {
+    float* acc;                   /* NULL: param is the accumulator; else fp32 [n], updated in place */
+    float* grad_out;              /* NULL or fp32 [n] (may be grad itself): receives the quantised gradient */
+    uint32_t index;               /* k: the parameter's position in the optimizer's flattened parameter list, < 2^29 */
+} mv_adamw_lp_tensor;
+int mv_adamw_lp_step(const mv_adamw_tensor* tensors_dev, const mv_adamw_lp_tensor* lp_dev, int n_tensors,
+                     int total_chunks, const float* hyper_dev, const mv_optim_lp* spec, void* stream);
+
 /* ---------------------------------------------------------------- segmentation loss (SURVEY.md §8f.4)
  * Fused nn.Upsample(size=(H, W), mode='bilinear', align_corners=False) + CrossEntropyLoss (reduction
  * 'mean', ignore_index) of the reference's segmentation head and train step (models/vit.py:355-371,

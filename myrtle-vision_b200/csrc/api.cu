@@ -122,7 +122,7 @@ int make_tmap_3d(CUtensorMap* map, const void* ptr, int dtype, uint64_t d0, uint
 }  // namespace mv
 
 extern "C" const char* mv_last_error(void) { return mv::g_err; }
-extern "C" int mv_version(void) { return 103; }
+extern "C" int mv_version(void) { return 104; }
 extern "C" int mv_set_overflow_flag(int* flag_dev) { mv::g_overflow = flag_dev; return 0; }
 extern "C" int64_t mv_launch_count(void) { return mv::g_launches; }
 

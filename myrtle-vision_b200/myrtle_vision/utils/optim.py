@@ -63,6 +63,64 @@ def create_optimizer(args, model, filter_bias_and_bn=True, fused=None):
     raise NotImplementedError("optimizer %r (the shipped configs use adamw)" % args.opt)
 
 
+_LP_KEYS = ("weight_quant", "grad_quant", "momentum_quant", "acc_quant", "grad_scaling", "seed")
+
+
+def _lp_quantizer(site, spec):
+    """train_config["optim_lp"][site] -> a qtorch.quant.quantizer (None for null)."""
+    from qtorch import FixedPoint, FloatingPoint
+    from qtorch.quant import quantizer
+    if spec is None:
+        return None
+    if not isinstance(spec, dict):
+        raise ValueError("optim_lp.%s: expected null or an object, got %r" % (site, spec))
+    kinds = [k for k in ("float", "fixed") if k in spec]
+    if len(kinds) != 1:
+        raise ValueError("optim_lp.%s: give exactly one of \"float\": [exp, man] or \"fixed\": [wl, fl]" % site)
+    allowed = {"float": {"float", "rounding"}, "fixed": {"fixed", "rounding", "clamp", "symmetric"}}[kinds[0]]
+    unknown = set(spec) - allowed
+    if unknown:
+        raise ValueError("optim_lp.%s: unknown keys %s" % (site, sorted(unknown)))
+    rounding = spec.get("rounding", "stochastic")
+    if rounding not in ("stochastic", "nearest"):
+        raise ValueError("optim_lp.%s: rounding must be \"stochastic\" or \"nearest\", got %r" % (site, rounding))
+    bits = spec[kinds[0]]
+    if not (isinstance(bits, (list, tuple)) and len(bits) == 2 and all(isinstance(b, int) for b in bits)):
+        raise ValueError("optim_lp.%s: %s needs two integers, got %r" % (site, kinds[0], bits))
+    if kinds[0] == "float":
+        if not (1 <= bits[0] <= 8 and 1 <= bits[1] <= 22):
+            raise ValueError("optim_lp.%s: float [exp, man] needs exp in 1..8 and man in 1..22, got %r" % (site, bits))
+        number = FloatingPoint(exp=bits[0], man=bits[1])
+    else:
+        if not (1 <= bits[0] <= 32 and 1 <= bits[1] <= 100):
+            raise ValueError("optim_lp.%s: fixed [wl, fl] needs wl in 1..32 and fl in 1..100, got %r" % (site, bits))
+        number = FixedPoint(wl=bits[0], fl=bits[1], clamp=bool(spec.get("clamp", True)),
+                            symmetric=bool(spec.get("symmetric", False)))
+    return quantizer(forward_number=number, forward_rounding=rounding)
+
+
+def wrap_optim_lp(optimizer, cfg):
+    """train_config["optim_lp"] -> qtorch.optim.OptimLP around `optimizer` (DESIGN.md section 7):
+    {"weight_quant": Q, "grad_quant": Q, "momentum_quant": Q, "acc_quant": Q, "grad_scaling": 1.0, "seed": null},
+    Q = null | {"float": [exp, man], "rounding": ...} | {"fixed": [wl, fl], "clamp": true, "symmetric": false,
+    "rounding": ...}, rounding "stochastic" (the default, as QPyTorch's) or "nearest".  Absent keys are null / 1.0."""
+    from qtorch.optim import OptimLP
+    if not isinstance(cfg, dict):
+        raise ValueError("optim_lp: expected an object, got %r" % (cfg,))
+    unknown = set(cfg) - set(_LP_KEYS)
+    if unknown:
+        raise ValueError("optim_lp: unknown keys %s (known: %s)" % (sorted(unknown), ", ".join(_LP_KEYS)))
+    scaling = cfg.get("grad_scaling", 1.0)
+    if not isinstance(scaling, (int, float)) or isinstance(scaling, bool) or not scaling > 0:
+        raise ValueError("optim_lp.grad_scaling: expected a positive number, got %r" % (scaling,))
+    seed = cfg.get("seed")
+    if seed is not None and (not isinstance(seed, int) or isinstance(seed, bool) or not 0 <= seed < 2 ** 64):
+        raise ValueError("optim_lp.seed: expected null or an integer in [0, 2^64), got %r" % (seed,))
+    q = {k: _lp_quantizer(k, cfg.get(k)) for k in _LP_KEYS[:4]}
+    return OptimLP(optimizer, weight_quant=q["weight_quant"], grad_scaling=float(scaling), grad_quant=q["grad_quant"],
+                   momentum_quant=q["momentum_quant"], acc_quant=q["acc_quant"], seed=seed)
+
+
 class CosineSchedule:
     """Epoch-indexed cosine decay with linear warm-up; `step(epoch)` sets the lr of every group."""
 

@@ -23,12 +23,14 @@ import torch.nn.functional as F
 from torch.utils.data import DataLoader
 from torch.utils.data.distributed import DistributedSampler
 
+from qtorch.optim import OptimLP
+
 from myrtle_vision.datasets.synthetic import SyntheticVision, detection_collate
 from myrtle_vision.models.matcher import pad_targets
 from myrtle_vision.utils.graph import GraphedTrainStep
 from myrtle_vision.utils.models import (get_models, get_optimizer_args, prepare_model_and_load_ckpt,
                                         save_checkpoint)
-from myrtle_vision.utils.optim import create_optimizer, create_scheduler
+from myrtle_vision.utils.optim import create_optimizer, create_scheduler, wrap_optim_lp
 from myrtle_vision.utils.parallel import DataParallel
 from myrtle_vision.utils.utils import (cleanup_distributed, get_batch_sizes, init_distributed,
                                        parse_config, seed_everything)
@@ -146,6 +148,9 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     net = DataParallel(vit) if num_gpus > 1 else vit
     optimizer_args = get_optimizer_args(train_config)
     optimizer = create_optimizer(optimizer_args, vit)
+    if train_config.get("optim_lp") is not None:
+        # qtorch.optim.OptimLP: low-precision weights, gradients, moments and accumulator (DESIGN.md section 7)
+        optimizer = wrap_optim_lp(optimizer, train_config["optim_lp"])
     lr_scheduler, _ = create_scheduler(optimizer_args, optimizer)
     criterion = build_criterion(task, train_config, data_config["number_of_classes"], device)
     iteration = prepare_model_and_load_ckpt(train_config=train_config, model=vit, optimizer=optimizer,
@@ -206,8 +211,8 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
             n_accum += 1
             if n_accum == n_batch_accum:
                 n_accum = 0
-                if hasattr(optimizer, "_operands"):
-                    # FusedAdamW: the backward's device-side overflow flag skips the update exactly like
+                if hasattr(optimizer, "_operands") or isinstance(optimizer, OptimLP):
+                    # FusedAdamW (or OptimLP): the backward's device-side overflow flag skips the update exactly like
                     # GradScaler.step() in the reference (classification/train.py:274-277), without a host sync
                     optimizer.step(found_inf=vit.engine().found_inf)
                     vit.engine().found_inf.zero_()

@@ -104,7 +104,12 @@ def quantizer(forward_number=None, backward_number=None, forward_rounding="stoch
                 grad = hook(grad)
             return grad
 
-    return _Rounding.apply
+    def quantize(x):
+        return _Rounding.apply(x)
+
+    # what qtorch.optim.OptimLP reads to run a recognised format in its fused optimizer kernel
+    quantize.forward_number, quantize.forward_rounding = forward_number, forward_rounding
+    return quantize
 
 
 class Quantizer(torch.nn.Module):
@@ -113,6 +118,7 @@ class Quantizer(torch.nn.Module):
         super().__init__()
         self.quantize = quantizer(forward_number, backward_number, forward_rounding,
                                   backward_rounding)
+        self.forward_number, self.forward_rounding = forward_number, forward_rounding
 
     def forward(self, x):
         return self.quantize(x)
