@@ -201,13 +201,16 @@ int mv_layernorm_q_bwd(const mv_layernorm_bwd_args* args, void* stream);
 /* out[c] += sum_r in[r,c]   (bias gradients); in_dtype MV_F16 or MV_F32 */
 int mv_colsum(const void* in, int in_dtype, int64_t ld, int rows, int cols, float* out, void* stream);
 /* img NCHW fp32 -> q(patches) [B*(H/P)*(W/P), P*P*C], (ph,pw,c) minor order (models/vit.py:271-275).
- * cls_slot != 0: each image gets one extra leading all-zero row (the class-token slot), so patch rows
- * line up 1:1 with token rows [B*N, .] for the embedding GEMM and its wgrad. */
+ * cls_slot = 1: each image gets one extra leading all-zero row (the class-token slot), so patch rows
+ * line up 1:1 with token rows [B*N, .] for the embedding GEMM and its wgrad.  cls_slot = 2: a leading and a
+ * trailing all-zero row per image (the class-token and distillation-token slots).  Any other value is an error. */
 int mv_patchify_q(const float* img, void* out, int out_dtype, int B, int C, int H, int W, int P,
                   int q_exp, int q_man, int cls_slot, void* stream);
 /* x[b,0,:] = q(q(cls) + pos_q[0,:]) for every image b (models/vit.py:283-310) */
 int mv_cls_rows(const float* cls, const float* pos_q, float* x, int B, int n_tokens, int D, int q_exp,
                 int q_man, void* stream);
+/* x[b,row,:] = q(tok[:]) for every image b: the distillation token, which gets no positional embedding */
+int mv_token_row(const float* tok, float* x, int B, int n_tokens, int D, int row, int q_exp, int q_man, void* stream);
 /* fp32 -> fp16 (saturating) / bf16 copy of n elements (n % 4 == 0) */
 int mv_convert_f32(const float* in, void* out, int out_dtype, int64_t n, void* stream);
 /* out_f32[i] = in[i] * s and / or out_f16[i] = fp16_sat(in[i] * s) for n elements (n % 4 == 0; either output may
@@ -357,6 +360,21 @@ int mv_adamw_lp_step(const mv_adamw_tensor* tensors_dev, const mv_adamw_lp_tenso
  * dy += d(sum of pixel losses)/dy.  The caller zeroes dy / acc and divides by acc[1]. */
 int mv_upsample_ce(const float* y, const int64_t* labels, float* dy, float* acc, int B, int C, int gh, int gw,
                    int H, int W, int64_t ignore_index, void* stream);
+
+/* ---------------------------------------------------------------- distillation loss (DESIGN.md section 7)
+ * The loss of DistillWrapper (models/distill.py), forward and backward in one pass over fp32 [B, C] student logits s,
+ * distillation-head logits d and teacher logits t (row pitch C), int64 labels y [B]:
+ *   row b:  ce = lse(s) - s[y],
+ *           soft (hard == 0): D = T^2 * sum_c p_c (log p_c - log q_c),  p = softmax(t / T), q = softmax(d / T)
+ *           hard (hard != 0): D = lse(d) - d[argmax t]  (the first maximal index, as torch.argmax)
+ *   loss = (1 - alpha) * mean_b ce + alpha * mean_b D      (F.kl_div's "batchmean", F.cross_entropy's "mean")
+ * d_student / d_distill (fp32 [B, C]) receive d loss / d s and d loss / d d; row_loss (fp32 [B]) is scratch that
+ * receives each row's (1 - alpha) ce + alpha D.  The batch sum is a fixed-order reduction (no float atomics): the
+ * result is deterministic.  A label outside [0, C) makes its row's loss and gradients NaN (no host sync to raise from;
+ * the overflow sink of the backward then skips the step).  C >= 2, T > 0, 0 <= alpha <= 1.  Two launches. */
+int mv_distill_loss(const float* student, const float* distill, const float* teacher, const int64_t* labels, int B,
+                    int C, float T, float alpha, int hard, float* loss, float* row_loss, float* d_student,
+                    float* d_distill, void* stream);
 
 /* ---------------------------------------------------------------- detection matching (SURVEY.md §8f.4)
  * scipy.optimize.linear_sum_assignment of the reference's HungarianMatcher (models/matcher.py:83-86) for a

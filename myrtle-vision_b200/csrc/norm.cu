@@ -409,10 +409,14 @@ patchify_kernel(const float* __restrict__ img, OutT* __restrict__ out, int B, in
     const int pdim = P * P * C;
     const int PC = P * C;
     const int64_t rows_per_img = int64_t(gh) * gw + cls_slot;
-    OutT* obase = out + (int64_t(b) * rows_per_img + cls_slot + int64_t(gy) * gw) * pdim;
+    OutT* obase = out + (int64_t(b) * rows_per_img + (cls_slot != 0) + int64_t(gy) * gw) * pdim;
     if (cls_slot && gy == 0) {          // row b*N + 0 is the (zero) slot of the class token
         OutT* z = out + int64_t(b) * rows_per_img * pdim;
         for (int i = threadIdx.x; i < pdim; i += blockDim.x) z[i] = OutT(0.f);
+        if (cls_slot == 2) {            // ... and row b*N + N-1 the (zero) slot of the distillation token
+            z += (rows_per_img - 1) * pdim;
+            for (int i = threadIdx.x; i < pdim; i += blockDim.x) z[i] = OutT(0.f);
+        }
     }
     const int mode = fq_mode(q_in);
     const int w4 = W >> 2;              // W % 4 == 0 checked on the host
@@ -455,6 +459,15 @@ __global__ void cls_row_kernel(const float* __restrict__ cls, const float* __res
     const int b = i / D, d = i % D;
     const float v = fq_nearest(fq_nearest(cls[d], q_ff) + pos_q[d], q_ff);
     x[(int64_t(b) * n_tokens) * D + d] = v;
+}
+
+// token row: x[b, row, :] = q_ff(tok) for every image (the distillation token: no positional embedding)
+__global__ void token_row_kernel(const float* __restrict__ tok, float* __restrict__ x, int B, int n_tokens, int D,
+                                 int row, FloatFmt q_ff) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= B * D) return;
+    const int b = i / D, d = i % D;
+    x[(int64_t(b) * n_tokens + row) * D + d] = fq_nearest(tok[d], q_ff);
 }
 
 // fp32 -> bf16 / fp16 conversion (gradient operand copies)
@@ -781,6 +794,7 @@ extern "C" int mv_colsum(const void* in, int in_dtype, int64_t ld, int rows, int
 extern "C" int mv_patchify_q(const float* img, void* out, int out_dtype, int B, int C, int H, int W, int P,
                              int q_exp, int q_man, int cls_slot, void* stream) {
     MV_CHECK(B > 0 && C > 0 && P > 0 && H % P == 0 && W % P == 0, "mv_patchify_q: image dims must be divisible by the patch size");
+    MV_CHECK(cls_slot >= 0 && cls_slot <= 2, "mv_patchify_q: cls_slot must be 0, 1 or 2");
     const FloatFmt q{q_exp, q_man};
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MV_CHECK(W % 4 == 0 && (reinterpret_cast<uintptr_t>(img) & 15) == 0, "mv_patchify_q: image rows must be 16-byte aligned (W % 4 == 0)");
@@ -789,10 +803,10 @@ extern "C" int mv_patchify_q(const float* img, void* out, int out_dtype, int B, 
     MV_CHECK(smem <= 200 * 1024, "mv_patchify_q: C * P * W too large for the shared-memory staging buffer");
     if (out_dtype == MV_F16) {
         MV_CUDA(cudaFuncSetAttribute(patchify_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        patchify_kernel<__half><<<grid, 256, smem, st>>>(img, (__half*)out, B, C, H, W, P, q, cls_slot ? 1 : 0);
+        patchify_kernel<__half><<<grid, 256, smem, st>>>(img, (__half*)out, B, C, H, W, P, q, cls_slot);
     } else if (out_dtype == MV_F32) {
         MV_CUDA(cudaFuncSetAttribute(patchify_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        patchify_kernel<float><<<grid, 256, smem, st>>>(img, (float*)out, B, C, H, W, P, q, cls_slot ? 1 : 0);
+        patchify_kernel<float><<<grid, 256, smem, st>>>(img, (float*)out, B, C, H, W, P, q, cls_slot);
     } else MV_CHECK(false, "mv_patchify_q: bad container");
     g_launches++;
     return check_cuda(cudaGetLastError(), "patchify launch");
@@ -805,6 +819,16 @@ extern "C" int mv_cls_rows(const float* cls, const float* pos_q, float* x, int B
     cls_row_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(cls, pos_q, x, B, n_tokens, D, q);
     g_launches++;
     return check_cuda(cudaGetLastError(), "cls rows launch");
+}
+
+extern "C" int mv_token_row(const float* tok, float* x, int B, int n_tokens, int D, int row, int q_exp, int q_man,
+                            void* stream) {
+    MV_CHECK(tok && x && B > 0 && D > 0 && row >= 0 && row < n_tokens, "mv_token_row: bad arguments");
+    const FloatFmt q{q_exp, q_man};
+    const int n = B * D;
+    token_row_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(tok, x, B, n_tokens, D, row, q);
+    g_launches++;
+    return check_cuda(cudaGetLastError(), "token row launch");
 }
 
 extern "C" int mv_convert_f32(const float* in, void* out, int out_dtype, int64_t n, void* stream) {

@@ -159,6 +159,10 @@ class EncoderEngine:
         # True once an optimizer (utils/fused_adamw.FusedAdamW) emits q(W) / q(W)^T itself after every
         # update: a CUDA-graph capture then leaves the re-quantisation out of the graph
         self.external_requant = False
+        # True for a model whose weights do not change while it is used (a distillation teacher, models/distill.py):
+        # the operands are quantised once and served from the cache inside a CUDA-graph capture, so a replay does not
+        # re-quantise them; outside a capture they are still rebuilt when the parameters change (e.g. load_state_dict)
+        self.frozen_weights = False
         # nn.Module.training of the owning model (ViT.forward sets it): dropout acts in training forwards only
         self.training = True
         # seed of the last forward that applied dropout: int64 [1] on the device (its 64 bits are the Philox key)
@@ -194,6 +198,8 @@ class EncoderEngine:
             return self._wq
         if capturing and self._wq is not None and self._wq_capture_done == self._capture_key():
             return self._wq          # already re-quantised once inside this capture (forward)
+        if capturing and self._wq is not None and self.frozen_weights:
+            return self._wq
         if self.exact:
             wq = {i: (mv.split_tf32(self.params[i].detach(), 1),
                       mv.split_tf32(self.params[i].detach().t().contiguous(), 1)) for i in idx}
@@ -316,7 +322,9 @@ class EncoderEngine:
         self.last_grad_round_seed = seed
         return seed
 
-    def forward(self, img, pos_full, cls_token, save):
+    def forward(self, img, pos_full, cls_token, save, token=None):
+        """token (optional, [1, 1, D]): a distillation token appended as the last row N - 1 of every image, with no
+        positional embedding (DESIGN.md section 7); pos_full then still holds the N - 1 rows of cls + grid."""
         # A training forward clears self.overflow and its backward closes the window (mv_overflow_update); inference
         # forwards report nothing.  The library keeps one process-wide flag pointer, so it is registered only while
         # this engine's own kernels run and cleared on the way out, exception or not: launches outside the step (other
@@ -329,19 +337,31 @@ class EncoderEngine:
             drops = self._draw_drops()
             self.step_grad_round_seed = self._draw_grad_round(save)
             if self.wide:
-                return self._forward_wide(img, pos_full, cls_token, save, drops)
-            x, saved = self._forward_16(img, pos_full, cls_token, save, drops)
+                return self._forward_wide(img, pos_full, cls_token, save, drops, token)
+            x, saved = self._forward_16(img, pos_full, cls_token, save, drops, token)
             if saved is not None:
                 saved["grad_round"] = self.step_grad_round_seed
             return x, saved
         finally:
             mv.set_overflow_flag(None)
 
-    def _forward_16(self, img, pos_full, cls_token, save, drops):
+    def _embed_inputs(self, pos_full, token, N, D):
+        """The patch-embedding GEMM's positional residual [N, D] and the patchify slot mode: with a token its last row
+        is zero (mv_token_row overwrites that row of x afterwards) and `patches` gets a zero row at both ends."""
+        pos32 = pos_full.detach().reshape(N - (token is not None), D)
+        if token is None:
+            return pos32.contiguous(), 1
+        return torch.cat((pos32, pos32.new_zeros(1, D))), 2
+
+    def _token_row(self, token, x, B, N, D):
+        if token is not None:
+            mv.token_row(token.detach().reshape(D).contiguous(), x, B, N, D, N - 1, q_ff=self.cfg.plan.ff)
+
+    def _forward_16(self, img, pos_full, cls_token, save, drops, token=None):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
-        N = (Hh // P) * (Ww // P) + 1
+        N = (Hh // P) * (Ww // P) + 1 + (token is not None)
         M, D, Mm, H = B * N, cfg.dim, cfg.mlp_dim, cfg.heads
         prm = [p.detach() for p in self.params]
         wq = self.quantised_weights()
@@ -349,16 +369,18 @@ class EncoderEngine:
         dev = img.device
 
         with self._range("patch_to_embedding"):
-            patches = mv.patchify_q(img, P, q_in=fmt, cls_slot=True)            # [M, P*P*C], zero cls rows
+            pos32, slots = self._embed_inputs(pos_full, token, N, D)
+            patches = mv.patchify_q(img, P, q_in=fmt, cls_slot=slots)           # [M, P*P*C], zero token rows
             x = torch.empty(M, D, dtype=torch.float32, device=dev)
-            pos32 = pos_full.detach().reshape(N, D).contiguous()
             mv.gemm(patches, wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                     rows_per_img=N)
             mv.cls_rows(cls_token.detach().reshape(D).contiguous(), pos32, x, B, N, D, q_ff=plan.ff)
+            self._token_row(token, x, B, N, D)
             if drops and drops.emb():
                 mv.dropout(x, drops.emb(), out=x)
 
-        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops} if save else None
+        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops,
+                 "token": token is not None} if save else None
         with self._range("transformer"):
             for l in range(cfg.depth):
                 b0 = 2 + PER_LAYER * l
@@ -496,14 +518,14 @@ class EncoderEngine:
         # ---- patch embedding: dW = dx^T patches (cls rows of `patches` are zero)
         mv.gemm(dx_h, saved["patches"], g[0], a_major=1, b_major=1, accumulate=True)
         wq_grad(0, 10 * cfg.depth)
-        return self._finish_backward(dx, S, B, N, D)
+        return self._finish_backward(dx, S, B, N, D, saved["token"])
 
-    def _finish_backward(self, dx, S, B, N, D):
+    def _finish_backward(self, dx, S, B, N, D, token=False):
         g, dev = self.gviews, dx.device
         dpos = torch.zeros(N * D, dtype=torch.float32, device=dev)
         mv.colsum(dx.view(B, N * D), dpos)
         dpos = dpos.view(1, N, D)
-        g[1].copy_(dpos[0, 1:].sum(0))                                     # bias: patch rows only
+        g[1].copy_(dpos[0, 1:N - token].sum(0))                            # bias: patch rows only
         inv = 1.0 / S
         slot = None
         if self.reducer is not None:
@@ -515,6 +537,11 @@ class EncoderEngine:
             slot = self.gflat[0:1]
         dpos = dpos * inv
         dcls = dpos[:, 0:1, :].clone()
+        dtok = None
+        if token:
+            # the token row has no positional embedding: its column sum is the token's gradient
+            dtok = dpos[:, N - 1:N, :].clone()
+            dpos = dpos[:, :N - 1, :]
         # hand autograd its own copy: self.gflat is reused (zeroed) by the next backward.  The same pass un-scales
         # (single GPU) and tests every parameter gradient for inf / NaN (the overflow sink)
         if self.reducer is not None:
@@ -524,7 +551,7 @@ class EncoderEngine:
         mv.overflow_update(self.overflow, self.scaler_state, shared_slot=slot)
         grads = [out[self.offsets[i]:self.offsets[i] + p.numel()].view_as(p)
                  for i, p in enumerate(self.params)]
-        return dpos, dcls, grads
+        return dpos, dcls, dtok, grads
 
     def _one(self):
         if getattr(self, "_one_t", None) is None:
@@ -537,11 +564,11 @@ class EncoderEngine:
     # wgrad therefore takes explicit transposes (mv_widen_transpose) instead of the in-place MN-major
     # reads of the 16-bit path.  Attention keeps the fp16 tcgen05 kernels: qkv / attention output /
     # their gradients carry 11 significant bits, the same as a tf32 operand.
-    def _forward_wide(self, img, pos_full, cls_token, save, drops):
+    def _forward_wide(self, img, pos_full, cls_token, save, drops, token=None):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
-        N = (Hh // P) * (Ww // P) + 1
+        N = (Hh // P) * (Ww // P) + 1 + (token is not None)
         M, D, Mm, H = B * N, cfg.dim, cfg.mlp_dim, cfg.heads
         prm = [p.detach() for p in self.params]
         wq = self.quantised_weights()
@@ -550,12 +577,13 @@ class EncoderEngine:
         ex = self.exact
         A_ = (lambda t: mv.split_tf32(t, 0)) if ex else (lambda t: t)        # A operand of a Linear
 
-        patches = mv.patchify_q(img, P, q_in=fmt, out_dtype=f32, cls_slot=True)
+        pos32, slots = self._embed_inputs(pos_full, token, N, D)
+        patches = mv.patchify_q(img, P, q_in=fmt, out_dtype=f32, cls_slot=slots)
         x = torch.empty(M, D, dtype=f32, device=dev)
-        pos32 = pos_full.detach().reshape(N, D).contiguous()
         mv.gemm(A_(patches), wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                 rows_per_img=N)
         mv.cls_rows(cls_token.detach().reshape(D).contiguous(), pos32, x, B, N, D, q_ff=plan.ff)
+        self._token_row(token, x, B, N, D)
         if drops and drops.emb():
             mv.dropout(x, drops.emb(), out=x)
 
@@ -571,7 +599,8 @@ class EncoderEngine:
                 mv.float_quantize(y, plan.ff[0], plan.ff[1], out=y)
             return y
 
-        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops} if save else None
+        saved = {"B": B, "N": N, "patches": patches, "layers": [], "drops": drops,
+                 "token": token is not None} if save else None
         for l in range(cfg.depth):
             b0 = 2 + PER_LAYER * l
             xn1, mean1, rstd1 = mv.layernorm_q_fwd(x, prm[b0], prm[b0 + 1], q_in=fmt, q_post=fmt,
@@ -724,23 +753,24 @@ class EncoderEngine:
         if drops and drops.emb():
             mv.dropout(dx, drops.emb(), out=dx)
         wgrad(dx, saved["patches"], g[0])
-        return self._finish_backward(dx, S, B, N, D)
+        return self._finish_backward(dx, S, B, N, D, saved["token"])
 
 
 class EncoderFunction(torch.autograd.Function):
     @classmethod
-    def apply(cls, engine, img, pos_full, cls_token, *params):
+    def apply(cls, engine, img, pos_full, cls_token, *params, token=None):
+        """token: optional distillation token [1, 1, D] (EncoderEngine.forward)."""
         # ctx.needs_input_grad follows requires_grad even under torch.no_grad(), and forward() itself always runs with
         # grad mode off, so grad mode is read here: without it the forward saves nothing and reports into no flag
         if not torch.is_grad_enabled():
-            return engine.forward(img, pos_full, cls_token, save=False)[0]
-        return super().apply(engine, img, pos_full, cls_token, *params)
+            return engine.forward(img, pos_full, cls_token, save=False, token=token)[0]
+        return super().apply(engine, img, pos_full, cls_token, token, *params)
 
     @staticmethod
-    def forward(ctx, engine, img, pos_full, cls_token, *params):
+    def forward(ctx, engine, img, pos_full, cls_token, token, *params):
         need = any(ctx.needs_input_grad)      # False when no input requires a gradient
         with torch.no_grad():
-            x, saved = engine.forward(img, pos_full, cls_token, save=need)
+            x, saved = engine.forward(img, pos_full, cls_token, save=need, token=token)
         ctx.engine, ctx.saved = engine, saved
         return x
 
@@ -752,6 +782,6 @@ class EncoderFunction(torch.autograd.Function):
         if engine.reducer is not None:
             engine.reducer.queue_finalize()
         with torch.no_grad():
-            dpos, dcls, g = engine.backward(saved, gx.contiguous())
+            dpos, dcls, dtok, g = engine.backward(saved, gx.contiguous())
         ctx.saved = None
-        return (None, None, dpos, dcls) + tuple(g)
+        return (None, None, dpos, dcls, dtok) + tuple(g)

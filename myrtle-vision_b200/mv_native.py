@@ -67,6 +67,15 @@ class LayerNormBwdArgs(ctypes.Structure):
     ]
 
 
+# ctypes signatures of entry points declared with full argument types (tests/test_distill_host.py holds them to the
+# header's prototypes)
+_P, _I, _F = ctypes.c_void_p, ctypes.c_int, ctypes.c_float
+SIGNATURES = {
+    "mv_token_row": [_P, _P, _I, _I, _I, _I, _I, _I, _P],
+    "mv_distill_loss": [_P, _P, _P, _P, _I, _I, _F, _F, _I, _P, _P, _P, _P, _P],
+}
+
+
 def so_path():
     return _SO
 
@@ -82,6 +91,9 @@ def lib():
         _lib = ctypes.CDLL(_SO)
         _lib.mv_last_error.restype = ctypes.c_char_p
         _lib.mv_launch_count.restype = ctypes.c_int64
+        for name, args in SIGNATURES.items():
+            fn = getattr(_lib, name)
+            fn.argtypes, fn.restype = args, ctypes.c_int
     return _lib
 
 
@@ -463,15 +475,18 @@ def colsum(x2d, out):
 
 
 def patchify_q(img, patch, q_in=None, out_dtype=torch.float16, cls_slot=False):
+    """cls_slot: False / 0 (patch rows only), True / 1 (a zero class-token row first per image) or 2 (a zero row first
+    and a zero row last per image: the class- and distillation-token slots)."""
     _need_cuda(img)
     img = img.contiguous().float()
     B, C, H, W = img.shape
-    rows = B * ((H // patch) * (W // patch) + (1 if cls_slot else 0))
+    cls_slot = int(cls_slot)
+    rows = B * ((H // patch) * (W // patch) + cls_slot)
     out = torch.empty(rows, patch * patch * C, dtype=out_dtype, device=img.device)
     q = _fmt(q_in)
     with _timed("patchify", 0.0, img.numel() * 4 + out.numel() * out.element_size()):
         _check(lib().mv_patchify_q(_ptr(img), _ptr(out), _DT[out_dtype], B, C, H, W, patch, q[0], q[1],
-                                   int(bool(cls_slot)), _stream()), "mv_patchify_q")
+                                   cls_slot, _stream()), "mv_patchify_q")
     return out
 
 
@@ -479,6 +494,34 @@ def cls_rows(cls, pos_q, x, B, n_tokens, D, q_ff=None):
     q = _fmt(q_ff)
     _check(lib().mv_cls_rows(_ptr(cls), _ptr(pos_q), _ptr(x), B, n_tokens, D, q[0], q[1], _stream()),
            "mv_cls_rows")
+
+
+def token_row(tok, x, B, n_tokens, D, row, q_ff=None):
+    """mv_token_row: x[b, row, :] = q_ff(tok) for every image of the token-major fp32 x [B * n_tokens, D]."""
+    _need_cuda(tok, x)
+    assert tok.dtype == torch.float32 and tok.is_contiguous() and tok.numel() == D
+    assert x.dtype == torch.float32 and x.is_contiguous() and x.numel() == B * n_tokens * D
+    q = _fmt(q_ff)
+    _check(lib().mv_token_row(_ptr(tok), _ptr(x), B, n_tokens, D, int(row), q[0], q[1], _stream()), "mv_token_row")
+
+
+def distill_loss(student, distill, teacher, labels, temperature, alpha, hard):
+    """mv_distill_loss: -> (loss fp32 [1], d loss / d student, d loss / d distill), all on the device.  student,
+    distill, teacher: fp32 [B, C]; labels: int64 [B]."""
+    _need_cuda(student, distill, teacher, labels)
+    student, distill, teacher = (t.detach().float().contiguous() for t in (student, distill, teacher))
+    labels = labels.contiguous()
+    assert student.dim() == 2 and student.shape == distill.shape == teacher.shape, "logits must all be [B, C]"
+    assert labels.dtype == torch.int64 and labels.shape == student.shape[:1], "labels must be int64 [B]"
+    B, C = student.shape
+    loss = torch.empty(1, dtype=torch.float32, device=student.device)
+    rows = torch.empty(B, dtype=torch.float32, device=student.device)
+    ds, dd = torch.empty_like(student), torch.empty_like(distill)
+    with _timed("distill_loss", 0.0, B * C * 4 * 5):
+        _check(lib().mv_distill_loss(_ptr(student), _ptr(distill), _ptr(teacher), _ptr(labels), B, C,
+                                     ctypes.c_float(temperature), ctypes.c_float(alpha), int(bool(hard)), _ptr(loss),
+                                     _ptr(rows), _ptr(ds), _ptr(dd), _stream()), "mv_distill_loss")
+    return loss, ds, dd
 
 
 def convert_f32(x, out_dtype=torch.float16, out=None):

@@ -1,8 +1,8 @@
 """Model factory and checkpoint helpers (reference: src/myrtle_vision/utils/models.py:25-141).
 
 `get_models(config)` keeps the JSON schema (`vit_config`, `data_config_path`) and returns
-`(vit, None)`; the distillation wrapper of the reference is broken upstream and out of scope
-(SURVEY.md §2 row 11), so a `distiller_config` raises."""
+`(vit, None)`, or `(vit, DistillWrapper)` when the config has a `distiller_config` (models/distill.py; the
+reference's wrapper is broken upstream, SURVEY.md §2 row 11, and is restated there)."""
 import torch
 
 from myrtle_vision.models.vit import ViT
@@ -15,8 +15,10 @@ def get_models(config, profile=False):
     data_config = config.get("data_config")
     if data_config is None:
         data_config = parse_config(config["data_config_path"])
+    distiller = None
     if "distiller_config" in config:
-        raise NotImplementedError("distillation is outside the B200 hot path")
+        from myrtle_vision.models.distill import parse_distiller_config
+        distiller = parse_distiller_config(config["distiller_config"], vit_config["decoder"])
     vit = ViT(
         decoder=vit_config["decoder"],
         image_size=vit_config["image_size"],
@@ -31,21 +33,34 @@ def get_models(config, profile=False):
         profile=profile,
         q_format=QFormat[vit_config["q_format"]],
     )
-    return vit, None
+    if distiller is None:
+        return vit, None
+    from myrtle_vision.models.distill import DistillWrapper, build_teacher
+    teacher = build_teacher(distiller["teacher"], data_config["number_of_classes"])
+    return vit, DistillWrapper(student=vit, teacher=teacher, temperature=distiller["temperature"],
+                               alpha=distiller["alpha"], hard=distiller["hard"])
 
 
-def save_checkpoint(model, optimizer, lr_scheduler, iteration, filepath):
-    torch.save({
+def save_checkpoint(model, optimizer, lr_scheduler, iteration, filepath, distiller=None):
+    """distiller (a DistillWrapper): its own parameters go under "distiller"; "model" stays the student's."""
+    state = {
         "model": model.state_dict(),
         "optimizer": optimizer.state_dict(),
         "lr_scheduler": lr_scheduler.state_dict() if lr_scheduler is not None else None,
         "iteration": iteration,
-    }, filepath)
+    }
+    if distiller is not None:
+        state["distiller"] = distiller.distiller_state_dict()
+    torch.save(state, filepath)
 
 
-def load_checkpoint(model, optimizer, lr_scheduler, filepath):
+def load_checkpoint(model, optimizer, lr_scheduler, filepath, distiller=None):
     checkpoint = torch.load(filepath, map_location="cpu")
     model.load_state_dict(checkpoint["model"])
+    if distiller is not None:
+        if "distiller" not in checkpoint:
+            raise KeyError("%s has no \"distiller\" entry to resume the distillation head from" % filepath)
+        distiller.load_distiller_state_dict(checkpoint["distiller"])
     if optimizer is not None:
         optimizer.load_state_dict(checkpoint["optimizer"])
     if lr_scheduler is not None and checkpoint.get("lr_scheduler") is not None:
@@ -53,10 +68,10 @@ def load_checkpoint(model, optimizer, lr_scheduler, filepath):
     return checkpoint["iteration"]
 
 
-def prepare_model_and_load_ckpt(train_config, model, optimizer=None, lr_scheduler=None):
+def prepare_model_and_load_ckpt(train_config, model, optimizer=None, lr_scheduler=None, distiller=None):
     if train_config["checkpoint_path"] != "":
         return load_checkpoint(model=model, optimizer=optimizer, lr_scheduler=lr_scheduler,
-                               filepath=train_config["checkpoint_path"])
+                               filepath=train_config["checkpoint_path"], distiller=distiller)
     return 0
 
 

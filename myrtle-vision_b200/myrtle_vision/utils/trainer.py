@@ -141,20 +141,29 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     val_loader = DataLoader(valset, num_workers=0, batch_size=batch_size, collate_fn=collate,
                             drop_last=train_config["drop_last_batch"]) if len(valset) else []
 
-    vit, _ = get_models(config)
+    vit, distiller = get_models(config)
     vit = vit.to(device)
     if task == "segmentation" and train_config.get("fused_seg_loss", True):
         vit.decoder.fused_loss = True        # training forward returns patch logits for the fused loss
-    net = DataParallel(vit) if num_gpus > 1 else vit
+    # distillation (config["distiller_config"], models/distill.py): the step trains the wrapper (student, token and
+    # head; the frozen teacher runs inside it), evaluation and checkpoints' "model" stay the student's
+    model = vit
+    if distiller is not None:
+        model = distiller.to(device)
+    net = DataParallel(model) if num_gpus > 1 else model
     optimizer_args = get_optimizer_args(train_config)
-    optimizer = create_optimizer(optimizer_args, vit)
+    optimizer = create_optimizer(optimizer_args, model)
     if train_config.get("optim_lp") is not None:
         # qtorch.optim.OptimLP: low-precision weights, gradients, moments and accumulator (DESIGN.md section 7)
         optimizer = wrap_optim_lp(optimizer, train_config["optim_lp"])
     lr_scheduler, _ = create_scheduler(optimizer_args, optimizer)
     criterion = build_criterion(task, train_config, data_config["number_of_classes"], device)
+    train_criterion = criterion
+    if distiller is not None:
+        from myrtle_vision.models.distill import DistillLoss
+        train_criterion = DistillLoss(distiller.temperature, distiller.alpha, distiller.hard)
     iteration = prepare_model_and_load_ckpt(train_config=train_config, model=vit, optimizer=optimizer,
-                                            lr_scheduler=lr_scheduler)
+                                            lr_scheduler=lr_scheduler, distiller=distiller)
     # detection: targets padded to a fixed [B, capacity] block and matched on the device (csrc/assign.cu),
     # so the criterion has no host synchronisation and the whole step is one CUDA graph like the other tasks;
     # "device_matching": false restores the host (SciPy) matcher between two captured graphs
@@ -170,7 +179,7 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     iters_per_val = train_config.get("iters_per_val", 0)
     log_every = train_config.get("log_every", 1)
     epoch_offset = max(0, int(batch_size * max(1, num_gpus) * iteration / max(1, len(trainset))))
-    vit.train()
+    model.train()
     if num_gpus > 1:
         dist.barrier()
     graphed, n_accum, last_val, history = None, 0, (0.0, 0.0), []
@@ -180,7 +189,7 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
         for imgs, targets in train_loader:
             if rank == 0 and n_accum == 0 and iters_per_checkpoint and iteration % iters_per_checkpoint == 0:
                 save_checkpoint(model=vit, optimizer=optimizer, lr_scheduler=lr_scheduler,
-                                iteration=iteration, filepath=f"{out_dir}/vit_{iteration:06}")
+                                iteration=iteration, filepath=f"{out_dir}/vit_{iteration:06}", distiller=distiller)
             if rank == 0 and n_accum == 0 and iters_per_val and iteration % iters_per_val == 0 and len(valset):
                 last_val = validation(task, val_loader, device, criterion, vit)
             if device_matching:
@@ -191,7 +200,7 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
             imgs, targets = imgs.to(device, non_blocking=True), to_device(targets, device)
             if use_graph:
                 if graphed is None:
-                    graphed = GraphedTrainStep(net, criterion, imgs, targets)
+                    graphed = GraphedTrainStep(net, train_criterion, imgs, targets)
                 loss = graphed(imgs, targets)
             elif split_graph:
                 # detection: the matcher runs on the host between forward and backward, so the model's
@@ -203,11 +212,11 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
                 loss.backward()
             else:
                 if n_accum == 0:
-                    vit.zero_grad(set_to_none=True)
-                loss = criterion(net(imgs), targets)
+                    model.zero_grad(set_to_none=True)
+                loss = train_criterion(net(imgs), targets)
                 loss.backward()
             if optimizer_args.clip_grad is not None:
-                torch.nn.utils.clip_grad_norm_(vit.parameters(), optimizer_args.clip_grad)
+                torch.nn.utils.clip_grad_norm_(model.parameters(), optimizer_args.clip_grad)
             n_accum += 1
             if n_accum == n_batch_accum:
                 n_accum = 0
