@@ -29,7 +29,6 @@ extern "C" {
 /* element container types */
 #define MV_F32 0
 #define MV_F16 1
-#define MV_BF16 2
 
 /* rounding modes (qtorch: "nearest" / "stochastic") */
 #define MV_ROUND_NEAREST 0
@@ -82,10 +81,11 @@ int mv_quantize_weight(const float* w, void* out, void* out_t, int out_dtype, in
  * C[M,N] = A * B^T over K, fp32 accumulate in TMEM, fused epilogue.
  *   a_major/b_major = 0: operand stored [M|N, K] row-major (K contiguous)   — forward, dgrad
  *                   = 1: operand stored [K, M|N] row-major (M|N contiguous) — wgrad (dY^T, X^T)
- *   a_dtype == b_dtype: MV_F16 or MV_BF16 (kind::f16; the hardware rejects f16 x bf16) or MV_F32 (kind::tf32)
+ *   a_dtype == b_dtype: MV_F16 (CTA-pair kernel, kind::f16) or MV_F32 (single-CTA kernel, kind::tf32);
+ *   out_dtype: MV_F16 or MV_F32.  Any other type is an error.
  * Epilogue, in this order (each optional):
  *   acc (+ bias[n]) -> q_out -> [EPI_GELU: save u; acc = gelu(acc)] -> [EPI_DGELU: acc *= gelu'(u)]
- *   -> (+ residual[m,n]) -> q_res -> store out (out_dtype) and out2 (out2_dtype)
+ *   -> (+ residual[m,n]) -> q_res -> store out (out_dtype)
  *   accumulate != 0: out (fp32) += acc with red.global.add (split-K wgrad); bias/residual/q ignored.
  */
 #define MV_EPI_NONE 0
@@ -102,7 +102,6 @@ typedef struct {
     const float* residual; int ld_res;   /* fp32 [M, ld_res] or NULL */
     void* aux; int ld_aux;        /* fp16, see MV_EPI_* */
     void* out; int ld_out; int out_dtype;
-    void* out2; int ld_out2; int out2_dtype;   /* optional second copy (e.g. bf16 for backward) */
     int epilogue;
     int q_out_exp, q_out_man;     /* exp == 0: identity */
     int q_res_exp, q_res_man;
@@ -112,14 +111,13 @@ typedef struct {
     float* colsum;                /* NULL, or fp32 [N]: colsum[n] += sum over m of the value stored to out[m, n] (fp32, before
                                    * the container rounding) with red.add — the bias gradient of the Linear whose output
                                    * gradient this GEMM produces, without a second pass over it.  CTA-pair kernel only. */
-    int transpose_out;            /* accumulate only: out is [N, M] (pitch ld_out) and receives out[n, m] += acc[m, n] */
-    int cluster;                  /* 0 = CTA-pair kernel (tcgen05 cta_group::2, 256 x tile_n cluster tiles; 16-bit operands);
-                                   * 1 = single-CTA kernel (always used for tf32); any other value is an error */
+    int transpose_out;            /* accumulate only: out is [N, M] (pitch ld_out) and receives out[n, m] += acc[m, n].
+                                   * CTA-pair kernel only. */
     /* Dropout (see "dropout mask" below); drop_seed == NULL: off.  The output [M, N] is the site tensor (C = N):
      * value (m, n) is multiplied by keep(seed, site, m*N + n) * drop_scale right after q_out — before the residual
      * add and q_res; in MV_EPI_GELU both gelu(u) and the stored gelu'(u) are multiplied before they are rounded, so the
-     * MV_EPI_DGELU backward applies the mask without knowing about it.  CTA-pair kernel only (16-bit operands), not
-     * with accumulate or colsum. */
+     * MV_EPI_DGELU backward applies the mask without knowing about it.  CTA-pair kernel only, not with accumulate
+     * or colsum. */
     const uint64_t* drop_seed;    /* device pointer to the 64-bit seed */
     uint32_t drop_thr;            /* keep when bits16 >= drop_thr; drop_thr = nearbyint(p * 65536) */
     float drop_scale;             /* 1 / (1 - p) in fp32 (0 for p == 1) */
@@ -128,9 +126,8 @@ typedef struct {
      * the output [M, N] is element i = m*N + n of the site tensor, rounded to (q_out_exp, q_out_man), which must be a
      * float format, with the bits that mv_float_quantize(..., MV_ROUND_STOCHASTIC, *round_seed, round_offset) uses for
      * element i.  The rounding takes q_out's place in the epilogue (before the gelu' multiply of MV_EPI_DGELU).  An fp16
-     * output raises the overflow flag where the value before or after rounding does not fit fp16.  CTA-pair kernel only
-     * (16-bit operands, cluster == 0), plain or MV_EPI_DGELU outputs (colsum allowed; no accumulate, out2, residual or
-     * dropout). */
+     * output raises the overflow flag where the value before or after rounding does not fit fp16.  CTA-pair kernel only,
+     * plain or MV_EPI_DGELU outputs (colsum allowed; no accumulate, residual or dropout). */
     const uint64_t* round_seed;   /* device pointer to the 64-bit seed */
     uint64_t round_offset;
 } mv_gemm_args;
@@ -211,8 +208,6 @@ int mv_cls_rows(const float* cls, const float* pos_q, float* x, int B, int n_tok
                 int q_man, void* stream);
 /* x[b,row,:] = q(tok[:]) for every image b: the distillation token, which gets no positional embedding */
 int mv_token_row(const float* tok, float* x, int B, int n_tokens, int D, int row, int q_exp, int q_man, void* stream);
-/* fp32 -> fp16 (saturating) / bf16 copy of n elements (n % 4 == 0) */
-int mv_convert_f32(const float* in, void* out, int out_dtype, int64_t n, void* stream);
 /* out_f32[i] = in[i] * s and / or out_f16[i] = fp16_sat(in[i] * s) for n elements (n % 4 == 0; either output may
  * be NULL, out_f32 may alias in), s = *scale_dev or, with invert != 0, its reciprocal.  The backward's power-of-two
  * gradient scale is chosen on the device (no host sync); this applies / removes it in one pass. */
@@ -260,14 +255,6 @@ int mv_widen_transpose(const void* in, int in_dtype, int64_t ld, int rows, int c
  * (product error ~2^-21), i.e. an fp32-grade Linear on the kind::tf32 tensor-core path. */
 int mv_split_tf32(const float* in, int64_t ld, int rows, int cols, float* out, int mode, void* stream);
 
-/* Library-wide switches (testing / A-B measurement).  "attn_sn": 1 (default) = sequences of at most
- * 272 keys use the resident-K/V short-sequence attention kernels, 0 = always the blocked kernels.
- * "quant_ctas" (1..16, default 8): grid cap of the elementwise quantiser kernels, CTAs per SM.
- * "sm_limit" (16..148) with "sm_limit_launches" (n >= 0): the next n launches of the persistent kernels (CTA-pair
- * mv_gemm, short-sequence attention, mv_layernorm_q_bwd) size their grids for that many SMs — for launches that run
- * beside a gradient all-reduce (measured no gain on B200 / NVSwitch, DESIGN.md section 6; default: no limit). */
-int mv_set_option(const char* name, int value);
-
 /* ---------------------------------------------------------------- attention (tcgen05, flash-style)
  * Attention.forward's (q @ k^T) * scale -> softmax -> @ v -> transpose/reshape (models/vit.py:87-97).
  * qkv: fp16 [B*N, 3*H*64] as written by the to_qkv GEMM (q | k | v, 64 columns per head).
@@ -277,8 +264,8 @@ int mv_attention_fwd(const void* qkv, void* out, int out_dtype, float* lse, int 
                      float scale, int q_out_exp, int q_out_man, void* stream);
 /* autograd backward of the above.  o: the saved forward output (fp16), d_o: fp16 gradient w.r.t. it,
  * delta: fp32 [B,H,N] scratch, dqkv: fp16 [B*N, 3*H*64] (dq | dk | dv).
- * dq_accum: fp32 [B*N, H*64] scratch.  Non-NULL: one pass over key blocks, dQ accumulated across
- * key blocks with fp32 red.add (fast path).  NULL: deterministic two-pass variant without atomics.
+ * dq_accum: fp32 [B*N, H*64] scratch: dQ is accumulated across key blocks with fp32 red.add.  Required when the
+ * short-sequence kernel does not take the sequence (N > 272); an error if NULL there.
  * dbias: NULL or fp32 [3*H*64] (16-byte aligned): += the to_qkv Linear's bias gradient, i.e. the column sums of
  * dqkv.  The short-sequence kernel fuses it: the q part from the dQ rows it stores; the v part as the column sums
  * of d_o (sum_k dV[k,:] = sum_q (sum_k P[q,k]) dO[q,:] and the rows of P sum to one); the k part is left untouched

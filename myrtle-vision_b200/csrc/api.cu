@@ -1,6 +1,5 @@
 // api.cu — error reporting, launch counter and host-side TMA descriptor construction.
 #include <stdarg.h>
-#include <string.h>
 
 #include "common.cuh"
 #include "../../include/mv_b200.h"
@@ -9,9 +8,6 @@ namespace mv {
 
 static thread_local char g_err[512] = "";
 int64_t g_launches = 0;
-int g_opt_quant_ctas = 8;       // grid cap of the elementwise quant kernels, CTAs per SM
-int g_opt_sm_limit = 148, g_opt_sm_limit_launches = 0;   // see persistent_sms() (common.cuh)
-int g_opt_attn_sn = 1;          // short-sequence attention kernels (attention_sn.cu) when N fits
 int* g_overflow = nullptr;      // device int registered with mv_set_overflow_flag (NULL: no overflow reporting)
 
 void set_error(const char* fmt, ...) {
@@ -51,7 +47,6 @@ static EncodeTiledFn get_encode_fn() {
 static CUtensorMapDataType tmap_dtype(int dtype, int* esz) {
     switch (dtype) {
         case MV_F16: *esz = 2; return CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-        case MV_BF16: *esz = 2; return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
         default: *esz = 4; return CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
     }
 }
@@ -122,15 +117,6 @@ int make_tmap_3d(CUtensorMap* map, const void* ptr, int dtype, uint64_t d0, uint
 }  // namespace mv
 
 extern "C" const char* mv_last_error(void) { return mv::g_err; }
-extern "C" int mv_version(void) { return 104; }
+extern "C" int mv_version(void) { return 105; }
 extern "C" int mv_set_overflow_flag(int* flag_dev) { mv::g_overflow = flag_dev; return 0; }
 extern "C" int64_t mv_launch_count(void) { return mv::g_launches; }
-
-extern "C" int mv_set_option(const char* name, int value) {
-    if (name != nullptr && strcmp(name, "attn_sn") == 0) { mv::g_opt_attn_sn = value; return 0; }
-    if (name != nullptr && strcmp(name, "sm_limit") == 0 && value >= 16 && value <= mv::kNumSMs) { mv::g_opt_sm_limit = value; return 0; }
-    if (name != nullptr && strcmp(name, "sm_limit_launches") == 0 && value >= 0) { mv::g_opt_sm_limit_launches = value; return 0; }
-    if (name != nullptr && strcmp(name, "quant_ctas") == 0 && value >= 1 && value <= 16) { mv::g_opt_quant_ctas = value; return 0; }
-    mv::set_error("mv_set_option: unknown option '%s'", name ? name : "(null)");
-    return 1;
-}

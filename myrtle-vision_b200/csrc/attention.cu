@@ -16,10 +16,9 @@
 // Forward:  S = Q K^T (TMEM) -> online softmax in registers -> P (fp16) to swizzled smem ->
 //           O_j = P V (TMEM) -> rescale-accumulate in registers -> q_out -> fp16 store.
 //           Saves L = m + log2(l) (log2 domain) per row for the backward.
-// Backward: two passes, no atomics, deterministic:
-//   KV pass (CTA = key block):  dV += P^T dO,  dK += dS^T Q       (MN-major A operands)
-//   Q  pass (CTA = query block): dQ += dS K
-//   with P = exp2(S*c - L), dS = P * (dP - Delta) * scale, dP = dO V^T, Delta = rowsum(dO*O).
+// Backward (CTA = 64-key block, attn_bwd64_kernel): dV += P^T dO, dK += dS^T Q (MN-major A operands) over the
+//   query blocks; dQ_i += dS K_j by fp32 red.add into a scratch buffer that dq_convert_kernel rounds into dqkv.
+//   P = exp2(S*c - L), dS = P * (dP - Delta) * scale, dP = dO V^T, Delta = rowsum(dO*O).
 #include "common.cuh"
 #include "quant_dev.cuh"
 #include "../../include/mv_b200.h"
@@ -32,7 +31,6 @@ constexpr int kAttThreads = 192;
 constexpr int kTile = 16384;          // 128 rows x 128 B
 constexpr int kStgPitchF = 36;        // floats per staged fp32 row chunk (32 + 4 pad: conflict-free 16 B accesses)
 constexpr uint32_t kIdescPV = make_idesc(0, 0, 0, 1, 128, 64);     // A K-major, B MN-major, N=64
-constexpr uint32_t kIdescTT = make_idesc(0, 0, 1, 1, 128, 64);     // A MN-major, B MN-major, N=64
 
 __device__ __forceinline__ float sat16f(float v) { return fminf(fmaxf(v, -65504.f), 65504.f); }
 // {lo, hi} -> packed fp16x2 with saturation to +-65504 in one F2FP
@@ -313,231 +311,9 @@ struct AttnBwdDev {
     const float* lse;
     const float* delta;
     __half* dqkv; int ld_dqkv;
-    float* dq_accum;          // KV pass only: fp32 [B*N, D]; non-null => dQ += dS K by red.add (no Q pass)
+    float* dq_accum;          // fp32 [B*N, D]: dQ += dS K by red.add
     int* ovf;                 // overflow sink (mv_set_overflow_flag) or NULL
 };
-
-// kModeKV = true : CTA owns key block blockIdx.x; loops over query blocks; emits dK, dV.
-// kModeKV = false: CTA owns query block blockIdx.x; loops over key blocks;  emits dQ.
-template <bool kModeKV>
-__global__ void __launch_bounds__(kAttThreads, 1)
-attn_bwd_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_do,
-                const AttnBwdDev p) {
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // 1024-aligned; offset arithmetic keeps the shared address space
-    uint8_t* sR0 = smem;                       // resident: K_j (KV) | Q_i (Q)
-    uint8_t* sR1 = smem + kTile;               // resident: V_j (KV) | dO_i (Q)
-    uint8_t* sRing = smem + 2 * kTile;         // [2 stages][X, Y]: (Q_i, dO_i) (KV) | (K_j, V_j) (Q)
-    uint8_t* sdS = smem + 6 * kTile;           // dS fp16, two 64-column sub-tiles
-    uint8_t* sP = smem + 8 * kTile;            // P fp16 (KV mode only)
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (kModeKV ? 10 : 8) * kTile);
-    uint64_t* res_full = bars;
-    uint64_t* ring_full = bars + 1;            // [2]
-    uint64_t* ring_empty = bars + 3;           // [2]
-    uint64_t* sdp_full = bars + 5;
-    uint64_t* pds_full = bars + 6;
-    uint64_t* pds_empty = bars + 7;
-    uint64_t* dq_full = bars + 8;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
-    const bool fuse_dq = kModeKV && p.dq_accum != nullptr;
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int blk0 = blockIdx.x * 128, h = blockIdx.y, b = blockIdx.z;
-    const int nblk = (p.N + 127) / 128;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmap_qkv);
-        tma_prefetch_desc(&tmap_do);
-        mbar_init(res_full, 1);
-        for (int s = 0; s < 2; s++) { mbar_init(&ring_full[s], 1); mbar_init(&ring_empty[s], 1); }
-        mbar_init(sdp_full, 1); mbar_init(pds_full, 4); mbar_init(pds_empty, 1); mbar_init(dq_full, 1);
-        fence_barrier_init();
-    }
-    if (warp == 1) tmem_alloc<512>(tmem_slot);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t tS = tmem_base, tdP = tmem_base + 128, tAcc0 = tmem_base + 256, tAcc1 = tmem_base + 320, tdQ = tmem_base + 384;
-
-    if (warp == 0) {
-        if (lane == 0) {
-            mbar_arrive_expect_tx(res_full, 2 * kTile);
-            if (kModeKV) {
-                tma_load_3d(sR0, &tmap_qkv, res_full, p.D + h * 64, blk0, b);        // K_j
-                tma_load_3d(sR1, &tmap_qkv, res_full, 2 * p.D + h * 64, blk0, b);    // V_j
-            } else {
-                tma_load_3d(sR0, &tmap_qkv, res_full, h * 64, blk0, b);              // Q_i
-                tma_load_3d(sR1, &tmap_do, res_full, h * 64, blk0, b);               // dO_i
-            }
-            for (int it = 0; it < nblk; it++) {
-                const int st = it & 1;
-                mbar_wait(&ring_empty[st], ((it >> 1) & 1) ^ 1);
-                mbar_arrive_expect_tx(&ring_full[st], 2 * kTile);
-                uint8_t* x = sRing + st * 2 * kTile;
-                if (kModeKV) {
-                    tma_load_3d(x, &tmap_qkv, &ring_full[st], h * 64, it * 128, b);             // Q_i
-                    tma_load_3d(x + kTile, &tmap_do, &ring_full[st], h * 64, it * 128, b);      // dO_i
-                } else {
-                    tma_load_3d(x, &tmap_qkv, &ring_full[st], p.D + h * 64, it * 128, b);       // K_j
-                    tma_load_3d(x + kTile, &tmap_qkv, &ring_full[st], 2 * p.D + h * 64, it * 128, b);   // V_j
-                }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0) {
-            const uint32_t aR0 = smem_u32(sR0), aR1 = smem_u32(sR1), adS = smem_u32(sdS), aP = smem_u32(sP);
-            mbar_wait(res_full, 0);
-            for (int it = 0; it < nblk; it++) {
-                const int st = it & 1;
-                mbar_wait(&ring_full[st], (it >> 1) & 1);
-                tc_fence_after();
-                const uint32_t aX = smem_u32(sRing + st * 2 * kTile), aY = aX + kTile;
-                // S = Q K^T ; dP = dO V^T   (all operands K-major over d)
-                const uint32_t aQ = kModeKV ? aX : aR0, aK = kModeKV ? aR0 : aX;
-                const uint32_t aDO = kModeKV ? aY : aR1, aV = kModeKV ? aR1 : aY;
-                // partial last blocks: only the keys / query rows that exist (rounded up to 16) are multiplied
-                const int kbase = kModeKV ? blk0 : it * 128, qbase = kModeKV ? it * 128 : blk0;
-                const int nk16 = (min(128, p.N - kbase) + 15) & ~15, nq16 = (min(128, p.N - qbase) + 15) & ~15;
-                const uint32_t idesc_s = make_idesc(0, 0, 0, 0, 128, nk16);
-#pragma unroll
-                for (int k = 0; k < 4; k++)
-                    umma_f16(tS, make_smem_desc_sw128(aQ + k * 32, 16, 1024), make_smem_desc_sw128(aK + k * 32, 16, 1024), idesc_s, k > 0);
-#pragma unroll
-                for (int k = 0; k < 4; k++)
-                    umma_f16(tdP, make_smem_desc_sw128(aDO + k * 32, 16, 1024), make_smem_desc_sw128(aV + k * 32, 16, 1024), idesc_s, k > 0);
-                umma_commit(sdp_full);
-                mbar_wait(pds_full, it & 1);
-                tc_fence_after();
-                if (kModeKV) {
-                    // dV[keys, d] += P^T dO : A = P as MN-major (M = keys), B = dO as MN-major (N = d); K = q rows
-                    for (int k = 0; k < (nq16 >> 4); k++)
-                        umma_f16(tAcc0, make_smem_desc_sw128(aP + k * 2048, kTile, 1024),
-                                 make_smem_desc_sw128(aDO + k * 2048, 8192, 1024), kIdescTT, (it > 0 || k > 0));
-                    // dK[keys, d] += dS^T Q
-                    for (int k = 0; k < (nq16 >> 4); k++)
-                        umma_f16(tAcc1, make_smem_desc_sw128(adS + k * 2048, kTile, 1024),
-                                 make_smem_desc_sw128(aQ + k * 2048, 8192, 1024), kIdescTT, (it > 0 || k > 0));
-                    if (fuse_dq) {
-                        // this key block's contribution to dQ_i = dS K_j, handed to the threads for red.add
-                        for (int k = 0; k < (nk16 >> 4); k++)
-                            umma_f16(tdQ, make_smem_desc_sw128(adS + (k >> 2) * kTile + (k & 3) * 32, 16, 1024),
-                                     make_smem_desc_sw128(aK + k * 2048, 8192, 1024), kIdescPV, k > 0);
-                        umma_commit(dq_full);
-                    }
-                } else {
-                    // dQ[q, d] += dS K : A = dS K-major over keys, B = K_j as MN-major (N = d); K = keys
-                    for (int k = 0; k < (nk16 >> 4); k++)
-                        umma_f16(tAcc0, make_smem_desc_sw128(adS + (k >> 2) * kTile + (k & 3) * 32, 16, 1024),
-                                 make_smem_desc_sw128(aK + k * 2048, 8192, 1024), kIdescPV, (it > 0 || k > 0));
-                }
-                umma_commit(&ring_empty[st]);
-                umma_commit(pds_empty);
-            }
-        }
-    } else {
-        const int quad = warp & 3;
-        const int r = quad * 32 + lane;
-        const uint32_t lane_off = uint32_t(quad * 32) << 16;
-        for (int it = 0; it < nblk; it++) {
-            // thread row = query row of the current q block
-            const int qrow = (kModeKV ? it * 128 : blk0) + r;
-            const int kbase = kModeKV ? blk0 : it * 128;
-            const bool q_ok = qrow < p.N;
-            float L = 0.f, dl = 0.f;
-            if (q_ok) {
-                const int64_t si = (int64_t(b) * p.H + h) * p.N + qrow;
-                L = p.lse[si]; dl = p.delta[si];
-            }
-            const int nk16 = (min(128, p.N - kbase) + 15) & ~15;
-            const int nq16 = (min(128, p.N - (kModeKV ? it * 128 : blk0)) + 15) & ~15;
-            // warps whose 32 rows lie beyond the rows the MMAs consume have nothing to produce
-            const int nchunk = (quad * 32 < nq16) ? ((nk16 + 31) >> 5) : 0;
-            mbar_wait(sdp_full, it & 1);
-            tc_fence_after();
-            mbar_wait(pds_empty, (it & 1) ^ 1);       // previous iteration's MMAs are done with sP / sdS
-#pragma unroll 1
-            for (int c = 0; c < nchunk; c++) {
-                uint32_t s[32], dp[32];
-                tmem_ld_32x32(tS + lane_off + c * 32, s);
-                tmem_ld_32x32(tdP + lane_off + c * 32, dp);
-                tmem_ld_wait();
-                uint32_t wp[16], wd[16];
-#pragma unroll
-                for (int t = 0; t < 16; t++) {
-                    float pv[2], dv[2];
-#pragma unroll
-                    for (int u = 0; u < 2; u++) {
-                        const bool ok = q_ok && (kbase + c * 32 + 2 * t + u < p.N);
-                        const float pe = ok ? ex2_fast(fmaf(__uint_as_float(s[2 * t + u]), p.scale_log2, -L)) : 0.f;
-                        pv[u] = pe;
-                        dv[u] = pe * (__uint_as_float(dp[2 * t + u]) - dl) * p.scale;
-                    }
-                    wp[t] = pack_h2(pv[0], pv[1]);
-                    wd[t] = pack_h2_sat(dv[0], dv[1]);
-                }
-                store_p_chunk(sdS, r, c, wd);
-                if (kModeKV) store_p_chunk(sP, r, c, wp);
-            }
-            fence_proxy_async();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(pds_full);
-            if (fuse_dq) {
-                mbar_wait(dq_full, it & 1);
-                tc_fence_after();
-                if (nchunk > 0) {
-                    float* dst = p.dq_accum + (int64_t(b) * p.N + qrow) * p.D + h * 64;
-#pragma unroll
-                    for (int c = 0; c < 2; c++) {
-                        uint32_t v[32];
-                        tmem_ld_32x32(tdQ + lane_off + c * 32, v);
-                        tmem_ld_wait();
-                        if (q_ok) {
-#pragma unroll
-                            for (int i = 0; i < 8; i++)
-                                atomicAdd(reinterpret_cast<float4*>(dst + c * 32) + i,
-                                          make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]),
-                                                      __uint_as_float(v[4 * i + 2]), __uint_as_float(v[4 * i + 3])));
-                        }
-                    }
-                }
-                tc_fence_before();
-            }
-        }
-        // all accumulating MMAs of the last iteration have retired
-        mbar_wait(pds_empty, (nblk - 1) & 1);
-        tc_fence_after();
-        const int orow = blk0 + r;              // key row (KV mode) or query row (Q mode)
-        for (int a = 0; a < (kModeKV ? 2 : 1); a++) {
-            uint32_t v[32];
-            // KV: acc0 = dV -> columns 2D + h*64 ; acc1 = dK -> columns D + h*64.  Q: acc0 = dQ -> h*64
-            const int col = kModeKV ? ((a == 0 ? 2 : 1) * p.D + h * 64) : h * 64;
-            __half* dst = p.dqkv + (int64_t(b) * p.N + orow) * p.ld_dqkv + col;
-#pragma unroll
-            for (int c = 0; c < 2; c++) {
-                tmem_ld_32x32((a == 0 ? tAcc0 : tAcc1) + lane_off + c * 32, v);
-                tmem_ld_wait();
-                if (orow < p.N) {
-                    float amax = 0.f;
-#pragma unroll
-                    for (int i = 0; i < 32; i++) amax = fmaxf(amax, fabsf(__uint_as_float(v[i])));
-                    raise_overflow(p.ovf, amax);
-#pragma unroll
-                    for (int i = 0; i < 4; i++)
-                        reinterpret_cast<uint4*>(dst + c * 32)[i] =
-                            make_uint4(pack_h2(sat16f(__uint_as_float(v[8 * i])), sat16f(__uint_as_float(v[8 * i + 1]))),
-                                       pack_h2(sat16f(__uint_as_float(v[8 * i + 2])), sat16f(__uint_as_float(v[8 * i + 3]))),
-                                       pack_h2(sat16f(__uint_as_float(v[8 * i + 4])), sat16f(__uint_as_float(v[8 * i + 5]))),
-                                       pack_h2(sat16f(__uint_as_float(v[8 * i + 6])), sat16f(__uint_as_float(v[8 * i + 7]))));
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 1) { tc_fence_after(); tmem_dealloc<512>(tmem_base); }
-}
 
 // ---------------------------------------------------------------------------------------------
 // Backward, 64-key blocks: 80 KB of shared memory and 256 TMEM columns per CTA so that two CTAs
@@ -781,14 +557,11 @@ dq_convert_kernel(const float* __restrict__ dq, __half* __restrict__ dqkv, int64
 }
 
 constexpr int kAttnFwdSmem = 5 * kTile + 1024 + 256;
-constexpr int kAttnBwdKVSmem = 10 * kTile + 1024 + 256;
-constexpr int kAttnBwdQSmem = 8 * kTile + 1024 + 256;
 
 }  // namespace mv
 
 using namespace mv;
 
-namespace mv { extern int g_opt_attn_sn; }
 extern "C" int mv_attention_sn_supported(int N);
 int mv_attention_fwd_sn(const void* qkv, void* out, int out_dtype, float* lse, int B, int H, int N,
                         float scale, int q_out_exp, int q_out_man, void* stream);
@@ -799,7 +572,7 @@ extern "C" int mv_attention_fwd(const void* qkv, void* out, int out_dtype, float
                                 float scale, int q_out_exp, int q_out_man, void* stream) {
     MV_CHECK(B > 0 && H > 0 && N > 0 && qkv && out, "mv_attention_fwd: bad arguments");
     MV_CHECK(out_dtype == MV_F16 || out_dtype == MV_F32, "mv_attention_fwd: bad output container");
-    if (g_opt_attn_sn && mv_attention_sn_supported(N))
+    if (mv_attention_sn_supported(N))
         return mv_attention_fwd_sn(qkv, out, out_dtype, lse, B, H, N, scale, q_out_exp, q_out_man, stream);
     const int D = H * 64;
     static bool attr_done = false;
@@ -826,13 +599,12 @@ extern "C" int mv_attention_bwd(const void* qkv, const void* o, const void* d_o,
                                 void* stream) {
     MV_CHECK(B > 0 && H > 0 && N > 0 && qkv && o && d_o && lse && delta && dqkv, "mv_attention_bwd: bad arguments");
     MV_CHECK((reinterpret_cast<uintptr_t>(dbias) & 15) == 0, "mv_attention_bwd: dbias must be 16-byte aligned");
-    if (g_opt_attn_sn && N <= 272)
+    if (N <= 272)
         return mv_attention_bwd_sn(qkv, o, d_o, lse, delta, dqkv, dbias, B, H, N, scale, stream);
+    MV_CHECK(dq_accum != nullptr, "mv_attention_bwd: N = %d > 272 needs dq_accum (fp32 [B*N, H*64] scratch)", N);
     const int D = H * 64;
     static bool attr_done = false;
     if (!attr_done) {
-        MV_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnBwdKVSmem));
-        MV_CUDA(cudaFuncSetAttribute(attn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnBwdQSmem));
         MV_CUDA(cudaFuncSetAttribute(attn_bwd64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnBwd64Smem));
         attr_done = true;
     }
@@ -850,27 +622,18 @@ extern "C" int mv_attention_bwd(const void* qkv, const void* o, const void* d_o,
     p.dqkv = reinterpret_cast<__half*>(dqkv); p.ld_dqkv = 3 * D;
     p.dq_accum = dq_accum;
     p.ovf = g_overflow;
-    dim3 grid((N + 127) / 128, H, B);
-    if (dq_accum != nullptr) {
-        // one pass: dK, dV per key block and dQ accumulated across key blocks with fp32 red.add
-        const int64_t n = int64_t(B) * N * D;
-        MV_CUDA(cudaMemsetAsync(dq_accum, 0, sizeof(float) * n, st));
-        CUtensorMap tk64;
-        if (make_tmap_3d(&tk64, qkv, MV_F16, 3 * D, N, B, 3 * D, uint64_t(N) * 3 * D, 64, 64, 1)) return 1;
-        dim3 grid64((N + 63) / 64, H, B);
-        attn_bwd64_kernel<<<grid64, kAttThreads, kAttnBwd64Smem, st>>>(tq, tk64, td, p);
-        g_launches++;
-        int64_t blocks = (n / 4 + 255) / 256;
-        if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-        dq_convert_kernel<<<int(blocks), 256, 0, st>>>(dq_accum, reinterpret_cast<__half*>(dqkv), int64_t(B) * N, D, 3 * D, g_overflow);
-        g_launches++;
-    } else {
-        // deterministic two-pass variant (no atomics): the Q pass recomputes S and dP
-        attn_bwd_kernel<true><<<grid, kAttThreads, kAttnBwdKVSmem, st>>>(tq, td, p);
-        g_launches++;
-        attn_bwd_kernel<false><<<grid, kAttThreads, kAttnBwdQSmem, st>>>(tq, td, p);
-        g_launches++;
-    }
+    // dK, dV per key block and dQ accumulated across key blocks with fp32 red.add
+    const int64_t n = int64_t(B) * N * D;
+    MV_CUDA(cudaMemsetAsync(dq_accum, 0, sizeof(float) * n, st));
+    CUtensorMap tk64;
+    if (make_tmap_3d(&tk64, qkv, MV_F16, 3 * D, N, B, 3 * D, uint64_t(N) * 3 * D, 64, 64, 1)) return 1;
+    dim3 grid64((N + 63) / 64, H, B);
+    attn_bwd64_kernel<<<grid64, kAttThreads, kAttnBwd64Smem, st>>>(tq, tk64, td, p);
+    g_launches++;
+    int64_t blocks = (n / 4 + 255) / 256;
+    if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
+    dq_convert_kernel<<<int(blocks), 256, 0, st>>>(dq_accum, reinterpret_cast<__half*>(dqkv), int64_t(B) * N, D, 3 * D, g_overflow);
+    g_launches++;
     if (check_cuda(cudaGetLastError(), "attention bwd launch")) return 1;
     // long sequences: the bias gradient is a separate pass over dqkv (the short-sequence kernel fuses it)
     if (dbias != nullptr) return mv_colsum(dqkv, MV_F16, 3 * D, B * N, 3 * D, dbias, stream);

@@ -1552,8 +1552,7 @@ int mv_attention_fwd_sn(const void* qkv, void* out, int out_dtype, float* lse, i
     p.q_out = FloatFmt{q_out_exp, q_out_man};
     p.lse = lse;
     const int n_bh = B * H;
-    const int sms = persistent_sms();
-    const int grid = n_bh < sms ? n_bh : sms;
+    const int grid = n_bh < kNumSMs ? n_bh : kNumSMs;
     attn_fwd_sn_kernel<<<grid, kSnFwdThreads, kSnFwdSmem, static_cast<cudaStream_t>(stream)>>>(t128, t16, p);
     g_launches++;
     return check_cuda(cudaGetLastError(), "attention fwd (short-sequence) launch");
@@ -1595,9 +1594,8 @@ int mv_attention_bwd_sn(const void* qkv, const void* o, const void* d_o, const f
     // Fused bias gradient: the kernel keeps per-head sums in registers, so a CTA must stay on one head — pair index =
     // blockIdx + n * grid with the grid a multiple of H (or one pair per CTA).  Same number of rounds as a full grid
     // whenever ceil(n_bh / grid) does not change (B = 256, H = 6: 11 rounds with 144 or 148 CTAs).
-    const int sms = persistent_sms();
-    const bool fuse = dbias != nullptr && H <= sms;
-    const int grid = n_bh <= sms ? n_bh : (fuse ? (sms / H) * H : sms);
+    const bool fuse = dbias != nullptr && H <= kNumSMs;
+    const int grid = n_bh <= kNumSMs ? n_bh : (fuse ? (kNumSMs / H) * H : kNumSMs);
     p.dbias = fuse ? dbias : nullptr;
     p.ovf = g_overflow;
     attn_bwd_sn_kernel<<<grid, kSnBwdThreads, kSnBwdSmem, st>>>(q128, q16, d128, d16, s128, p);

@@ -2,7 +2,6 @@
 // Hand-written for this repo; no CUTLASS/CuTe in the product path.
 #pragma once
 #include <cuda.h>
-#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -28,17 +27,6 @@ int check_cuda(cudaError_t e, const char* what);
     } while (0)
 
 constexpr int kNumSMs = 148;
-// SMs the persistent kernels (CTA-pair GEMM, short-sequence attention, LayerNorm backward) size their grids for.  Normally
-// all 148.  Data-parallel training lowers it for the few launches that run beside a gradient all-reduce (options
-// "sm_limit" + "sm_limit_launches"): a persistent kernel strides a FIXED share of the work per CTA, so when NCCL's CTAs hold
-// some SMs its last CTAs run as a second wave and the kernel takes twice as long; sized for the SMs that are free, it loses
-// only their share.
-extern int g_opt_sm_limit, g_opt_sm_limit_launches;
-inline int persistent_sms() {
-    if (g_opt_sm_limit_launches <= 0) return kNumSMs;
-    g_opt_sm_limit_launches--;
-    return g_opt_sm_limit < kNumSMs ? (g_opt_sm_limit & ~1) : kNumSMs;
-}
 
 // Overflow sink (mv_set_overflow_flag): kernels that round gradient values into fp16 containers keep the largest
 // |value| they convert and raise the flag when it would not fit (>= 65520 rounds past 65504: the container
@@ -343,7 +331,7 @@ __host__ __device__ constexpr uint32_t make_idesc(int a_fmt, int b_fmt, int a_ma
 }
 
 // ------------------------------------------------------- host: TMA maps
-// dtype: 0 = f32 (4 B), 1 = f16, 2 = bf16.  2-D row-major tensor [rows, cols] with row pitch
+// dtype: MV_F32 (4 B) or MV_F16 (2 B).  2-D row-major tensor [rows, cols] with row pitch
 // `ld` elements; box = [box_rows, box_cols]; 128-byte swizzle.
 int make_tmap_2d(CUtensorMap* map, const void* ptr, int dtype, uint64_t rows, uint64_t cols,
                  uint64_t ld, uint32_t box_rows, uint32_t box_cols);

@@ -23,12 +23,11 @@ constexpr int BM = 128;
 constexpr int kATileBytes = BM * 128;                 // A tile per stage: 128 rows x 128 B = 16 KB
 constexpr int kEpiWarps = 16;                         // four warps per TMEM lane quadrant
 constexpr int kGemmThreads = 64 + 32 * kEpiWarps;
-template <int BN> struct GemmCfg {
-    static constexpr int kBTileBytes = BN * 128;
-    static constexpr int kStageBytes = kATileBytes + kBTileBytes;
-    static constexpr int kStages = BN == 128 ? 6 : 4;
-    static constexpr int kSmem = kStages * kStageBytes + 1024 /*align slack*/ + 256 /*barriers*/;
-};
+// single-CTA kernel: 128 x 128 tiles, 6-stage ring
+constexpr int kGemmBN = 128;
+constexpr int kGemmStages = 6;
+constexpr int kGemmStageBytes = kATileBytes + kGemmBN * 128;
+constexpr int kGemmSmem = kGemmStages * kGemmStageBytes + 1024 /*align slack*/ + 256 /*barriers*/;
 
 // Debug timeline (tools/trace_gemm.py, library built with MV_NVCC_FLAGS=-DMV_GEMM_TRACE): CTA 0 stamps
 // clock64() at the hand-offs between the MMA issuer and two of its epilogue warps.  Record = {event, index, clock}.
@@ -58,7 +57,6 @@ struct GemmDev {
     const float* residual; int ld_res;
     __half* aux; int ld_aux;
     void* out; int ld_out; int out_dtype;
-    void* out2; int ld_out2; int out2_dtype;
     int epilogue;
     FloatFmt q_out, q_res;
     int accumulate;
@@ -170,15 +168,6 @@ __device__ __forceinline__ void store16(__half* dst, const float (&v)[16]) {
                                                      *reinterpret_cast<uint32_t*>(&h2), *reinterpret_cast<uint32_t*>(&h3));
     }
 }
-__device__ __forceinline__ void store16(__nv_bfloat16* dst, const float (&v)[16]) {
-#pragma unroll
-    for (int j = 0; j < 2; j++) {
-        __nv_bfloat162 h0 = __floats2bfloat162_rn(v[8 * j + 0], v[8 * j + 1]), h1 = __floats2bfloat162_rn(v[8 * j + 2], v[8 * j + 3]);
-        __nv_bfloat162 h2 = __floats2bfloat162_rn(v[8 * j + 4], v[8 * j + 5]), h3 = __floats2bfloat162_rn(v[8 * j + 6], v[8 * j + 7]);
-        reinterpret_cast<uint4*>(dst)[j] = make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1),
-                                                     *reinterpret_cast<uint32_t*>(&h2), *reinterpret_cast<uint32_t*>(&h3));
-    }
-}
 // row-major store of 16 consecutive outputs; fp16 stores saturate (gradient operands)
 __device__ __forceinline__ void store_out16(void* base, int dtype, int64_t row, int ld, int col,
                                             float (&v)[16], bool vec_ok, int nvalid) {
@@ -186,75 +175,24 @@ __device__ __forceinline__ void store_out16(void* base, int dtype, int64_t row, 
         float* p = reinterpret_cast<float*>(base) + row * ld + col;
         if (vec_ok) store16(p, v);
         else for (int j = 0; j < 16; j++) if (j < nvalid) p[j] = v[j];
-    } else if (dtype == MV_F16) {
+    } else {
 #pragma unroll
         for (int j = 0; j < 16; j++) v[j] = sat16(v[j]);
         __half* p = reinterpret_cast<__half*>(base) + row * ld + col;
         if (vec_ok) store16(p, v);
         else for (int j = 0; j < 16; j++) if (j < nvalid) p[j] = __float2half_rn(v[j]);
-    } else {
-        __nv_bfloat16* p = reinterpret_cast<__nv_bfloat16*>(base) + row * ld + col;
-        if (vec_ok) store16(p, v);
-        else for (int j = 0; j < 16; j++) if (j < nvalid) p[j] = __float2bfloat16_rn(v[j]);
     }
 }
 
-template <typename T> __device__ __forceinline__ void store_row32(T* dst, const float (&v)[32]);
-template <> __device__ __forceinline__ void store_row32<float>(float* dst, const float (&v)[32]) {
-#pragma unroll
-    for (int j = 0; j < 8; j++)
-        reinterpret_cast<float4*>(dst)[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-}
-template <> __device__ __forceinline__ void store_row32<__half>(__half* dst, const float (&v)[32]) {
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-        __half2 h0 = __floats2half2_rn(sat16(v[8 * j + 0]), sat16(v[8 * j + 1]));
-        __half2 h1 = __floats2half2_rn(sat16(v[8 * j + 2]), sat16(v[8 * j + 3]));
-        __half2 h2 = __floats2half2_rn(sat16(v[8 * j + 4]), sat16(v[8 * j + 5]));
-        __half2 h3 = __floats2half2_rn(sat16(v[8 * j + 6]), sat16(v[8 * j + 7]));
-        reinterpret_cast<uint4*>(dst)[j] =
-            make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1),
-                       *reinterpret_cast<uint32_t*>(&h2), *reinterpret_cast<uint32_t*>(&h3));
-    }
-}
-template <> __device__ __forceinline__ void store_row32<__nv_bfloat16>(__nv_bfloat16* dst, const float (&v)[32]) {
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-        __nv_bfloat162 h0 = __floats2bfloat162_rn(v[8 * j + 0], v[8 * j + 1]);
-        __nv_bfloat162 h1 = __floats2bfloat162_rn(v[8 * j + 2], v[8 * j + 3]);
-        __nv_bfloat162 h2 = __floats2bfloat162_rn(v[8 * j + 4], v[8 * j + 5]);
-        __nv_bfloat162 h3 = __floats2bfloat162_rn(v[8 * j + 6], v[8 * j + 7]);
-        reinterpret_cast<uint4*>(dst)[j] =
-            make_uint4(*reinterpret_cast<uint32_t*>(&h0), *reinterpret_cast<uint32_t*>(&h1),
-                       *reinterpret_cast<uint32_t*>(&h2), *reinterpret_cast<uint32_t*>(&h3));
-    }
-}
-
-__device__ __forceinline__ void store_out(void* base, int dtype, int64_t row, int ld, int col,
-                                          const float (&v)[32], bool vec_ok, int ncols_valid) {
-    if (dtype == MV_F32) {
-        float* p = reinterpret_cast<float*>(base) + row * ld + col;
-        if (vec_ok) store_row32<float>(p, v);
-        else for (int j = 0; j < 32; j++) if (j < ncols_valid) p[j] = v[j];
-    } else if (dtype == MV_F16) {
-        __half* p = reinterpret_cast<__half*>(base) + row * ld + col;
-        if (vec_ok) store_row32<__half>(p, v);
-        else for (int j = 0; j < 32; j++) if (j < ncols_valid) p[j] = __float2half_rn(sat16(v[j]));
-    } else {
-        __nv_bfloat16* p = reinterpret_cast<__nv_bfloat16*>(base) + row * ld + col;
-        if (vec_ok) store_row32<__nv_bfloat16>(p, v);
-        else for (int j = 0; j < 32; j++) if (j < ncols_valid) p[j] = __float2bfloat16_rn(v[j]);
-    }
-}
-
-// kEsz: operand element size (2: f16/bf16, kind::f16; 4: tf32-in-fp32, kind::tf32)
-template <int BN, int kEsz>
+// Single-CTA kernel: tf32-in-fp32 operands (kind::tf32), 128 x 128 tiles.
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
             const GemmDev p) {
-    constexpr int kStages = GemmCfg<BN>::kStages;
-    constexpr int kStageBytes = GemmCfg<BN>::kStageBytes;
+    constexpr int BN = kGemmBN;
+    constexpr int kStages = kGemmStages;
+    constexpr int kStageBytes = kGemmStageBytes;
     constexpr int kTileBytes = kATileBytes;
+    constexpr int kEsz = 4;                    // operand element size
     constexpr int BK = 128 / kEsz;             // elements of K per stage (one 128-byte swizzle row)
     constexpr int UMMA_K = 32 / kEsz;          // K elements per tcgen05.mma
     constexpr int kMnChunk = 128 / kEsz;       // MN elements per 128-byte row (MN-major tiles)
@@ -351,8 +289,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                         const uint64_t adesc = make_smem_desc_sw128(sa + k * a_kstep, a_lbo, 1024);
                         const uint64_t bdesc = make_smem_desc_sw128(sb + k * b_kstep, b_lbo, 1024);
                         const uint32_t accum = (kb > kb0 || k > 0) ? 1u : 0u;
-                        if (kEsz == 2) umma_f16(tmem_d, adesc, bdesc, p.idesc, accum);
-                        else umma_tf32(tmem_d, adesc, bdesc, p.idesc, accum);
+                        umma_tf32(tmem_d, adesc, bdesc, p.idesc, accum);
                     }
                     umma_commit(&empty_bar[stage]);            // frees the smem slot when the MMAs retire
                     if (++stage == kStages) { stage = 0; phase ^= 1; }
@@ -482,11 +419,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                 const int esz_o = p.out_dtype == MV_F32 ? 4 : 2;
                 const bool vec_o = full && ((p.ld_out * esz_o) % 16 == 0);
                 store_out16(p.out, p.out_dtype, m, p.ld_out, n, v, vec_o, nvalid);
-                if (p.out2 != nullptr) {
-                    const int esz_2 = p.out2_dtype == MV_F32 ? 4 : 2;
-                    const bool vec_2 = full && ((p.ld_out2 * esz_2) % 16 == 0);
-                    store_out16(p.out2, p.out2_dtype, m, p.ld_out2, n, v, vec_2, nvalid);
-                }
             }
             tc_fence_before();
             __syncwarp();
@@ -503,7 +435,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
 }
 
 // =====================================================================================
-// CTA-pair kernel (cta_group::2): the default for 16-bit operands.
+// CTA-pair kernel (cta_group::2): fp16 operands.
 //
 // A cluster of two CTAs (one TPC) owns a 256 x BN output tile.  Each CTA stages its own 128 rows
 // of A and BN/2 rows of B (one third less L2->SM operand traffic per flop than two independent
@@ -524,7 +456,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
 // put five warps on one scheduler's 16 K registers, which caps every thread at 96 registers and makes the
 // epilogues with residual / aux prefetch spill; 14 warps (12 + 2) allow 128.  The elementwise-heavy GELU /
 // gelu' epilogues (N = 1536 outputs) are bound by issue slots and latency and run faster on 16 warps; every
-// other epilogue runs faster on 12 spill-free ones (measured per shape, gpurun_out/probe_gemm2*.log).
+// other epilogue runs faster on 12 spill-free ones (measured per shape).
 constexpr int kStgPitch = 36;                                  // floats per staged row: 32 + 4 pad
 constexpr int kStgBytesPerWarp = 32 * kStgPitch * 4;           // 4608
 // AUX: the gelu' epilogue's second operand (aux, fp16 [M, N]) arrives by TMA, one 32 x 32 chunk per epilogue warp, requested
@@ -555,25 +487,17 @@ __device__ __forceinline__ uint2 pack4_f16_sat(const float (&v)[4]) {
     asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r.y) : "f"(v[3]), "f"(v[2]));
     return r;
 }
-__device__ __forceinline__ uint2 pack4_bf16(const float (&v)[4]) {
-    __nv_bfloat162 a = __floats2bfloat162_rn(v[0], v[1]), b = __floats2bfloat162_rn(v[2], v[3]);
-    return make_uint2(*reinterpret_cast<uint32_t*>(&a), *reinterpret_cast<uint32_t*>(&b));
-}
-// 4 consecutive outputs of one row; vec: 16-byte (fp32) / 8-byte (16-bit) aligned and all 4 in range
+// 4 consecutive outputs of one row; vec: 16-byte (fp32) / 8-byte (fp16) aligned and all 4 in range
 __device__ __forceinline__ void store_out4(void* base, int dtype, int64_t row, int ld, int col,
                                            const float (&v)[4], bool vec, int nvalid) {
     if (dtype == MV_F32) {
         float* o = reinterpret_cast<float*>(base) + row * ld + col;
         if (vec) *reinterpret_cast<float4*>(o) = make_float4(v[0], v[1], v[2], v[3]);
         else for (int j = 0; j < 4; j++) if (j < nvalid) o[j] = v[j];
-    } else if (dtype == MV_F16) {
+    } else {
         __half* o = reinterpret_cast<__half*>(base) + row * ld + col;
         if (vec) *reinterpret_cast<uint2*>(o) = pack4_f16_sat(v);
         else for (int j = 0; j < 4; j++) if (j < nvalid) o[j] = __float2half_rn(sat16(v[j]));
-    } else {
-        __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(base) + row * ld + col;
-        if (vec) *reinterpret_cast<uint2*>(o) = pack4_bf16(v);
-        else for (int j = 0; j < 4; j++) if (j < nvalid) o[j] = __float2bfloat16_rn(v[j]);
     }
 }
 
@@ -833,7 +757,7 @@ __device__ __forceinline__ void epi_chunk_acc_t(const GemmDev& p, const EpiWarp&
     __syncwarp();
 }
 
-// Generic path: tails in M / N, unaligned pitches, bf16 / second outputs.  Same arithmetic, rolled loops.
+// Generic path: tails in M / N, unaligned pitches.  Same arithmetic, rolled loops.
 // kDrop: the dropout mask element by element (any N).  kSR: q_out rounds stochastically, element by element (any N).
 template <bool kDrop = false, bool kSR = false>
 __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWarp& w, uint32_t taddr, uint32_t release,
@@ -897,7 +821,6 @@ __device__ __forceinline__ void epi_chunk_generic(const GemmDev& p, const EpiWar
             if (p.out_dtype == MV_F16 && (kSR || !w.mode_out) && !w.mode_res && p.epilogue != MV_EPI_GELU)
                 for (int j = 0; j < 4; j++) if (j < nvalid) raise_overflow(p.ovf, fabsf(v[j]));
             store_out4(p.out, p.out_dtype, m, p.ld_out, n, v, false, nvalid);
-            if (p.out2 != nullptr) store_out4(p.out2, p.out2_dtype, m, p.ld_out2, n, v, false, nvalid);
         }
         if (p.colsum != nullptr && !p.accumulate)
             for (int j = 0; j < 4; j++) if (j < nvalid) atomicAdd(p.colsum + n + j, cs[j]);
@@ -1268,7 +1191,7 @@ static int launch_gemm2(const CUtensorMap& ta, const CUtensorMap& tb, const Gemm
 
 using namespace mv;
 
-// CTA-pair path: 16-bit operands, 256 x BN cluster tiles
+// CTA-pair path: fp16 operands, 256 x BN cluster tiles
 static int gemm2_host(const mv_gemm_args* a, void* stream) {
     constexpr int BK = 64;
     // BN: least padding of N, ties to the wider tile; MN-major B is staged in 64-element chunks per CTA
@@ -1300,12 +1223,11 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     p.m_tiles = (a->M + 255) / 256;
     p.n_tiles = (a->N + BN - 1) / BN;
     p.kb_total = (a->K + BK - 1) / BK;
-    const int sms = persistent_sms();
     int splits = 1;
     if (a->accumulate) {
         // split K so that the work units fill whole rounds of the 74 clusters: the split count (at most two
         // rounds' worth) with the best units / (rounds * clusters); ties go to fewer splits (fewer red.adds)
-        const int tiles = p.m_tiles * p.n_tiles, clusters = sms / 2;
+        const int tiles = p.m_tiles * p.n_tiles, clusters = kNumSMs / 2;
         double best = -1.0;
         for (int sp = 1; sp <= p.kb_total && sp * tiles <= 2 * clusters; sp++) {
             const int units = sp * tiles;
@@ -1316,13 +1238,11 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     p.kb_per_split = (p.kb_total + splits - 1) / splits;
     p.splits = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
     p.a_major = a->a_major; p.b_major = a->b_major;
-    const int fmt = a->a_dtype == MV_BF16 ? 1 : 0;
-    p.idesc = make_idesc(fmt, fmt, a->a_major, a->b_major, 256, BN == 384 ? 256 : BN);
-    p.idesc2 = make_idesc(fmt, fmt, a->a_major, a->b_major, 256, 128);
+    p.idesc = make_idesc(0, 0, a->a_major, a->b_major, 256, BN == 384 ? 256 : BN);
+    p.idesc2 = make_idesc(0, 0, a->a_major, a->b_major, 256, 128);
     p.bias = a->bias; p.residual = a->residual; p.ld_res = a->ld_res;
     p.aux = reinterpret_cast<__half*>(a->aux); p.ld_aux = a->ld_aux;
     p.out = a->out; p.ld_out = a->ld_out; p.out_dtype = a->out_dtype;
-    p.out2 = a->out2; p.ld_out2 = a->ld_out2; p.out2_dtype = a->out2_dtype;
     p.epilogue = a->epilogue;
     p.q_out = FloatFmt{a->q_out_exp, a->q_out_man};
     p.q_res = FloatFmt{a->q_res_exp, a->q_res_man};
@@ -1332,8 +1252,8 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     p.colsum = a->accumulate ? nullptr : a->colsum;
     p.ovf = g_overflow;
     const bool drop = a->drop_seed != nullptr;
-    MV_CHECK(!drop || (!a->accumulate && a->colsum == nullptr && a->out2 == nullptr),
-             "mv_gemm: dropout needs a plain output (no accumulate, colsum or out2)");
+    MV_CHECK(!drop || (!a->accumulate && a->colsum == nullptr),
+             "mv_gemm: dropout needs a plain output (no accumulate or colsum)");
     MV_CHECK(!drop || a->epilogue != MV_EPI_DGELU, "mv_gemm: the gelu' epilogue takes its mask from aux, not from drop_seed");
     p.drop = DropDev{a->drop_seed, a->drop_thr, a->drop_scale, a->drop_site};
     const bool srnd = a->round_seed != nullptr;
@@ -1346,7 +1266,7 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
         const int qo = srnd ? 0 : qkind(a->q_out_exp, a->q_out_man), qr = qkind(a->q_res_exp, a->q_res_man);
         const int res = a->residual == nullptr ? 0 : (a->rows_per_img > 0 ? 2 : 1);
         const int cs = a->colsum != nullptr ? 1 : 0;
-        const bool ok = a->out2 == nullptr && (a->ld_out & 3) == 0 && (a->bias == nullptr || al(a->bias, 16)) &&
+        const bool ok = (a->ld_out & 3) == 0 && (a->bias == nullptr || al(a->bias, 16)) &&
                         (cs == 0 || al(a->colsum, 16)) &&
                         (res == 0 || ((a->ld_res & 3) == 0 && al(a->residual, 16))) &&
                         (a->aux == nullptr || ((a->ld_aux & 3) == 0 && al(a->aux, 8))) &&
@@ -1372,7 +1292,7 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     }
 
     const int units = p.m_tiles * p.n_tiles * p.splits;
-    const int grid = 2 * (units < sms / 2 ? units : sms / 2);
+    const int grid = 2 * (units < kNumSMs / 2 ? units : kNumSMs / 2);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     int rc;
     // 16 epilogue warps only where 12 would be unbalanced: BN = 256 is 8 chunks over 3 column groups (3 / 3 / 2)
@@ -1410,8 +1330,8 @@ static int gemm2_host(const mv_gemm_args* a, void* stream) {
     else if (aux_tma) rc = launch_gemm2<256, 16, 1>(ta, tb, p, grid, st, &taux);
     else if (res_tma) rc = launch_gemm2<192, 12, 2>(ta, tb, p, grid, st, &taux);
     else if (BN == 256) rc = heavy ? launch_gemm2<256, 16>(ta, tb, p, grid, st) : launch_gemm2<256, 12>(ta, tb, p, grid, st);
-    else if (BN == 192) rc = heavy ? launch_gemm2<192, 16>(ta, tb, p, grid, st) : launch_gemm2<192, 12>(ta, tb, p, grid, st);
-    else rc = heavy ? launch_gemm2<128, 16>(ta, tb, p, grid, st) : launch_gemm2<128, 12>(ta, tb, p, grid, st);
+    else if (BN == 192) rc = launch_gemm2<192, 12>(ta, tb, p, grid, st);
+    else rc = launch_gemm2<128, 12>(ta, tb, p, grid, st);
     if (rc) return rc;
     g_launches++;
     return check_cuda(cudaGetLastError(), "gemm2 launch");
@@ -1421,45 +1341,41 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     MV_CHECK(a != nullptr, "mv_gemm: null args");
     MV_CHECK(a->M > 0 && a->N > 0 && a->K > 0, "mv_gemm: bad shape %dx%dx%d", a->M, a->N, a->K);
     MV_CHECK(a->A && a->B && a->out, "mv_gemm: null operand");
+    MV_CHECK((a->a_dtype == MV_F16 || a->a_dtype == MV_F32) && a->b_dtype == a->a_dtype,
+             "mv_gemm: A and B must share one element type, MV_F16 or MV_F32 (got %d x %d)", a->a_dtype, a->b_dtype);
+    MV_CHECK(a->out_dtype == MV_F16 || a->out_dtype == MV_F32, "mv_gemm: output type %d is neither MV_F16 nor MV_F32", a->out_dtype);
     const bool tf32 = a->a_dtype == MV_F32;
-    MV_CHECK(a->a_dtype == a->b_dtype, "mv_gemm: A and B must share one element type (tcgen05 kind::f16 rejects f16 x bf16)");
     if (a->accumulate) MV_CHECK(a->out_dtype == MV_F32, "mv_gemm: accumulate needs an fp32 output");
-    MV_CHECK(a->cluster == 0 || a->cluster == 1, "mv_gemm: cluster %d (0: CTA-pair kernel, 1: single-CTA kernel)", a->cluster);
-    MV_CHECK(!a->transpose_out || (a->accumulate && !tf32 && a->cluster == 0),
-             "mv_gemm: transpose_out needs accumulate on the CTA-pair kernel (16-bit operands, cluster == 0)");
+    MV_CHECK(!a->transpose_out || (a->accumulate && !tf32),
+             "mv_gemm: transpose_out needs accumulate on the CTA-pair kernel (fp16 operands)");
     if (a->epilogue == MV_EPI_GELU || a->epilogue == MV_EPI_DGELU) MV_CHECK(a->aux != nullptr, "mv_gemm: GELU epilogues need aux");
     if (a->round_seed != nullptr) {
-        MV_CHECK(!tf32 && a->cluster == 0,
-                 "mv_gemm: stochastic rounding is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
+        MV_CHECK(!tf32, "mv_gemm: stochastic rounding is only fused into the CTA-pair kernel (fp16 operands)");
         MV_CHECK(a->q_out_exp >= 1 && a->q_out_exp <= 8 && a->q_out_man >= 1 && a->q_out_man <= 22,
                  "mv_gemm: q_out (%d, %d) is not a float format to round stochastically", a->q_out_exp, a->q_out_man);
-        MV_CHECK(!a->accumulate && a->out2 == nullptr && a->drop_seed == nullptr && a->residual == nullptr &&
-                 a->epilogue != MV_EPI_GELU,
-                 "mv_gemm: stochastic rounding needs a plain or gelu' output (no accumulate, out2, dropout, residual or GELU)");
+        MV_CHECK(!a->accumulate && a->drop_seed == nullptr && a->residual == nullptr && a->epilogue != MV_EPI_GELU,
+                 "mv_gemm: stochastic rounding needs a plain or gelu' output (no accumulate, dropout, residual or GELU)");
     }
-    if (!tf32 && a->cluster == 0) return gemm2_host(a, stream);      // CTA-pair kernel (default)
-    MV_CHECK(a->colsum == nullptr, "mv_gemm: colsum is only fused into the CTA-pair kernel (16-bit operands, cluster == 0)");
-    MV_CHECK(a->drop_seed == nullptr, "mv_gemm: dropout is only fused into the CTA-pair kernel (16-bit operands, cluster == 0); "
+    if (!tf32) return gemm2_host(a, stream);
+    // tf32: the single-CTA kernel
+    MV_CHECK(a->colsum == nullptr, "mv_gemm: colsum is only fused into the CTA-pair kernel (fp16 operands)");
+    MV_CHECK(a->drop_seed == nullptr, "mv_gemm: dropout is only fused into the CTA-pair kernel (fp16 operands); "
                                       "apply mv_dropout to the output instead");
-    const int esz = tf32 ? 4 : 2;
-    const int BK = 128 / esz;
+    constexpr int BK = 32;                     // tf32 elements per 128-byte row
+    constexpr int BN = kGemmBN;
     static bool attr_done = false;
     if (!attr_done) {
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<128, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<128>::kSmem));
-        MV_CUDA(cudaFuncSetAttribute(gemm_kernel<256, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<256>::kSmem));
+        MV_CUDA(cudaFuncSetAttribute(gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGemmSmem));
         attr_done = true;
     }
-    // 128x256 tiles cut the L2->SM operand traffic per flop by a quarter; use them when N tiles evenly
-    const int BN = (!tf32 && a->N % 256 == 0 && a->tile_n != 128) ? 256 : 128;
 
     CUtensorMap ta, tb;
     // K-major operand [rows = M|N, cols = K]: box = 128 rows x 128 B of K.
     // MN-major operand stored [K, M|N]: box = BK k-rows x 128 B of M|N.
-    if (a->a_major == 0) { if (make_tmap_2d(&ta, a->A, a->a_dtype, a->M, a->K, a->lda, BM, BK)) return 1; }
-    else                 { if (make_tmap_2d(&ta, a->A, a->a_dtype, a->K, a->M, a->lda, BK, 128 / esz)) return 1; }
-    if (a->b_major == 0) { if (make_tmap_2d(&tb, a->B, a->b_dtype, a->N, a->K, a->ldb, BN / 2, BK)) return 1; }
-    else                 { if (make_tmap_2d(&tb, a->B, a->b_dtype, a->K, a->N, a->ldb, BK, 128 / esz)) return 1; }
+    if (a->a_major == 0) { if (make_tmap_2d(&ta, a->A, MV_F32, a->M, a->K, a->lda, BM, BK)) return 1; }
+    else                 { if (make_tmap_2d(&ta, a->A, MV_F32, a->K, a->M, a->lda, BK, BK)) return 1; }
+    if (a->b_major == 0) { if (make_tmap_2d(&tb, a->B, MV_F32, a->N, a->K, a->ldb, BN / 2, BK)) return 1; }
+    else                 { if (make_tmap_2d(&tb, a->B, MV_F32, a->K, a->N, a->ldb, BK, BK)) return 1; }
 
     GemmDev p;
     p.trace = nullptr;
@@ -1477,13 +1393,10 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
     p.kb_per_split = (p.kb_total + splits - 1) / splits;
     p.splits = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
     p.a_major = a->a_major; p.b_major = a->b_major;
-    const int afmt = tf32 ? 2 : (a->a_dtype == MV_BF16 ? 1 : 0);
-    const int bfmt = tf32 ? 2 : (a->b_dtype == MV_BF16 ? 1 : 0);
-    p.idesc = make_idesc(afmt, bfmt, a->a_major, a->b_major, BM, BN);
+    p.idesc = make_idesc(2, 2, a->a_major, a->b_major, BM, BN);
     p.bias = a->bias; p.residual = a->residual; p.ld_res = a->ld_res;
     p.aux = reinterpret_cast<__half*>(a->aux); p.ld_aux = a->ld_aux;
     p.out = a->out; p.ld_out = a->ld_out; p.out_dtype = a->out_dtype;
-    p.out2 = a->out2; p.ld_out2 = a->ld_out2; p.out2_dtype = a->out2_dtype;
     p.epilogue = a->epilogue;
     p.q_out = FloatFmt{a->q_out_exp, a->q_out_man};
     p.q_res = FloatFmt{a->q_res_exp, a->q_res_man};
@@ -1495,11 +1408,7 @@ extern "C" int mv_gemm(const mv_gemm_args* a, void* stream) {
 
     const int units = p.m_tiles * p.n_tiles * p.splits;
     const int grid = units < kNumSMs ? units : kNumSMs;
-    const size_t smem = BN == 256 ? GemmCfg<256>::kSmem : GemmCfg<128>::kSmem;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (tf32) gemm_kernel<128, 4><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
-    else if (BN == 256) gemm_kernel<256, 2><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
-    else gemm_kernel<128, 2><<<grid, kGemmThreads, smem, st>>>(ta, tb, p);
+    gemm_kernel<<<grid, kGemmThreads, kGemmSmem, static_cast<cudaStream_t>(stream)>>>(ta, tb, p);
     g_launches++;
     return check_cuda(cudaGetLastError(), "gemm launch");
 }

@@ -470,25 +470,6 @@ __global__ void token_row_kernel(const float* __restrict__ tok, float* __restric
     x[(int64_t(b) * n_tokens + row) * D + d] = fq_nearest(tok[d], q_ff);
 }
 
-// fp32 -> bf16 / fp16 conversion (gradient operand copies)
-template <typename OutT>
-__global__ void __launch_bounds__(256)
-convert_kernel(const float* __restrict__ in, OutT* __restrict__ out, int64_t n4) {
-    const int64_t stride = int64_t(gridDim.x) * blockDim.x;
-    for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n4; i += stride) {
-        const float4 v = __ldcs(reinterpret_cast<const float4*>(in) + i);
-        uint2 u;
-        if (sizeof(OutT) == 2 && std::is_same<OutT, __nv_bfloat16>::value) {
-            __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
-            u = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
-        } else {
-            __half2 lo = __floats2half2_rn(sat16(v.x), sat16(v.y)), hi = __floats2half2_rn(sat16(v.z), sat16(v.w));
-            u = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
-        }
-        reinterpret_cast<uint2*>(out)[i] = u;
-    }
-}
-
 // out32 = in * s and / or out16 = fp16(in * s), s = *scale_dev or its reciprocal (a power of two: exact).
 // The loss-scale style gradient scale lives in device memory, so no host synchronisation.
 __global__ void __launch_bounds__(256)
@@ -557,7 +538,7 @@ static decltype(kKernel) ln_bwd_ready() {
 template <int NV>
 static int launch_ln_bwd(const mv_layernorm_bwd_args& a, cudaStream_t st) {
     int grid = (a.rows + kLnWarps - 1) / kLnWarps;
-    const int cap = persistent_sms() * 2;
+    const int cap = kNumSMs * 2;
     if (grid > cap) grid = cap;
     const size_t smem = size_t(kLnWarps) * 3 * a.D * sizeof(float);
     const FloatFmt q_in{a.q_in_exp, a.q_in_man}, q_grad{a.q_grad_exp, a.q_grad_man};
@@ -829,20 +810,6 @@ extern "C" int mv_token_row(const float* tok, float* x, int B, int n_tokens, int
     token_row_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(tok, x, B, n_tokens, D, row, q);
     g_launches++;
     return check_cuda(cudaGetLastError(), "token row launch");
-}
-
-extern "C" int mv_convert_f32(const float* in, void* out, int out_dtype, int64_t n, void* stream) {
-    MV_CHECK(n % 4 == 0, "mv_convert_f32: n must be a multiple of 4");
-    if (n == 0) return 0;
-    const int64_t n4 = n / 4;
-    int64_t blocks = (n4 + 255) / 256;
-    if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (out_dtype == MV_BF16) convert_kernel<__nv_bfloat16><<<int(blocks), 256, 0, st>>>(in, (__nv_bfloat16*)out, n4);
-    else if (out_dtype == MV_F16) convert_kernel<__half><<<int(blocks), 256, 0, st>>>(in, (__half*)out, n4);
-    else MV_CHECK(false, "mv_convert_f32: bad dtype");
-    g_launches++;
-    return check_cuda(cudaGetLastError(), "convert launch");
 }
 
 extern "C" int mv_scale_f32(const float* in, const float* scale_dev, int invert, float* out_f32, void* out_f16, int64_t n,

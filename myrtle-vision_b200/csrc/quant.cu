@@ -257,10 +257,9 @@ __global__ void quant_scalar_kernel(const float* __restrict__ in, OutT* __restri
     }
 }
 
-extern int g_opt_quant_ctas;
 static inline int grid_for(int64_t work_items, int per_block) {
     int64_t blocks = (work_items + per_block - 1) / per_block;
-    const int64_t cap = int64_t(kNumSMs) * g_opt_quant_ctas;   // resident CTAs of 256 threads per SM (8; option "quant_ctas")
+    const int64_t cap = int64_t(kNumSMs) * 8;   // resident CTAs of 256 threads per SM
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     return int(blocks);

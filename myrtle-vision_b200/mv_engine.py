@@ -151,11 +151,6 @@ class EncoderEngine:
         self.scaler_state = torch.tensor([0.0, 1024.0, 0.0], dtype=torch.float32, device=self.dev)
         self.reducer = None      # set by parallel.DataParallel: called with flat gradient slices
         self.bucket_blocks = max(1, int(os.environ.get("MV_DP_BUCKET_BLOCKS", "3")))   # encoder blocks per all-reduce
-        # The persistent kernels launched right behind a bucket's all-reduce are sized for the SMs NCCL leaves free
-        # (mv_set_option "sm_limit" / "sm_limit_launches", csrc/common.cuh persistent_sms): on a full-size grid their
-        # last CTAs wait for an SM and run as a second wave — the kernel takes twice as long.
-        self.dp_sm_limit = int(os.environ.get("MV_DP_SM_LIMIT", "148"))      # off: measured no gain at N = 2 and N = 8 (DESIGN §6)
-        self.dp_limit_launches = int(os.environ.get("MV_DP_LIMIT_LAUNCHES", "4"))
         # True once an optimizer (utils/fused_adamw.FusedAdamW) emits q(W) / q(W)^T itself after every
         # update: a CUDA-graph capture then leaves the re-quantisation out of the graph
         self.external_requant = False
@@ -512,9 +507,6 @@ class EncoderEngine:
                 top = min(cfg.depth, l + self.bucket_blocks)
                 lo, hi = self.offsets[b0], self.offsets[2 + PER_LAYER * top]
                 self.reducer.reduce_slice(self.gflat[lo:hi], 1.0 / S)
-                if self.reducer.world > 1 and self.dp_sm_limit < 148 and l > 0:
-                    mv.set_option("sm_limit", self.dp_sm_limit)
-                    mv.set_option("sm_limit_launches", self.dp_limit_launches)
         # ---- patch embedding: dW = dx^T patches (cls rows of `patches` are zero)
         mv.gemm(dx_h, saved["patches"], g[0], a_major=1, b_major=1, accumulate=True)
         wq_grad(0, 10 * cfg.depth)

@@ -13,11 +13,11 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _SO = os.path.join(_HERE, "csrc", os.environ.get("MV_ALT_LIB") or "libmv_b200.so")   # MV_ALT_LIB: an experiment build (tools/build_variant.sh)
 _lib = None
 
-F32, F16, BF16 = 0, 1, 2
+F32, F16 = 0, 1
 ROUND_NEAREST, ROUND_STOCHASTIC = 0, 1
 EPI_NONE, EPI_GELU, EPI_DGELU = 0, 1, 2
 
-_DT = {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16}
+_DT = {torch.float32: F32, torch.float16: F16}
 
 
 class MvError(RuntimeError):
@@ -33,7 +33,6 @@ class GemmArgs(ctypes.Structure):
         ("residual", ctypes.c_void_p), ("ld_res", ctypes.c_int),
         ("aux", ctypes.c_void_p), ("ld_aux", ctypes.c_int),
         ("out", ctypes.c_void_p), ("ld_out", ctypes.c_int), ("out_dtype", ctypes.c_int),
-        ("out2", ctypes.c_void_p), ("ld_out2", ctypes.c_int), ("out2_dtype", ctypes.c_int),
         ("epilogue", ctypes.c_int),
         ("q_out_exp", ctypes.c_int), ("q_out_man", ctypes.c_int),
         ("q_res_exp", ctypes.c_int), ("q_res_man", ctypes.c_int),
@@ -42,7 +41,6 @@ class GemmArgs(ctypes.Structure):
         ("tile_n", ctypes.c_int),
         ("colsum", ctypes.c_void_p),
         ("transpose_out", ctypes.c_int),
-        ("cluster", ctypes.c_int),
         ("drop_seed", ctypes.c_void_p), ("drop_thr", ctypes.c_uint32), ("drop_scale", ctypes.c_float),
         ("drop_site", ctypes.c_int),
         ("round_seed", ctypes.c_void_p), ("round_offset", ctypes.c_uint64),
@@ -95,11 +93,6 @@ def lib():
             fn = getattr(_lib, name)
             fn.argtypes, fn.restype = args, ctypes.c_int
     return _lib
-
-
-def set_option(name, value):
-    """Library-wide switch (mv_set_option in include/mv_b200.h), e.g. set_option("attn_sn", 0)."""
-    _check(lib().mv_set_option(name.encode(), int(value)), "mv_set_option")
 
 
 def _check(rc, what):
@@ -332,13 +325,13 @@ def quantize_weight(w, exp, man, out_dtype=torch.float16, transpose=True, out=No
 
 
 # ------------------------------------------------------------------------ GEMM
-def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None, out2=None,
+def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
          epilogue=EPI_NONE, q_out=None, q_res=None, accumulate=False, rows_per_img=0,
-         M=None, N=None, K=None, tag=None, tile_n=0, cluster=0, colsum=None, transpose_out=False, drop=None,
+         M=None, N=None, K=None, tag=None, tile_n=0, colsum=None, transpose_out=False, drop=None,
          grad_round=None):
     """out[M,N] = A . B^T over K with the fused epilogue of mv_gemm (include/mv_b200.h).
     a_major/b_major = 0: operand is [M|N, K] (K contiguous); 1: operand is [K, M|N].
-    cluster = 0: CTA-pair kernel (16-bit operands), 1: single-CTA kernel (always used for tf32).
+    fp16 operands run on the CTA-pair kernel, fp32 operands (tf32) on the single-CTA kernel.
     drop = (seed, p, site): dropout of the output after q_out (seed: int64 [1] CUDA tensor), None: off.
     grad_round = (seed, offset): q_out rounds stochastically, None: nearest."""
     _need_cuda(A, B, out)
@@ -351,8 +344,9 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
         N = B.shape[0] if b_major == 0 else B.shape[1]
     a = GemmArgs()
     a.M, a.N, a.K = M, N, K
-    a.A, a.lda, a.a_dtype, a.a_major = A.data_ptr(), A.stride(0), _DT[A.dtype], a_major
-    a.B, a.ldb, a.b_dtype, a.b_major = B.data_ptr(), B.stride(0), _DT[B.dtype], b_major
+    # an element type without a code (e.g. bf16) goes in as -1: mv_gemm rejects it with the reason, before any launch
+    a.A, a.lda, a.a_dtype, a.a_major = A.data_ptr(), A.stride(0), _DT.get(A.dtype, -1), a_major
+    a.B, a.ldb, a.b_dtype, a.b_major = B.data_ptr(), B.stride(0), _DT.get(B.dtype, -1), b_major
     a.bias = bias.data_ptr() if bias is not None else None
     if residual is not None:
         assert residual.dtype == torch.float32 and residual.stride(-1) == 1
@@ -360,9 +354,7 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
     if aux is not None:
         assert aux.dtype == torch.float16
         a.aux, a.ld_aux = aux.data_ptr(), aux.stride(-2)
-    a.out, a.ld_out, a.out_dtype = out.data_ptr(), out.stride(-2), _DT[out.dtype]
-    if out2 is not None:
-        a.out2, a.ld_out2, a.out2_dtype = out2.data_ptr(), out2.stride(-2), _DT[out2.dtype]
+    a.out, a.ld_out, a.out_dtype = out.data_ptr(), out.stride(-2), _DT.get(out.dtype, -1)
     a.epilogue = epilogue
     if q_out:
         a.q_out_exp, a.q_out_man = q_out
@@ -371,7 +363,6 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
     a.accumulate = int(bool(accumulate))
     a.rows_per_img = rows_per_img
     a.tile_n = tile_n
-    a.cluster = cluster
     a.transpose_out = int(bool(transpose_out))
     if colsum is not None:
         assert colsum.dtype == torch.float32 and colsum.is_contiguous() and colsum.numel() == N
@@ -395,8 +386,6 @@ def gemm(A, B, out, *, a_major=0, b_major=0, bias=None, residual=None, aux=None,
             nbytes += (rows_per_img if rows_per_img else M) * N * 4
         if aux is not None:
             nbytes += M * N * 2
-        if out2 is not None:
-            nbytes += M * N * out2.element_size()
     with _timed(kind, flop, nbytes):
         _check(lib().mv_gemm(ctypes.byref(a), _stream()), "mv_gemm")
     return out
@@ -524,16 +513,6 @@ def distill_loss(student, distill, teacher, labels, temperature, alpha, hard):
     return loss, ds, dd
 
 
-def convert_f32(x, out_dtype=torch.float16, out=None):
-    _need_cuda(x)
-    x = x.contiguous()
-    if out is None:
-        out = torch.empty(x.shape, dtype=out_dtype, device=x.device)
-    _check(lib().mv_convert_f32(_ptr(x), _ptr(out), _DT[out.dtype], ctypes.c_int64(x.numel()),
-                                _stream()), "mv_convert_f32")
-    return out
-
-
 def scale_f32(x, scale, *, invert=False, out=None, out_h=None, want_f32=True, want_f16=False):
     """(x * scale [or / scale]) as fp32 and / or saturating fp16, `scale` a 0-dim / 1-element device tensor."""
     _need_cuda(x, scale)
@@ -634,7 +613,7 @@ def attention_fwd(qkv, B, H, N, *, scale=0.125, q_out=None, out_dtype=torch.floa
 
 
 def attention_bwd(qkv, o, d_o, lse, B, H, N, *, scale=0.125, dqkv=None, delta=None,
-                  deterministic=False, dq_accum=None, dbias=None):
+                  dq_accum=None, dbias=None):
     """d_o fp16 [B*N, D] -> dqkv fp16 [B*N, 3D] (dq | dk | dv).  dbias fp32 [3D] (optional) += column sums
     of dqkv, the to_qkv bias gradient."""
     _need_cuda(qkv, o, d_o, lse)
@@ -646,11 +625,11 @@ def attention_bwd(qkv, o, d_o, lse, B, H, N, *, scale=0.125, dqkv=None, delta=No
         delta = torch.empty(B, H, N, dtype=torch.float32, device=qkv.device)
     if dbias is not None:
         assert dbias.dtype == torch.float32 and dbias.is_contiguous() and dbias.numel() == 3 * H * 64
-    if not deterministic and dq_accum is None:
+    if dq_accum is None:
         dq_accum = torch.empty(B * N, H * 64, dtype=torch.float32, device=qkv.device)
     with _timed("attn_bwd", 10.0 * B * H * N * N * 64, B * N * H * 64 * 2 * (3 + 1 + 1 + 3)):
         rc = lib().mv_attention_bwd(_ptr(qkv), _ptr(o), _ptr(d_o), _ptr(lse), _ptr(delta),
-                                    None if deterministic else _ptr(dq_accum), _ptr(dqkv), _ptr(dbias), B,
+                                    _ptr(dq_accum), _ptr(dqkv), _ptr(dbias), B,
                                     H, N, ctypes.c_float(scale), _stream())
     _check(rc, "mv_attention_bwd")
     return dqkv

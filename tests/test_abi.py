@@ -62,6 +62,24 @@ def test_error_reporting_without_a_gpu(lib):
     assert lib.mv_version() >= 100
 
 
+@pytest.mark.parametrize("field", ["a_dtype", "out_dtype"])
+def test_gemm_rejects_other_element_types_without_a_gpu(lib, field):
+    """mv_gemm takes MV_F16 / MV_F32 operands and outputs only; type 2 (bf16, which no kernel reads or writes) is
+    rejected before anything touches a device.  The pointers are never dereferenced."""
+    import mv_native
+    lib.mv_last_error.restype = ctypes.c_char_p
+    a = mv_native.GemmArgs()
+    a.M = a.N = a.K = a.lda = a.ldb = a.ld_out = 128
+    a.A = a.B = a.out = 1 << 20
+    a.a_dtype = a.b_dtype = a.out_dtype = mv_native.F16
+    if field == "a_dtype":
+        a.a_dtype = a.b_dtype = 2
+    else:
+        a.out_dtype = 2
+    assert lib.mv_gemm(ctypes.byref(a), None) != 0
+    assert b"MV_F16" in lib.mv_last_error()
+
+
 def test_missing_library_fails_loudly(monkeypatch):
     import mv_native
     monkeypatch.setattr(mv_native, "_lib", None)

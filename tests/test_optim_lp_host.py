@@ -33,7 +33,7 @@ def test_header_declares_the_entry_point_and_version():
     assert re.search(r"int mv_adamw_lp_step\(const mv_adamw_tensor\* tensors_dev, const mv_adamw_lp_tensor\* lp_dev,",
                      text)
     api = open(os.path.join(ROOT, "myrtle-vision_b200", "csrc", "api.cu")).read()
-    assert "return 104;" in api
+    assert "return 105;" in api
 
 
 def test_import_and_qtorch_signature():

@@ -6,9 +6,9 @@ python tools/probe_formats.py > $O/probe_formats.log 2>&1; echo "formats rc=$?"
 ncu --metrics gpu__time_duration.sum --clock-control none -c 1500 --csv --log-file $O/r1c_launches.csv \
     python bench.py --steps 2 --warmup 3 --no-cpu-baseline --no-graph --no-kernel-timing > $O/r1c_ncu_list.log 2>&1; echo "launch list rc=$?"
 NCU="ncu --set full --clock-control none --import-source on -f"
-$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_fc1_gelu python tools/prof_gemm_one.py 1536 384 gelu 0 > $O/r1c_p1.log 2>&1; echo "p1 rc=$?"
-$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_fc2_res python tools/prof_gemm_one.py 384 1536 res 0 > $O/r1c_p2.log 2>&1; echo "p2 rc=$?"
-$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_wgrad python tools/prof_gemm_one.py 1536 384 wgrad 0 > $O/r1c_p3.log 2>&1; echo "p3 rc=$?"
+$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_fc1_gelu python tools/prof_gemm_one.py 1536 384 gelu > $O/r1c_p1.log 2>&1; echo "p1 rc=$?"
+$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_fc2_res python tools/prof_gemm_one.py 384 1536 res > $O/r1c_p2.log 2>&1; echo "p2 rc=$?"
+$NCU -k regex:gemm2 -s 3 -c 1 -o $O/r1c_gemm_wgrad python tools/prof_gemm_one.py 1536 384 wgrad > $O/r1c_p3.log 2>&1; echo "p3 rc=$?"
 $NCU -k regex:attn_fwd_sn -s 2 -c 1 -o $O/r1c_attn_fwd_sn python tools/prof_attn_one.py > $O/r1c_p4.log 2>&1; echo "p4 rc=$?"
 $NCU -k regex:attn_bwd_sn -s 2 -c 1 -o $O/r1c_attn_bwd_sn python tools/prof_attn_one.py bwd > $O/r1c_p5.log 2>&1; echo "p5 rc=$?"
 $NCU -k regex:ln_fwd -s 2 -c 1 -o $O/r1c_ln_fwd python tools/prof_elementwise_one.py ln_fwd > $O/r1c_p6.log 2>&1; echo "p6 rc=$?"

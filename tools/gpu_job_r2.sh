@@ -9,8 +9,8 @@ $L > $O/r2_plain_list.log 2>&1 && ncu --metrics gpu__time_duration.sum --clock-c
 NCU="ncu --set full --clock-control none --import-source on -f"
 python tools/prof_attn_one.py bwd > $O/r2_p1.log 2>&1 && $NCU -k regex:attn_bwd_sn -s 2 -c 1 -o $O/r2_attn_bwd_sn python tools/prof_attn_one.py bwd > $O/r2_p1n.log 2>&1; echo "attn bwd rc=$?"
 $NCU -k regex:attn_fwd_sn -s 2 -c 1 -o $O/r2_attn_fwd_sn python tools/prof_attn_one.py bwd > $O/r2_p2n.log 2>&1; echo "attn fwd rc=$?"
-python tools/prof_gemm_one.py 1536 384 dgelu 0 > $O/r2_p3.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_dgelu python tools/prof_gemm_one.py 1536 384 dgelu 0 > $O/r2_p3n.log 2>&1; echo "dgelu rc=$?"
-python tools/prof_gemm_one.py 384 384 res 0 > $O/r2_p4.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_proj_res python tools/prof_gemm_one.py 384 384 res 0 > $O/r2_p4n.log 2>&1; echo "proj res rc=$?"
-python tools/prof_gemm_one.py 1536 384 gelu 0 > $O/r2_p5.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_gelu python tools/prof_gemm_one.py 1536 384 gelu 0 > $O/r2_p5n.log 2>&1; echo "gelu rc=$?"
+python tools/prof_gemm_one.py 1536 384 dgelu > $O/r2_p3.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_dgelu python tools/prof_gemm_one.py 1536 384 dgelu > $O/r2_p3n.log 2>&1; echo "dgelu rc=$?"
+python tools/prof_gemm_one.py 384 384 res > $O/r2_p4.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_proj_res python tools/prof_gemm_one.py 384 384 res > $O/r2_p4n.log 2>&1; echo "proj res rc=$?"
+python tools/prof_gemm_one.py 1536 384 gelu > $O/r2_p5.log 2>&1 && $NCU -k regex:gemm2 -s 3 -c 1 -o $O/r2_gemm_gelu python tools/prof_gemm_one.py 1536 384 gelu > $O/r2_p5n.log 2>&1; echo "gelu rc=$?"
 python tools/prof_segloss_one.py > $O/r2_p6.log 2>&1 && $NCU -k regex:upsample_ce -s 2 -c 1 -o $O/r2_segloss python tools/prof_segloss_one.py > $O/r2_p6n.log 2>&1; echo "segloss rc=$?"
 python tools/prof_elementwise_one.py quant > $O/r2_p7.log 2>&1 && $NCU -k regex:quant_vec16 -s 1 -c 1 -o $O/r2_quant python tools/prof_elementwise_one.py quant > $O/r2_p7n.log 2>&1; echo "quant rc=$?"

@@ -1,5 +1,5 @@
 """Long-sequence attention timing (detection config: B=8, H=6, N=2501): forward, backward with fused dQ
-red.add, deterministic two-pass backward."""
+red.add."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "myrtle-vision_b200")); sys.path.insert(0, ROOT)
@@ -21,6 +21,5 @@ def timeit(fn, n=10):
 fl = 4.0 * B * H * N * N * 64
 ms = timeit(lambda: mv.attention_fwd(qkv, B, H, N, q_out=(5, 10)))
 print("fwd %.3f ms  %.0f TFLOP/s" % (ms, fl / ms / 1e9))
-for det in (False, True):
-    ms = timeit(lambda: mv.attention_bwd(qkv, out, do, lse, B, H, N, deterministic=det))
-    print("bwd deterministic=%s %.3f ms  %.0f TFLOP/s (2.5x fwd flops)" % (det, ms, 2.5 * fl / ms / 1e9))
+ms = timeit(lambda: mv.attention_bwd(qkv, out, do, lse, B, H, N))
+print("bwd %.3f ms  %.0f TFLOP/s (2.5x fwd flops)" % (ms, 2.5 * fl / ms / 1e9))
