@@ -363,6 +363,59 @@ int mv_distill_loss(const float* student, const float* distill, const float* tea
                     int C, float T, float alpha, int hard, float* loss, float* row_loss, float* d_student,
                     float* d_distill, void* stream);
 
+/* ---------------------------------------------------------------- Mixup / CutMix (DESIGN.md section 7)
+ * timm 0.5.4's Mixup / mixup_target / SoftTargetCrossEntropy, with the randomness drawn on the device.  Image b is
+ * mixed with its partner B - 1 - b (B even).  One "unit" is the whole batch (MV_MIX_BATCH), the pair {i, B - 1 - i}
+ * (MV_MIX_PAIR, unit i < B / 2) or one image (MV_MIX_ELEM, unit b).  Per unit: with probability prob the unit is mixed
+ * (else lam = 1, untouched); CutMix with probability switch_prob when both alphas are > 0, else the kind whose alpha is
+ * > 0; lam ~ Beta(alpha, alpha) of that kind.
+ *   Mixup:  pixel = fl32(fl32(w_self * a) + fl32(w_other * p)), w_self = fp32(lam), w_other = fp32(1 - lam) (fp64
+ *           difference); a the image's pixel, p the partner's.
+ *   CutMix: r = sqrt(1 - lam), cut_h = int(H r), cut_w = int(W r), cy ~ U{0..H-1}, cx ~ U{0..W-1},
+ *           y0 = clip(cy - cut_h / 2, 0, H), y1 = clip(cy + cut_h / 2, 0, H) (x alike); pixels in [y0, y1) x [x0, x1)
+ *           come from the partner and lam becomes 1 - (y1 - y0)(x1 - x0) / (H W).
+ * "Mix stream": every draw of a unit is a Philox4x32-10 block with key = the 64-bit seed (device memory, drawn per
+ * training forward from torch's generator) and counter = {unit, draw index, rank, MV_MIX_TAG}:
+ *   draw 0:                  word 0: the mix test, 1: the CutMix switch, 2: cy, 3: cx (u = (word + 0.5) 2^-32)
+ *   draw 1 + 17 g:           word 0: U of the alpha < 1 boost Gamma(alpha + 1) U^(1 / alpha) of Gamma draw g
+ *   draw 2 + 17 g + k:       attempt k < 16 of Marsaglia-Tsang (fp64) for Gamma draw g: words 0, 1 a Box-Muller normal,
+ *                            word 2 the acceptance test.  After 16 rejections the draw returns d = alpha' - 1/3
+ *                            (times the boost); the probability of that is below 1e-20 for every alpha.
+ *   lam = X / (X + Y) with X the Gamma draw g = 0, Y g = 1 (lam = 1/2 if both are 0).
+ * rank (data-parallel rank) separates ranks that share the seed.  A pure function of (seed, rank, B, H, W, spec). */
+#define MV_MIX_BATCH 0
+#define MV_MIX_PAIR 1
+#define MV_MIX_ELEM 2
+#define MV_MIX_TAG 0x4d495855u
+typedef struct {
+    float mixup_alpha, cutmix_alpha;   /* >= 0, not both 0 */
+    float prob, switch_prob;           /* in [0, 1] */
+    int mode;                          /* MV_MIX_* */
+} mv_mix_spec;
+/* one per image */
+typedef struct {
+    float lam;                         /* target weight of the image's own label (after the CutMix correction) */
+    float w_self, w_other;             /* the Mixup multipliers (1, 0 for CutMix and unmixed images) */
+    int cutmix;                        /* 1: the box comes from the partner */
+    int y0, y1, x0, x1;                /* the box (empty unless cutmix) */
+} mv_mix_rec;
+/* recs_dev: B records.  One launch. */
+int mv_mix_draw(const int64_t* seed_dev, int rank, int B, int H, int W, mv_mix_spec spec, mv_mix_rec* recs_dev,
+                void* stream);
+/* mv_patchify_q of the mixed batch (the records applied to img before q_in), without materialising it.  A Mixup image
+ * also reads its partner's rows, a CutMix image the partner's 16-byte vectors that overlap the box, an unmixed one
+ * nothing more. */
+int mv_patchify_mix_q(const float* img, const mv_mix_rec* recs_dev, void* out, int out_dtype, int B, int C, int H,
+                      int W, int P, int q_exp, int q_man, int cls_slot, void* stream);
+/* Soft-target cross-entropy over fp32 logits x [B, C] (row pitch C), int64 labels y [B]:
+ *   t_b = lam_b s(y_b) + (1 - lam_b) s(y_{B-1-b}),  s(y) = off + (on - off) e_y,  off = smoothing / C,
+ *   on = 1 - smoothing + off;   loss = mean_b sum_c -t_bc log_softmax(x_b)_c,   dlogits = (softmax(x) - t) / B.
+ * recs_dev == NULL: lam = 1 (F.cross_entropy(x, y, label_smoothing=smoothing)).  row_loss: fp32 [B] scratch.  A label
+ * outside [0, C) that carries weight (lam_b > 0 for y_b, lam_b < 1 for the partner's) makes the row's loss and
+ * gradients NaN.  C >= 2, 0 <= smoothing <= 1, B even when recs_dev != NULL.  Fixed-order batch sum; two launches. */
+int mv_mix_ce_loss(const float* logits, const int64_t* labels, const mv_mix_rec* recs_dev, int B, int C,
+                   float smoothing, float* loss, float* row_loss, float* dlogits, void* stream);
+
 /* ---------------------------------------------------------------- detection matching (SURVEY.md §8f.4)
  * scipy.optimize.linear_sum_assignment of the reference's HungarianMatcher (models/matcher.py:83-86) for a
  * whole batch in one launch, one warp per image.  cost: fp32 [B, Q, Tmax], image b uses columns

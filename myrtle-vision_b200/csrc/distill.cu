@@ -145,6 +145,13 @@ distill_loss_sum_kernel(const float* __restrict__ row_loss, int B, float* __rest
     if (threadIdx.x == 0) loss[0] = v[0] / float(B);
 }
 
+// loss[0] = mean of row_loss[0, B) with distill_loss_sum_kernel (also the batch sum of mixup.cu's loss)
+int row_mean_launch(const float* row_loss, int B, float* loss, cudaStream_t st) {
+    distill_loss_sum_kernel<<<1, kDlThreads, 0, st>>>(row_loss, B, loss);
+    g_launches++;
+    return check_cuda(cudaGetLastError(), "row mean launch");
+}
+
 }  // namespace mv
 
 using namespace mv;

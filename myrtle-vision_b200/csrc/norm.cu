@@ -394,10 +394,11 @@ colsum_kernel(const T* __restrict__ in, int64_t ld, int rows, int cols, float* _
 
 // patchify + input quant:  img NCHW fp32 -> patches [B*gh*gw, p*p*C] with (ph, pw, c) minor
 // order (src/myrtle_vision/models/vit.py:271-275), each value through q_in, fp16/fp32 container.
-template <typename OutT>
+// kMix: image b is first mixed with image B - 1 - b as recs[b] says (mv_patchify_mix_q); recs is unused otherwise.
+template <typename OutT, bool kMix>
 __global__ void __launch_bounds__(256)
 patchify_kernel(const float* __restrict__ img, OutT* __restrict__ out, int B, int C, int H, int W,
-                int P, FloatFmt q_in, int cls_slot) {
+                int P, FloatFmt q_in, int cls_slot, const mv_mix_rec* __restrict__ recs) {
     // One CTA per (b, patch row gy).  Phase 1 reads the C x P image rows (W contiguous floats each,
     // 16-byte loads), quantises and scatters them into shared memory at their OUTPUT position
     // [gx][ph][pw][c] (the index arithmetic is per 16-byte load, not per element); phase 2 copies the
@@ -420,10 +421,36 @@ patchify_kernel(const float* __restrict__ img, OutT* __restrict__ out, int B, in
     }
     const int mode = fq_mode(q_in);
     const int w4 = W >> 2;              // W % 4 == 0 checked on the host
+    [[maybe_unused]] mv_mix_rec rec;
+    if constexpr (kMix) {               // the record, read once per CTA
+        __shared__ mv_mix_rec sm_rec;
+        if (threadIdx.x == 0) sm_rec = recs[b];
+        __syncthreads();
+        rec = sm_rec;
+    }
     for (int i = threadIdx.x; i < C * P * w4; i += blockDim.x) {
         const int wv = i % w4, r = i / w4;                 // r = c * P + ph
         const int c = r / P, ph = r % P;
         float4 v = __ldcs(reinterpret_cast<const float4*>(img + ((int64_t(b) * C + c) * H + gy * P + ph) * W) + wv);
+        if constexpr (kMix) {
+            const int y = gy * P + ph, x = wv * 4;
+            const float4* prow = reinterpret_cast<const float4*>(img + ((int64_t(B - 1 - b) * C + c) * H + y) * W) + wv;
+            if (rec.cutmix) {                              // only the vectors that overlap the box read the partner
+                if (y >= rec.y0 && y < rec.y1 && x + 4 > rec.x0 && x < rec.x1) {
+                    const float4 p = __ldcs(prow);
+                    if (x >= rec.x0 && x < rec.x1) v.x = p.x;
+                    if (x + 1 >= rec.x0 && x + 1 < rec.x1) v.y = p.y;
+                    if (x + 2 >= rec.x0 && x + 2 < rec.x1) v.z = p.z;
+                    if (x + 3 >= rec.x0 && x + 3 < rec.x1) v.w = p.w;
+                }
+            } else if (rec.w_other != 0.f || rec.w_self != 1.f) {   // Mixup: two rounded products, one rounded add
+                const float4 p = __ldcs(prow);
+                v.x = __fadd_rn(__fmul_rn(rec.w_self, v.x), __fmul_rn(rec.w_other, p.x));
+                v.y = __fadd_rn(__fmul_rn(rec.w_self, v.y), __fmul_rn(rec.w_other, p.y));
+                v.z = __fadd_rn(__fmul_rn(rec.w_self, v.z), __fmul_rn(rec.w_other, p.z));
+                v.w = __fadd_rn(__fmul_rn(rec.w_self, v.w), __fmul_rn(rec.w_other, p.w));
+            }
+        }
         if (mode == 1) v = fq_half4_f32(v);
         else { v.x = fq_apply(v.x, mode, q_in); v.y = fq_apply(v.y, mode, q_in); v.z = fq_apply(v.z, mode, q_in); v.w = fq_apply(v.w, mode, q_in); }
         const int w = wv * 4;
@@ -772,25 +799,40 @@ extern "C" int mv_colsum(const void* in, int in_dtype, int64_t ld, int rows, int
     return check_cuda(cudaGetLastError(), "colsum launch");
 }
 
-extern "C" int mv_patchify_q(const float* img, void* out, int out_dtype, int B, int C, int H, int W, int P,
-                             int q_exp, int q_man, int cls_slot, void* stream) {
-    MV_CHECK(B > 0 && C > 0 && P > 0 && H % P == 0 && W % P == 0, "mv_patchify_q: image dims must be divisible by the patch size");
-    MV_CHECK(cls_slot >= 0 && cls_slot <= 2, "mv_patchify_q: cls_slot must be 0, 1 or 2");
+template <bool kMix>
+static int patchify_launch(const char* fn, const float* img, const mv_mix_rec* recs, void* out, int out_dtype, int B,
+                           int C, int H, int W, int P, int q_exp, int q_man, int cls_slot, void* stream) {
+    MV_CHECK(B > 0 && C > 0 && P > 0 && H % P == 0 && W % P == 0, "%s: image dims must be divisible by the patch size", fn);
+    MV_CHECK(cls_slot >= 0 && cls_slot <= 2, "%s: cls_slot must be 0, 1 or 2", fn);
     const FloatFmt q{q_exp, q_man};
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    MV_CHECK(W % 4 == 0 && (reinterpret_cast<uintptr_t>(img) & 15) == 0, "mv_patchify_q: image rows must be 16-byte aligned (W % 4 == 0)");
+    MV_CHECK(W % 4 == 0 && (reinterpret_cast<uintptr_t>(img) & 15) == 0, "%s: image rows must be 16-byte aligned (W %% 4 == 0)", fn);
     const int grid = B * (H / P);
     const size_t smem = size_t(C) * P * W * (out_dtype == MV_F16 ? 2 : 4);
-    MV_CHECK(smem <= 200 * 1024, "mv_patchify_q: C * P * W too large for the shared-memory staging buffer");
+    MV_CHECK(smem <= 200 * 1024, "%s: C * P * W too large for the shared-memory staging buffer", fn);
     if (out_dtype == MV_F16) {
-        MV_CUDA(cudaFuncSetAttribute(patchify_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        patchify_kernel<__half><<<grid, 256, smem, st>>>(img, (__half*)out, B, C, H, W, P, q, cls_slot);
+        MV_CUDA(cudaFuncSetAttribute(patchify_kernel<__half, kMix>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+        patchify_kernel<__half, kMix><<<grid, 256, smem, st>>>(img, (__half*)out, B, C, H, W, P, q, cls_slot, recs);
     } else if (out_dtype == MV_F32) {
-        MV_CUDA(cudaFuncSetAttribute(patchify_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-        patchify_kernel<float><<<grid, 256, smem, st>>>(img, (float*)out, B, C, H, W, P, q, cls_slot);
-    } else MV_CHECK(false, "mv_patchify_q: bad container");
+        MV_CUDA(cudaFuncSetAttribute(patchify_kernel<float, kMix>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+        patchify_kernel<float, kMix><<<grid, 256, smem, st>>>(img, (float*)out, B, C, H, W, P, q, cls_slot, recs);
+    } else MV_CHECK(false, "%s: bad container", fn);
     g_launches++;
     return check_cuda(cudaGetLastError(), "patchify launch");
+}
+
+extern "C" int mv_patchify_q(const float* img, void* out, int out_dtype, int B, int C, int H, int W, int P,
+                             int q_exp, int q_man, int cls_slot, void* stream) {
+    return patchify_launch<false>("mv_patchify_q", img, nullptr, out, out_dtype, B, C, H, W, P, q_exp, q_man, cls_slot,
+                                  stream);
+}
+
+extern "C" int mv_patchify_mix_q(const float* img, const mv_mix_rec* recs_dev, void* out, int out_dtype, int B, int C,
+                                 int H, int W, int P, int q_exp, int q_man, int cls_slot, void* stream) {
+    MV_CHECK(recs_dev != nullptr, "mv_patchify_mix_q: null records");
+    MV_CHECK(B > 0 && B % 2 == 0, "mv_patchify_mix_q: the batch must be even (got B=%d)", B);
+    return patchify_launch<true>("mv_patchify_mix_q", img, recs_dev, out, out_dtype, B, C, H, W, P, q_exp, q_man,
+                                 cls_slot, stream);
 }
 
 extern "C" int mv_cls_rows(const float* cls, const float* pos_q, float* x, int B, int n_tokens, int D,

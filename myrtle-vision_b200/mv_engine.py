@@ -317,9 +317,11 @@ class EncoderEngine:
         self.last_grad_round_seed = seed
         return seed
 
-    def forward(self, img, pos_full, cls_token, save, token=None):
+    def forward(self, img, pos_full, cls_token, save, token=None, mix=None):
         """token (optional, [1, 1, D]): a distillation token appended as the last row N - 1 of every image, with no
-        positional embedding (DESIGN.md section 7); pos_full then still holds the N - 1 rows of cls + grid."""
+        positional embedding (DESIGN.md section 7); pos_full then still holds the N - 1 rows of cls + grid.
+        mix (optional): Mixup / CutMix records (mv_native.mix_draw): the encoder sees the mixed batch, mixed inside the
+        patch gather; the saved patches are the mixed ones, so the backward needs nothing else."""
         # A training forward clears self.overflow and its backward closes the window (mv_overflow_update); inference
         # forwards report nothing.  The library keeps one process-wide flag pointer, so it is registered only while
         # this engine's own kernels run and cleared on the way out, exception or not: launches outside the step (other
@@ -332,8 +334,8 @@ class EncoderEngine:
             drops = self._draw_drops()
             self.step_grad_round_seed = self._draw_grad_round(save)
             if self.wide:
-                return self._forward_wide(img, pos_full, cls_token, save, drops, token)
-            x, saved = self._forward_16(img, pos_full, cls_token, save, drops, token)
+                return self._forward_wide(img, pos_full, cls_token, save, drops, token, mix)
+            x, saved = self._forward_16(img, pos_full, cls_token, save, drops, token, mix)
             if saved is not None:
                 saved["grad_round"] = self.step_grad_round_seed
             return x, saved
@@ -352,7 +354,12 @@ class EncoderEngine:
         if token is not None:
             mv.token_row(token.detach().reshape(D).contiguous(), x, B, N, D, N - 1, q_ff=self.cfg.plan.ff)
 
-    def _forward_16(self, img, pos_full, cls_token, save, drops, token=None):
+    def _patchify(self, img, mix, P, out_dtype, slots):
+        if mix is None:
+            return mv.patchify_q(img, P, q_in=self.fmt, out_dtype=out_dtype, cls_slot=slots)
+        return mv.patchify_mix_q(img, mix, P, q_in=self.fmt, out_dtype=out_dtype, cls_slot=slots)
+
+    def _forward_16(self, img, pos_full, cls_token, save, drops, token=None, mix=None):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
@@ -365,7 +372,7 @@ class EncoderEngine:
 
         with self._range("patch_to_embedding"):
             pos32, slots = self._embed_inputs(pos_full, token, N, D)
-            patches = mv.patchify_q(img, P, q_in=fmt, cls_slot=slots)           # [M, P*P*C], zero token rows
+            patches = self._patchify(img, mix, P, f16, slots)                    # [M, P*P*C], zero token rows
             x = torch.empty(M, D, dtype=torch.float32, device=dev)
             mv.gemm(patches, wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                     rows_per_img=N)
@@ -556,7 +563,7 @@ class EncoderEngine:
     # wgrad therefore takes explicit transposes (mv_widen_transpose) instead of the in-place MN-major
     # reads of the 16-bit path.  Attention keeps the fp16 tcgen05 kernels: qkv / attention output /
     # their gradients carry 11 significant bits, the same as a tf32 operand.
-    def _forward_wide(self, img, pos_full, cls_token, save, drops, token=None):
+    def _forward_wide(self, img, pos_full, cls_token, save, drops, token=None, mix=None):
         cfg, plan, fmt = self.cfg, self.cfg.plan, self.fmt
         B, C, Hh, Ww = img.shape
         P = cfg.patch
@@ -570,7 +577,7 @@ class EncoderEngine:
         A_ = (lambda t: mv.split_tf32(t, 0)) if ex else (lambda t: t)        # A operand of a Linear
 
         pos32, slots = self._embed_inputs(pos_full, token, N, D)
-        patches = mv.patchify_q(img, P, q_in=fmt, out_dtype=f32, cls_slot=slots)
+        patches = self._patchify(img, mix, P, f32, slots)
         x = torch.empty(M, D, dtype=f32, device=dev)
         mv.gemm(A_(patches), wq[0][0], x, bias=prm[1], q_out=plan.out, residual=pos32, q_res=plan.ff,
                 rows_per_img=N)
@@ -750,19 +757,19 @@ class EncoderEngine:
 
 class EncoderFunction(torch.autograd.Function):
     @classmethod
-    def apply(cls, engine, img, pos_full, cls_token, *params, token=None):
-        """token: optional distillation token [1, 1, D] (EncoderEngine.forward)."""
+    def apply(cls, engine, img, pos_full, cls_token, *params, token=None, mix=None):
+        """token: optional distillation token [1, 1, D]; mix: optional Mixup / CutMix records (EncoderEngine.forward)."""
         # ctx.needs_input_grad follows requires_grad even under torch.no_grad(), and forward() itself always runs with
         # grad mode off, so grad mode is read here: without it the forward saves nothing and reports into no flag
         if not torch.is_grad_enabled():
-            return engine.forward(img, pos_full, cls_token, save=False, token=token)[0]
-        return super().apply(engine, img, pos_full, cls_token, token, *params)
+            return engine.forward(img, pos_full, cls_token, save=False, token=token, mix=mix)[0]
+        return super().apply(engine, img, pos_full, cls_token, token, mix, *params)
 
     @staticmethod
-    def forward(ctx, engine, img, pos_full, cls_token, token, *params):
+    def forward(ctx, engine, img, pos_full, cls_token, token, mix, *params):
         need = any(ctx.needs_input_grad)      # False when no input requires a gradient
         with torch.no_grad():
-            x, saved = engine.forward(img, pos_full, cls_token, save=need, token=token)
+            x, saved = engine.forward(img, pos_full, cls_token, save=need, token=token, mix=mix)
         ctx.engine, ctx.saved = engine, saved
         return x
 
@@ -776,4 +783,4 @@ class EncoderFunction(torch.autograd.Function):
         with torch.no_grad():
             dpos, dcls, dtok, g = engine.backward(saved, gx.contiguous())
         ctx.saved = None
-        return (None, None, dpos, dcls, dtok) + tuple(g)
+        return (None, None, dpos, dcls, dtok, None) + tuple(g)

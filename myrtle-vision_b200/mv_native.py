@@ -65,12 +65,30 @@ class LayerNormBwdArgs(ctypes.Structure):
     ]
 
 
-# ctypes signatures of entry points declared with full argument types (tests/test_distill_host.py holds them to the
-# header's prototypes)
+MIX_MODES = {"batch": 0, "pair": 1, "elem": 2}       # MV_MIX_BATCH / MV_MIX_PAIR / MV_MIX_ELEM
+
+
+class MixSpec(ctypes.Structure):
+    _fields_ = [("mixup_alpha", ctypes.c_float), ("cutmix_alpha", ctypes.c_float), ("prob", ctypes.c_float),
+                ("switch_prob", ctypes.c_float), ("mode", ctypes.c_int)]
+
+
+class MixRec(ctypes.Structure):
+    """One mv_mix_rec; on the device the records of a batch are an int32 [B, 8] tensor (mix_records reads it)."""
+    _fields_ = [("lam", ctypes.c_float), ("w_self", ctypes.c_float), ("w_other", ctypes.c_float),
+                ("cutmix", ctypes.c_int), ("y0", ctypes.c_int), ("y1", ctypes.c_int), ("x0", ctypes.c_int),
+                ("x1", ctypes.c_int)]
+
+
+# ctypes signatures of entry points declared with full argument types (tests/test_distill_host.py and
+# tests/test_mixup_host.py hold them to the header's prototypes)
 _P, _I, _F = ctypes.c_void_p, ctypes.c_int, ctypes.c_float
 SIGNATURES = {
     "mv_token_row": [_P, _P, _I, _I, _I, _I, _I, _I, _P],
     "mv_distill_loss": [_P, _P, _P, _P, _I, _I, _F, _F, _I, _P, _P, _P, _P, _P],
+    "mv_mix_draw": [_P, _I, _I, _I, _I, MixSpec, _P, _P],
+    "mv_patchify_mix_q": [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P],
+    "mv_mix_ce_loss": [_P, _P, _P, _I, _I, _F, _P, _P, _P, _P],
 }
 
 
@@ -477,6 +495,68 @@ def patchify_q(img, patch, q_in=None, out_dtype=torch.float16, cls_slot=False):
         _check(lib().mv_patchify_q(_ptr(img), _ptr(out), _DT[out_dtype], B, C, H, W, patch, q[0], q[1],
                                    cls_slot, _stream()), "mv_patchify_q")
     return out
+
+
+def mix_draw(seed, B, H, W, spec, rank=0, recs=None):
+    """mv_mix_draw: -> the records of one mixed batch, int32 [B, 8] on the device (mv_mix_rec each: use mix_records to
+    read them).  seed: a 1-element int64 CUDA tensor; spec: a MixSpec."""
+    _need_cuda(seed)
+    assert seed.dtype == torch.int64 and seed.numel() == 1
+    if recs is None:
+        recs = torch.empty(B, 8, dtype=torch.int32, device=seed.device)
+    assert recs.dtype == torch.int32 and recs.shape == (B, 8) and recs.is_contiguous()
+    _check(lib().mv_mix_draw(_ptr(seed), int(rank), int(B), int(H), int(W), spec, _ptr(recs), _stream()),
+           "mv_mix_draw")
+    return recs
+
+
+def mix_records(recs):
+    """int32 [B, 8] records -> {"lam", "w_self", "w_other": fp32 [B]; "cutmix", "y0", "y1", "x0", "x1": int32 [B]}."""
+    f = recs[:, :3].view(torch.float32)
+    out = {"lam": f[:, 0], "w_self": f[:, 1], "w_other": f[:, 2]}
+    out.update({k: recs[:, 3 + i] for i, k in enumerate(("cutmix", "y0", "y1", "x0", "x1"))})
+    return out
+
+
+def _check_recs(recs, B):
+    _need_cuda(recs)
+    assert recs.dtype == torch.int32 and recs.shape == (B, 8) and recs.is_contiguous(), "records must be int32 [B, 8]"
+
+
+def patchify_mix_q(img, recs, patch, q_in=None, out_dtype=torch.float16, cls_slot=False):
+    """patchify_q of the batch mixed as the records (mix_draw) say, in one pass (mv_patchify_mix_q)."""
+    _need_cuda(img)
+    img = img.contiguous().float()
+    B, C, H, W = img.shape
+    _check_recs(recs, B)
+    cls_slot = int(cls_slot)
+    rows = B * ((H // patch) * (W // patch) + cls_slot)
+    out = torch.empty(rows, patch * patch * C, dtype=out_dtype, device=img.device)
+    q = _fmt(q_in)
+    with _timed("patchify_mix", 0.0, img.numel() * 8 + out.numel() * out.element_size()):
+        _check(lib().mv_patchify_mix_q(_ptr(img), _ptr(recs), _ptr(out), _DT[out_dtype], B, C, H, W, patch, q[0], q[1],
+                                       cls_slot, _stream()), "mv_patchify_mix_q")
+    return out
+
+
+def mix_ce_loss(logits, labels, recs, smoothing):
+    """mv_mix_ce_loss: -> (loss fp32 [1], d loss / d logits), on the device.  logits fp32 [B, C], labels int64 [B],
+    recs the records of the mixed batch or None (unmixed: label-smoothed cross-entropy)."""
+    _need_cuda(logits, labels)
+    logits = logits.detach().float().contiguous()
+    labels = labels.contiguous()
+    assert logits.dim() == 2, "logits must be [B, C]"
+    assert labels.dtype == torch.int64 and labels.shape == logits.shape[:1], "labels must be int64 [B]"
+    B, C = logits.shape
+    if recs is not None:
+        _check_recs(recs, B)
+    loss = torch.empty(1, dtype=torch.float32, device=logits.device)
+    rows = torch.empty(B, dtype=torch.float32, device=logits.device)
+    dx = torch.empty_like(logits)
+    with _timed("mix_ce_loss", 0.0, B * C * 4 * 3):
+        _check(lib().mv_mix_ce_loss(_ptr(logits), _ptr(labels), _ptr(recs), B, C, ctypes.c_float(smoothing),
+                                    _ptr(loss), _ptr(rows), _ptr(dx), _stream()), "mv_mix_ce_loss")
+    return loss, dx
 
 
 def cls_rows(cls, pos_q, x, B, n_tokens, D, q_ff=None):

@@ -310,9 +310,12 @@ class ViT(nn.Module):
         return {"pred_logits": self._linear(dec.class_embed, t, 0),
                 "pred_boxes": self._linear(dec.bbox_embed, t, 2).sigmoid()}
 
-    def forward(self, img: torch.Tensor, distill_token: Optional[torch.Tensor] = None):
+    def forward(self, img: torch.Tensor, distill_token: Optional[torch.Tensor] = None,
+                mix: Optional[torch.Tensor] = None):
         """distill_token ([1, 1, dim], classification only): appended to the sequence as its last row, without a
-        positional embedding (models/distill.py); the forward then returns (logits, encoder output of that row)."""
+        positional embedding (models/distill.py); the forward then returns (logits, encoder output of that row).
+        mix (classification only): Mixup / CutMix records (utils/mixup.py): the encoder sees the batch mixed as they
+        say, mixed inside the patch gather."""
         if not img.is_cuda:
             raise RuntimeError("myrtle-vision_b200 runs on CUDA (sm_100a) only; there is no CPU "
                                "fallback — move the model and the batch to a B200")
@@ -321,13 +324,18 @@ class ViT(nn.Module):
                 raise ValueError("a distillation token needs decoder='classification', not %r" % (self.task,))
             if tuple(distill_token.shape) != (1, 1, self.dim):
                 raise ValueError("distill_token must be [1, 1, %d], got %s" % (self.dim, tuple(distill_token.shape)))
+        if mix is not None:
+            if self.task != "classification":
+                raise ValueError("Mixup / CutMix needs decoder='classification', not %r" % (self.task,))
+            if distill_token is not None:
+                raise ValueError("Mixup / CutMix together with a distillation token is not supported")
         b, c, h, w = img.shape
         p = self.patch_size
         engine = self.engine()
         engine.training = self.training          # dropout (self.dropout_p, self.emb_dropout_p) in training mode only
         pos_full = self._pos_full(h // p, w // p)
         x = mv_engine.EncoderFunction.apply(engine, img, pos_full, self.cls_token,
-                                            *engine.params, token=distill_token)
+                                            *engine.params, token=distill_token, mix=mix)
         self._grad_round_seed = engine.step_grad_round_seed      # the decoder's stubs round with the encoder's seed
         with engine._range("mlp_head"):
             if distill_token is not None:

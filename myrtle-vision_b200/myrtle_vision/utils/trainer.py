@@ -28,6 +28,7 @@ from qtorch.optim import OptimLP
 from myrtle_vision.datasets.synthetic import SyntheticVision, detection_collate
 from myrtle_vision.models.matcher import pad_targets
 from myrtle_vision.utils.graph import GraphedTrainStep
+from myrtle_vision.utils.mixup import MixupLoss, MixupWrapper, build_mixup, parse_mix_config
 from myrtle_vision.utils.models import (get_models, get_optimizer_args, prepare_model_and_load_ckpt,
                                         save_checkpoint)
 from myrtle_vision.utils.optim import create_optimizer, create_scheduler, wrap_optim_lp
@@ -124,6 +125,8 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     train_config["local_batch_size"] = batch_size
     train_config["global_batch_size"] = batch_size * n_batch_accum * max(1, num_gpus)
     train_config["n_batch_accum"] = n_batch_accum
+    # Mixup / CutMix / label smoothing (DeiT's train_config keys, utils/mixup.py): validated before anything is built
+    mix = parse_mix_config(train_config, task, batch_size, "distiller_config" in config)
     if num_gpus > 1:
         init_distributed(rank, num_gpus, **dist_config)
     torch.cuda.set_device(rank)
@@ -150,9 +153,13 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     model = vit
     if distiller is not None:
         model = distiller.to(device)
+    elif mix["active"]:
+        # the step trains the wrapper, which mixes each training batch; it has no parameters of its own, so the
+        # optimizer and checkpoints are the ViT's, and validation runs the bare ViT on unmixed images, as DeiT
+        model = MixupWrapper(vit, build_mixup(mix, data_config["number_of_classes"]))
     net = DataParallel(model) if num_gpus > 1 else model
     optimizer_args = get_optimizer_args(train_config)
-    optimizer = create_optimizer(optimizer_args, model)
+    optimizer = create_optimizer(optimizer_args, distiller if distiller is not None else vit)
     if train_config.get("optim_lp") is not None:
         # qtorch.optim.OptimLP: low-precision weights, gradients, moments and accumulator (DESIGN.md section 7)
         optimizer = wrap_optim_lp(optimizer, train_config["optim_lp"])
@@ -162,6 +169,8 @@ def train_deit(rank, num_gpus, config, task=None, max_iterations=None):
     if distiller is not None:
         from myrtle_vision.models.distill import DistillLoss
         train_criterion = DistillLoss(distiller.temperature, distiller.alpha, distiller.hard)
+    elif mix["active"] or mix["smoothing"] > 0:
+        train_criterion = MixupLoss(mix["smoothing"])        # soft targets; smoothing alone: unmixed logits
     iteration = prepare_model_and_load_ckpt(train_config=train_config, model=vit, optimizer=optimizer,
                                             lr_scheduler=lr_scheduler, distiller=distiller)
     # detection: targets padded to a fixed [B, capacity] block and matched on the device (csrc/assign.cu),
